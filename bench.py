@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun)
     python bench.py --impl reference ...                     CPU arm (oracle port, see below)
+    python bench.py ... --dump-outputs DIR                   also write the last timed step's clustering as DIR/*.npy
 
 Workload (config.workload): synthetic 1M unique 12-mers, phage-display shape, Zipf abundance,
 BLOSUM62, Hammock's automatic parameters (T=20, X=3, K=25000) -- BASELINE.json configs[2], the
@@ -113,7 +114,29 @@ def cpu_sample(d, M, params, p1_steps, p2_queries):
     dt = time.time() - t
     pairs = R.counters["p1_pairs"] + R.counters["p2_pairs_early"]
     return {"seconds": dt, "pairs": pairs, "pairs_per_s": pairs / dt, "cores": cores, "p1_steps": p1_steps,
-            "p2_queries": p2_queries, "status": R.status}
+            "p2_queries": p2_queries, "status": R.status, "result": R}
+
+
+DUMP_LIMIT_BYTES = 60_000_000
+
+
+def dump_outputs(out_dir, r, limit=DUMP_LIMIT_BYTES):
+    """Write the clustering a caller receives (cluster_id, member_rank, result_order, n_multi) as <out_dir>/<name>.npy in
+    float64, which holds the int32 results exactly, so that two builds can be compared output for output.  If the whole
+    set would exceed `limit` bytes, each array longer than its share is replaced by a fixed, seeded sample of its
+    elements, and the sampled positions are written beside it as <name>_index.npy."""
+    outputs = {"cluster_id": r.cluster_id, "member_rank": r.member_rank, "result_order": r.result_order,
+               "n_multi": r.n_multi}
+    os.makedirs(out_dir, exist_ok=True)
+    whole = sum(np.size(a) for a in outputs.values()) * 8 <= limit
+    cap = limit // (16 * len(outputs))             # 8 B per sampled value + 8 B per position
+    for name, a in outputs.items():
+        a = np.asarray(a, dtype=np.float64).reshape(-1)
+        if not whole and a.size > cap:
+            idx = np.sort(np.random.default_rng(SEED).choice(a.size, cap, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def golden_digest(name):
@@ -183,7 +206,11 @@ def main():
     ap.add_argument("--n", type=int, default=N_SEQ, help="debug only: smaller synthetic set")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the clustering the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # the contract is ONE JSON line on stdout: libraries (NCCL prints its version) write to fd 1 too,
     # so everything but the final line is sent to stderr
     real_stdout = os.fdopen(os.dup(1), "w")
@@ -202,6 +229,8 @@ def main():
             s = cpu_sample(d, M, params, 500, 5000)
             if i >= args.warmup:
                 vals.append(s)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, vals[-1]["result"])
         # phase sizes of the full job (independent of who computes them)
         T, X, P, K = params
         p1_steps = K  # >= K steps are needed to open K clusters
@@ -296,6 +325,10 @@ def main():
     barrier()
     wall = time.time() - t_wall
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        last = ctx.download()          # every rank holds the whole clustering; rank 0 writes it
+        if rank == 0:
+            dump_outputs(args.dump_outputs, last)
     ms_per_step = max_over_ranks(float(np.mean(dev_ms)))
     sections = ctx.section_ms()
 

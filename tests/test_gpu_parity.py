@@ -339,6 +339,28 @@ def test_s1m_properties(blosum62, golden_dir):
     ctx.close()
 
 
+def test_bench_dump_outputs_match_the_oracle(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the clustering of the last timed step (float64 .npy): equal to the oracle's
+    full run on the same seeded input, here on a small set"""
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "3", "--n", "20000",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, cwd=root, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2 and line["config"]["n_sequences"] == 20000
+    d, M, (T, X, P, K) = bench.workload(20000)
+    R = oracle_run(d, M, T, X, P, K)
+    assert R.status == 0
+    got = {k: np.load(tmp_path / f"{k}.npy") for k in ("cluster_id", "member_rank", "result_order", "n_multi")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert (got["cluster_id"] == R.cluster_id).all() and (got["member_rank"] == R.member_rank).all()
+    assert (got["result_order"] == R.result_order).all() and got["n_multi"].tolist() == [R.n_multi]
+    assert line["result_digest"] == hb.result_digest(R.cluster_id, R.member_rank, R.result_order)
+
+
 def test_cpp_host_driver_end_to_end(tmp_path, golden_dir, blosum62):
     """hammock_greedy (C++ host side + C ABI): fasta in, the reference's result files out; compared with the
     Python mirror's writers on the same clustering and with the MUSI golden assignment."""

@@ -740,3 +740,42 @@ def test_reference_arm_of_the_bench_runs_on_the_cpu():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": "seq/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["extrapolated"] is True and "workload" in d["config"]
+
+
+def test_bench_dump_outputs_of_the_reference_arm(tmp_path):
+    """`--dump-outputs DIR` writes the clustering of the last timed step as float64 .npy files: here the bounded oracle
+    sample of the reference arm, which must equal the same bounded oracle run on the same seeded input"""
+    import subprocess
+    import sys
+    import bench
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "0",
+                        "--n", "20000", "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, cwd=ROOT,
+                       timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d, M, (T, X, P, K) = bench.workload(20000)
+    R = O.greedy_cluster(d["residues"], d["offsets"], d["abundance"], M, T, X, P, K, max_p1_steps=500, max_p2_queries=5000)
+    assert R.status == 0
+    assert sorted(os.listdir(tmp_path / "dump")) == ["cluster_id.npy", "member_rank.npy", "n_multi.npy", "result_order.npy"]
+    got = {k: np.load(tmp_path / "dump" / f"{k}.npy") for k in ("cluster_id", "member_rank", "result_order", "n_multi")}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert (got["cluster_id"] == R.cluster_id).all() and (got["member_rank"] == R.member_rank).all()
+    assert (got["result_order"] == R.result_order).all() and got["n_multi"].tolist() == [R.n_multi]
+
+
+def test_bench_dump_outputs_samples_what_exceeds_the_limit(tmp_path):
+    """outputs above the size limit are replaced by a fixed, seeded sample with its positions; small ones stay whole"""
+    import bench
+    rng = np.random.default_rng(1)
+    r = hb.GreedyResult(rng.integers(0, 1 << 30, 5000).astype(np.int32), rng.integers(0, 9, 5000).astype(np.int32),
+                        np.arange(300, dtype=np.int32), 7, {})
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), r, limit=16 * 4 * 1000)
+    for k, a in (("cluster_id", r.cluster_id), ("member_rank", r.member_rank)):
+        idx = np.load(tmp_path / "a" / f"{k}_index.npy")
+        v = np.load(tmp_path / "a" / f"{k}.npy")
+        assert len(idx) == len(v) == 1000 and len(np.unique(idx)) == 1000
+        assert (v == a[idx.astype(np.int64)]).all()
+        assert (idx == np.load(tmp_path / "b" / f"{k}_index.npy")).all()
+    assert (np.load(tmp_path / "a" / "result_order.npy") == r.result_order).all()
+    assert not os.path.exists(tmp_path / "a" / "result_order_index.npy")
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 16 * 4 * 1000 + 8 * 128
