@@ -42,7 +42,7 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
-EXPORTS = ["hmk_abi_version", "hmk_greedy_cluster", "hmk_greedy_cluster_multi", "hmk_clinkage_cluster", "hmk_create", "hmk_destroy", "hmk_upload", "hmk_run",
+EXPORTS = ["hmk_abi_version", "hmk_greedy_cluster", "hmk_greedy_cluster_multi", "hmk_clinkage_cluster", "hmk_clinkage_run", "hmk_create", "hmk_destroy", "hmk_upload", "hmk_run",
            "hmk_download", "hmk_get_stats", "hmk_get_section_ms", "hmk_set_option", "hmk_score_block",
            "hmk_timer_begin", "hmk_timer_end", "hmk_measure_peaks", "hmk_nccl_unique_id", "hmk_init_distributed", "hmk_release_cached"]
 SECTIONS = ["p1_select", "p1_partner", "p1_cluster", "p1_intra", "p1_resolve", "p2_setup", "p2_filter", "p2_check",
@@ -70,6 +70,8 @@ def load():
     L.hmk_greedy_cluster_multi.argtypes = [C.POINTER(GreedyIn), C.POINTER(GreedyOut), i32p, C.c_int32, cp, sz]
     L.hmk_clinkage_cluster.restype = C.c_int
     L.hmk_clinkage_cluster.argtypes = [C.POINTER(GreedyIn), C.POINTER(GreedyOut), C.c_int, cp, sz]
+    L.hmk_clinkage_run.restype = C.c_int
+    L.hmk_clinkage_run.argtypes = [vp, C.POINTER(GreedyIn), C.POINTER(GreedyOut), cp, sz]
     L.hmk_create.restype = C.c_int
     L.hmk_create.argtypes = [C.POINTER(vp), C.c_int, cp, sz]
     L.hmk_destroy.restype = None

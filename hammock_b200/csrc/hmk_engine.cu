@@ -107,6 +107,11 @@ struct DevBuf {
         CK(cudaMalloc(&p, std::max<size_t>(n, 1) * sizeof(T)));
         cap = n;
     }
+    void release() {
+        if (p) CK(cudaFree(p));
+        p = nullptr;
+        cap = 0;
+    }
     void grow_keep(size_t n, size_t used, cudaStream_t st) {
         if (n <= cap) return;
         T* q = nullptr;
@@ -166,6 +171,8 @@ struct Options {
     int64_t persistent = 1;       // 1: filter kernel as one CTA per SM taking database chunks dynamically; 0: static grid
     int64_t p2_first = 0;         // queries in the first phase-2 window (0 = automatic)
     int64_t xhit_cap = 0;         // capacity of the kept-hit buffer (0 = automatic: the last run's need, else 96 per sequence)
+    int64_t clinkage_dense_max = 32768;   // exact complete linkage: largest n that takes the dense n x n path
+    int64_t clinkage_threads = 0;         // threads of the sparse chain kernel (0 = automatic, from the row lengths)
 };
 
 class Engine {
@@ -227,6 +234,7 @@ public:
     void download(hmk_greedy_out* out);
     void score_block(const int32_t* first, int32_t nf, const int32_t* second, int32_t ns, int32_t* scores);
     int clinkage(const hmk_greedy_in* in, hmk_greedy_out* out);
+    std::string status_msg;      // details of the last non-zero status, when there are any
     hmk_stats stats{};
     int error_step = -1;
     void timer_begin() { CK(cudaSetDevice(device_)); CK(cudaEventRecord(ev_t0_, st_)); }
@@ -320,6 +328,12 @@ private:
         d_ac_cnt_, d_ac_slot_, d_ac_score_, d_dirty_a_;
     DevBuf<int4> d_ac_full_, d_ac_best_;
     DevBuf<int32_t> d_sched_, d_clD_, d_cli_, d_lsort_;
+    // sparse complete-linkage rows (see clinkage_rows)
+    DevBuf<int64_t> d_cloff_;
+    DevBuf<unsigned long long> d_cldeg_;
+    DevBuf<uint64_t> d_clrows_, d_clalt_;
+    DevBuf<int32_t> d_cltwin_, d_clrel_;
+    int clinkage_rows(int* threads);
     bool lsort_ = false;
     // phase-1 partner-search hits kept for phase 2 (opt.reuse): buffer, 64-bit counters [0] appended, [1] valid
     DevBuf<int4> d_xhits_;
@@ -1559,14 +1573,17 @@ void Engine::score_block(const int32_t* first, int32_t nf, const int32_t* second
 }
 
 // ---------------------------------------------------------------- exact complete-linkage clustering (SURVEY.md 8f N1)
-// ClinkageSequenceClusterer.cluster (ClinkageSequenceClusterer.java:43-124): dense pair scores from the bulk kernel,
-// nearest-neighbour chain in hmk_clinkage_chain.  Returns the status; fills `out` on success.
+// ClinkageSequenceClusterer.cluster (ClinkageSequenceClusterer.java:43-124).  n <= opt.clinkage_dense_max: dense pair
+// scores from the bulk kernel, nearest-neighbour chain in hmk_clinkage_chain.  Larger n: the entries scoring >= T only
+// (clinkage_rows), chain in hmk_clinkage_chain_sparse -- the same result.  Returns the status; fills `out` on success.
 int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     upload(in);
     stats = hmk_stats{};
     stats.error_step = -1;
+    status_msg.clear();
     launches_ = bulk_launches_ = 0;
     ev_used_ = 0; bulk_events_.clear(); sections_.clear(); sec_open_ = -1;
+    for (double& v : section_ms) v = 0;
     if (!out || (n_ > 0 && (!out->cluster_id || !out->member_rank || !out->result_order)))
         throw std::invalid_argument("hmk_clinkage_cluster: null output array");
     out->n_result = 0; out->n_multi = 0; out->error_step = -1;
@@ -1574,12 +1591,14 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
         throw std::invalid_argument("hmk_clinkage_cluster: no sequences (the reference throws NoSuchElementException)");
     if (bad_residue_) return HMK_ERR_BAD_RESIDUE;
     if (!sym_) return HMK_STATUS_UNSUPPORTED;          // CachedClusterScorer keeps one value per unordered pair of clusters
-    if (n_ > 32768) return HMK_STATUS_UNSUPPORTED;     // n x n int32 scores; the reference switches to greedy above 10 000
     if (n_ >= 2 && X_ >= min_len_) return HMK_ERR_SHIFT_TOO_BIG;
+    const bool sparse = n_ > opt.clinkage_dense_max;
     const size_t n = (size_t)n_;
-    d_clD_.reserve(n * n);
     CK(cudaEventRecord(ev_a_, st_));
-    {   // D[q][i] = sequenceScore(seq i, seq q) (symmetric), one batch of profiles at a time
+    sec(0);
+    int threads = HMK_CL_THREADS;
+    if (!sparse) {   // D[q][i] = sequenceScore(seq i, seq q) (symmetric), one batch of profiles at a time
+        d_clD_.reserve(n * n);
         std::vector<int32_t> ids(n_);
         std::iota(ids.begin(), ids.end(), 0);
         CK(cudaMemcpyAsync(d_sidx_.p, ids.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, st_));
@@ -1595,8 +1614,13 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
             a.dense = d_clD_.p + (size_t)q0 * n; a.dense_stride = n_;
             launch_bulk(HMK_MODE_DENSE, a, d_sidx_.p + q0, 1);
         }
+        hmk_clinkage_threshold<<<sm_count_ * 8, 256, 0, st_>>>(d_clD_.p, n * n, T_);
+        stats.bulk_pairs = (int64_t)n * (int64_t)n;
+    } else {
+        const int rc = clinkage_rows(&threads);
+        if (rc) { sec(-1); return rc; }
     }
-    hmk_clinkage_threshold<<<sm_count_ * 8, 256, 0, st_>>>(d_clD_.p, n * n, T_);
+    sec(2);
     int acap = 16;
     while (n_ > (int)(acap * 0.75f)) acap *= 2;          // java.util.HashMap: doubled whenever size > 0.75 x capacity
     int rcap = 16;
@@ -1605,7 +1629,9 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     d_cli_.reserve((size_t)acap * 2 + maxid * 4 + n * 8 + 1 + (size_t)rcap * 4 + 8);
     HmkClinkage C{};
     int32_t* p = d_cli_.p;
-    C.n = n_; C.T = T_; C.D = d_clD_.p; C.ab = d_ab_.p; C.acap = acap;
+    C.n = n_; C.T = T_; C.ab = d_ab_.p; C.acap = acap;
+    if (sparse) { C.row_off = d_cloff_.p; C.rows = d_clrows_.p; C.twin = d_cltwin_.p; }
+    else C.D = d_clD_.p;
     C.a_head = p; p += acap; C.a_tail = p; p += acap;
     C.a_next = p; p += maxid; C.a_prev = p; p += maxid; C.slot_of = p; p += maxid; C.r_next = p; p += maxid;
     C.id_of = p; p += n; C.size_of = p; p += n; C.mhead = p; p += n; C.mtail = p; p += n; C.mnext = p; p += n;
@@ -1613,9 +1639,11 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     C.r_head = p; p += (size_t)rcap * 4; C.rcap_max = rcap;
     C.out_scalars = p; p += 8;
     C.cluster_id = d_cluster_id_.p; C.member_rank = d_member_rank_.p;
-    hmk_clinkage_chain<<<1, HMK_CL_THREADS, 0, st_>>>(C);
+    if (sparse) hmk_clinkage_chain_sparse<<<1, threads, 0, st_>>>(C);
+    else hmk_clinkage_chain<<<1, HMK_CL_THREADS, 0, st_>>>(C);
     CK(cudaGetLastError());
     launches_ += 2;
+    sec(-1);
     CK(cudaEventRecord(ev_c_, st_));
     int32_t sc[8];
     CK(cudaMemcpyAsync(sc, C.out_scalars, sizeof(sc), cudaMemcpyDeviceToHost, st_));
@@ -1623,8 +1651,19 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, ev_a_, ev_c_));
     stats.total_ms = ms; stats.phase1_ms = ms;
+    double bulk_ms = 0;
+    for (auto& pr : bulk_events_) {
+        float t = 0;
+        CK(cudaEventElapsedTime(&t, pr.first, pr.second));
+        bulk_ms += t;
+    }
+    for (auto& sct : sections_) {
+        float t = 0;
+        CK(cudaEventElapsedTime(&t, sct.second.first, sct.second.second));
+        section_ms[sct.first] += t;
+    }
+    stats.bulk_kernel_ms = bulk_ms;
     stats.bulk_launches = bulk_launches_; stats.total_launches = launches_;
-    stats.bulk_pairs = (int64_t)n * (int64_t)n;
     stats.p1_steps = sc[3];                          // nearest-neighbour searches
     stats.fast_path = fast_ ? 1 : 0;
     stats.lane_bits = fast_ ? (sc_.lane16 ? 16 : 8) : 32;
@@ -1635,6 +1674,123 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     CK(cudaStreamSynchronize(st_));
     out->n_result = sc[0];
     out->n_multi = sc[1];
+    return HMK_OK;
+}
+
+// Sparse complete-linkage scores: every pair of the upper triangle scoring >= T, found by the bulk kernel's EMIT mode one
+// query batch at a time (queries [q0, q0 + B) against the thread-side ids [q0, n); pairs with id <= query are dropped),
+// stored as rows of BOTH directions with int64 offsets, each row sorted by neighbour slot, plus the twin index of every
+// entry.  Two scoring passes: the first counts the entries per row (a batch whose hits overflow the buffer is re-run with
+// a bigger one), the second scatters them -- the pair scores are cheap next to the chain, device memory is not.  Before
+// the rows are allocated their bytes are compared with the free device memory: HMK_STATUS_UNSUPPORTED with the count of
+// valid pairs in status_msg when they do not fit.  *threads = block size of the chain kernel.
+int Engine::clinkage_rows(int* threads) {
+    const int n = n_;
+    d_clD_.release();     // the dense matrix of an earlier call on this context
+    std::vector<int32_t> ids(n);
+    std::iota(ids.begin(), ids.end(), 0);
+    CK(cudaMemcpyAsync(d_sidx_.p, ids.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, st_));
+    const int chunk = HMK_MAXBATCH;
+    if (fast_) d_prof_.reserve((size_t)chunk * sc_.prof_words);
+    d_cldeg_.reserve((size_t)n + 1); d_cloff_.reserve((size_t)n + 1);
+    CK(cudaMemsetAsync(d_cldeg_.p, 0, sizeof(unsigned long long) * ((size_t)n + 1), st_));
+    d_hits_.reserve(std::max<size_t>(d_hits_.cap, (size_t)1 << 20));
+    auto score_batch = [&](int q0, int sn) {
+        CK(cudaMemsetAsync(d_counts_.p, 0, sizeof(unsigned int), st_));
+        if (fast_) launch_profiles(HMK_PROF_QUERY, d_sidx_.p + q0, sn, d_prof_.p, sc_, st_);
+        HmkBulkArgs a{};
+        a.prof = d_prof_.p; a.nq = sn;
+        a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = q0; a.ndb = n - q0;
+        a.hits = d_hits_.p; a.hit_count = d_counts_.p; a.hit_cap = (unsigned int)std::min<size_t>(d_hits_.cap, UINT32_MAX);
+        launch_bulk(HMK_MODE_EMIT, a, d_sidx_.p + q0, 1);
+        stats.bulk_pairs += (int64_t)sn * (n - q0);
+    };
+    const int grid = sm_count_ * 4;
+    for (int q0 = 0; q0 < n; q0 += chunk) {          // pass 1: entries per row
+        const int sn = std::min(chunk, n - q0);
+        for (;;) {
+            score_batch(q0, sn);
+            CK(cudaMemcpyAsync(h_scalars_, d_counts_.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st_));
+            CK(cudaStreamSynchronize(st_));
+            const size_t cnt = *reinterpret_cast<unsigned int*>(h_scalars_);
+            if (cnt <= d_hits_.cap) break;
+            d_hits_.reserve(cnt + cnt / 4);          // the hit counter kept counting past the capacity: re-run the batch
+        }
+        hmk_cl_count_hits<<<grid, 256, 0, st_>>>(d_hits_.p, d_counts_.p, (unsigned int)d_hits_.cap, q0, n, d_cldeg_.p);
+        CK(cudaGetLastError());
+        launches_++;
+    }
+    size_t bytes = 0;
+    unsigned long long* off = reinterpret_cast<unsigned long long*>(d_cloff_.p);
+    CK(cub::DeviceScan::ExclusiveSum(nullptr, bytes, d_cldeg_.p, off, n + 1, st_));
+    d_cub_.reserve(bytes);
+    CK(cub::DeviceScan::ExclusiveSum(d_cub_.p, bytes, d_cldeg_.p, off, n + 1, st_));
+    std::vector<int64_t> h_off((size_t)n + 1);
+    CK(cudaMemcpyAsync(h_off.data(), d_cloff_.p, sizeof(int64_t) * ((size_t)n + 1), cudaMemcpyDeviceToHost, st_));
+    CK(cudaStreamSynchronize(st_));
+    const size_t E = (size_t)h_off[n];
+    size_t maxrow = 0;
+    for (int i = 0; i < n; i++) maxrow = std::max<size_t>(maxrow, (size_t)(h_off[i + 1] - h_off[i]));
+    // the rows are sorted in groups of consecutive rows (cub's segmented sort counts items in int)
+    const size_t group_cap = std::max<size_t>(maxrow, std::min<size_t>(E, (size_t)1 << 28));
+    size_t sort_bytes = 0;
+    {
+        cub::DoubleBuffer<uint64_t> db(nullptr, nullptr);
+        CK(cub::DeviceSegmentedSort::SortKeys(nullptr, sort_bytes, db, (int)std::max<size_t>(group_cap, 1), n, d_clrel_.p,
+                                              d_clrel_.p + 1, st_));
+    }
+    const size_t need = E * (sizeof(uint64_t) + sizeof(int32_t)) + group_cap * sizeof(uint64_t) + sort_bytes +
+                        ((size_t)n + 1) * sizeof(int32_t);
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    const size_t have = free_b + d_clrows_.cap * sizeof(uint64_t) + d_cltwin_.cap * sizeof(int32_t) +
+                        d_clalt_.cap * sizeof(uint64_t) + d_cub_.cap + d_clrel_.cap * sizeof(int32_t);
+    stats.xhits_kept = (int64_t)E;
+    if (need > have) {
+        status_msg = "exact complete-linkage clustering of " + std::to_string(n) + " sequences: " + std::to_string(E / 2) +
+                     " valid pairs (" + std::to_string(E) + " directed entries) need " + std::to_string(need) +
+                     " bytes of device memory, " + std::to_string(have) + " are available";
+        return HMK_STATUS_UNSUPPORTED;
+    }
+    sec(1);
+    d_clrows_.reserve(E); d_cltwin_.reserve(E); d_clalt_.reserve(group_cap); d_cub_.reserve(sort_bytes);
+    d_clrel_.reserve((size_t)n + 1);
+    stats.xhits_capacity = (int64_t)d_clrows_.cap;
+    CK(cudaMemsetAsync(d_cldeg_.p, 0, sizeof(unsigned long long) * ((size_t)n + 1), st_));
+    for (int q0 = 0; q0 < n; q0 += chunk) {          // pass 2: the same hits (the buffer already fits every batch), scattered
+        score_batch(q0, std::min(chunk, n - q0));
+        hmk_cl_scatter_hits<<<grid, 256, 0, st_>>>(d_hits_.p, d_counts_.p, (unsigned int)d_hits_.cap, q0, n, d_cloff_.p,
+                                                   d_cldeg_.p, d_clrows_.p);
+        CK(cudaGetLastError());
+        launches_++;
+    }
+    for (int r0 = 0; r0 < n;) {                      // rows sorted by neighbour slot (slots are unique in a row)
+        int r1 = r0 + 1;
+        while (r1 < n && (size_t)(h_off[r1 + 1] - h_off[r0]) <= group_cap) r1++;
+        const size_t items = (size_t)(h_off[r1] - h_off[r0]);
+        if (items > 1) {
+            hmk_cl_rel_offsets<<<(r1 - r0 + 256) / 256, 256, 0, st_>>>(d_cloff_.p, r0, r1 - r0, d_clrel_.p);
+            CK(cudaGetLastError());
+            uint64_t* base = d_clrows_.p + h_off[r0];
+            cub::DoubleBuffer<uint64_t> db(base, d_clalt_.p);
+            size_t b2 = d_cub_.cap;
+            CK(cub::DeviceSegmentedSort::SortKeys(d_cub_.p, b2, db, (int)items, r1 - r0, d_clrel_.p, d_clrel_.p + 1, st_));
+            if (db.Current() != base)
+                CK(cudaMemcpyAsync(base, db.Current(), sizeof(uint64_t) * items, cudaMemcpyDeviceToDevice, st_));
+            launches_ += 2;
+        }
+        r0 = r1;
+    }
+    if (E) {
+        hmk_cl_twins<<<sm_count_ * 8, 256, 0, st_>>>(d_cloff_.p, d_clrows_.p, n, d_cltwin_.p);
+        CK(cudaGetLastError());
+        launches_++;
+    }
+    // a step passes over one row a few times and ends with barriers: a block about as wide as the mean row (rows only
+    // shrink), at least 128 threads
+    int t = 128;
+    while (t < HMK_CL_THREADS && (size_t)t * n < E) t *= 2;
+    *threads = opt.clinkage_threads > 0 ? (int)opt.clinkage_threads : t;
     return HMK_OK;
 }
 
@@ -1749,7 +1905,7 @@ static const char* status_text(int rc) {
         case HMK_STATUS_NULL_CLUSTER: return "NullPointerException: nearest cluster object without a cluster (see error_step)";
         case HMK_STATUS_BAD_RESIDUE: return "FileFormatException: residue code outside 0..23";
         case HMK_STATUS_UNSUPPORTED: return "unsupported input for the exact complete-linkage clusterer: asymmetric substitution matrix, "
-                                            "more than 32768 sequences, or a java.util.HashMap bin that would be treeified";
+                                            "valid pairs beyond the free device memory, or a java.util.HashMap bin that would be treeified";
         default: return "";
     }
 }
@@ -1863,10 +2019,13 @@ int hmk_set_option(hmk_ctx* ctx, const char* name, int64_t value) {
         {"xhit_cap", &o.xhit_cap, 0, (int64_t)1 << 30}, {"p2_first", &o.p2_first, 0, 1 << 24},
         {"persistent", &o.persistent, 0, 1},        {"reserve", &o.reserve, 1, 64},
         {"min_iters", &o.min_iters, 1, 64},         {"bucket_aux", &o.bucket_aux, 0, 1},
+        {"clinkage_dense_max", &o.clinkage_dense_max, 0, 32768},
+        {"clinkage_threads", &o.clinkage_threads, 0, HMK_CL_THREADS},
     };
     for (const Knob& k : knobs) {
         if (s != k.name) continue;
         if (value < k.lo || value > k.hi) return HMK_STATUS_BAD_ARG;
+        if (k.slot == &o.clinkage_threads && value % 32) return HMK_STATUS_BAD_ARG;   // whole warps
         *k.slot = value;
         return HMK_STATUS_OK;
     }
@@ -1910,7 +2069,16 @@ int hmk_clinkage_cluster(const hmk_greedy_in* in, hmk_greedy_out* out, int devic
         auto& slot = cached_ctx()[device];
         if (!slot) slot.reset(new hmk_ctx(device));
         int rc = slot->engine.clinkage(in, out);
-        if (rc) set_err(errbuf, errlen, status_text(rc));
+        if (rc) set_err(errbuf, errlen, slot->engine.status_msg.empty() ? status_text(rc) : slot->engine.status_msg.c_str());
+        return rc;
+    });
+}
+
+int hmk_clinkage_run(hmk_ctx* ctx, const hmk_greedy_in* in, hmk_greedy_out* out, char* errbuf, size_t errlen) {
+    if (!ctx || !in || !out) return HMK_STATUS_BAD_ARG;
+    return guarded(errbuf, errlen, [&] {
+        int rc = ctx->engine.clinkage(in, out);
+        if (rc) set_err(errbuf, errlen, ctx->engine.status_msg.empty() ? status_text(rc) : ctx->engine.status_msg.c_str());
         return rc;
     });
 }

@@ -2370,7 +2370,13 @@ __global__ void __launch_bounds__(1024) hmk_peak_lds(int iters, int32_t* out) {
 
 struct HmkClinkage {
     int32_t n, T;
-    int32_t* D;            // [n][n]
+    int32_t* D;            // dense path: [n][n]
+    // sparse path (hmk_clinkage_chain_sparse): the entries with score >= T, both directions, each row sorted by slot.
+    // Entry = (neighbour slot << 32) | (uint32) score; a killed entry has score HMK_JMIN.  twin[e] = position of the
+    // mirror entry (in the row of e's neighbour, pointing back at e's row), relative to the start of that row.
+    const int64_t* row_off;   // [n + 1]
+    uint64_t* rows;
+    const int32_t* twin;
     const int32_t* ab;
     int32_t acap;          // capacity of the activeClusters table
     int32_t* a_head;       // [acap] -1 = empty bin
@@ -2404,52 +2410,151 @@ __global__ void hmk_clinkage_threshold(int32_t* D, size_t total, int32_t T) {
         if (D[i] < T) D[i] = HMK_CL_BELOW;
 }
 
-__global__ void __launch_bounds__(HMK_CL_THREADS) hmk_clinkage_chain(const HmkClinkage C) {
+// ---- helpers shared by the dense and the sparse chain kernel
+// activeClusters.add(id): append at the tail of its bin; a bin that already holds 7 entries would become a tree in the
+// JDK (different order) -> `treeified`.  One thread.  Returns the bin.
+__device__ __forceinline__ int hmk_cl_set_add(const HmkClinkage& C, int32_t id, int32_t& treeified) {
+    const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(C.acap - 1));
+    HMK_CHECK(id >= 1 && id < 2 * C.n + 3 && b >= 0 && b < C.acap);
+    int len = 0;
+    for (int k = C.a_head[b]; k >= 0; k = C.a_next[k]) len++;
+    if (len >= 7) treeified = 1;
+    C.a_next[id] = -1; C.a_prev[id] = C.a_tail[b];
+    if (C.a_tail[b] >= 0) C.a_next[C.a_tail[b]] = id; else C.a_head[b] = id;
+    C.a_tail[b] = id;
+    return b;
+}
+
+// activeClusters.remove(id).  One thread.
+__device__ __forceinline__ void hmk_cl_set_remove(const HmkClinkage& C, int32_t id) {
+    const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(C.acap - 1));
+    HMK_CHECK(id >= 1 && id < 2 * C.n + 3 && b >= 0 && b < C.acap);
+    const int32_t p = C.a_prev[id], nx = C.a_next[id];
+    if (p >= 0) C.a_next[p] = nx; else C.a_head[b] = nx;
+    if (nx >= 0) C.a_prev[nx] = p; else C.a_tail[b] = p;
+}
+
+// the n singleton clusters, ids 1..n (:48-54): slot tables by all threads, then the set in id order by thread 0.
+// Returns (on thread 0) the lowest non-empty bin.  Ends with a barrier.
+__device__ __forceinline__ int hmk_cl_init(const HmkClinkage& C, int32_t& treeified) {
+    const int n = C.n;
+    for (int b = threadIdx.x; b < C.acap; b += blockDim.x) { C.a_head[b] = -1; C.a_tail[b] = -1; }
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        C.id_of[i] = i + 1; C.slot_of[i + 1] = i; C.size_of[i] = C.ab[i];
+        C.mhead[i] = i; C.mtail[i] = i; C.mnext[i] = -1;
+    }
+    __syncthreads();
+    int lowest = C.acap;
+    if (threadIdx.x == 0) {
+        treeified = 0;
+        for (int id = 1; id <= n; id++) lowest = min(lowest, hmk_cl_set_add(C, id, treeified));   // insertion order = id order
+    }
+    __syncthreads();
+    return lowest;
+}
+
+// merge bookkeeping of thread 0 (:95-109): new Cluster(top.getSequences() ++ nearest.getSequences(), ++currentId) in slot
+// ts, the nearest's slot bs dies.  Returns the bin of the new id.
+__device__ __forceinline__ int hmk_cl_merge(const HmkClinkage& C, int32_t top, int32_t best, int ts, int bs, int32_t& cur_id,
+                                            int32_t& treeified) {
+    cur_id++;
+    HMK_CHECK(cur_id < 2 * C.n + 3 && bs >= 0 && bs < C.n && ts >= 0 && ts < C.n && bs != ts);
+    hmk_cl_set_remove(C, top);
+    hmk_cl_set_remove(C, best);
+    C.mnext[C.mtail[ts]] = C.mhead[bs];
+    C.mtail[ts] = C.mtail[bs];
+    C.size_of[ts] = hmk_wadd(C.size_of[ts], C.size_of[bs]);
+    C.id_of[ts] = cur_id; C.id_of[bs] = -1;
+    C.slot_of[cur_id] = ts;
+    return hmk_cl_set_add(C, cur_id, treeified);
+}
+
+// the last cluster is ready too (:116); then new ArrayList(readyClusters): bucket order of a table that grew with the set
+// (capacity 16, doubled whenever the size exceeded 0.75 x capacity).  Thread 0; `from_bin` <= the lowest non-empty bin;
+// `nr` (ready clusters so far) counts the last one on return.
+__device__ __forceinline__ void hmk_cl_finish(const HmkClinkage& C, int32_t& nr, int from_bin, int32_t treeified, int32_t searches) {
+    for (int b = from_bin; b < C.acap; b++)
+        if (C.a_head[b] >= 0) { C.ready[nr++] = C.a_head[b]; break; }
+    HMK_CHECK(nr <= C.n);
+    // the set as HashMap builds it: append at the bin's tail, double the table (bins split in order) whenever the size
+    // exceeds 0.75 x capacity
+    int rcap = 16, rsize = 0;
+    int32_t* head = C.r_head;                     // two (head, tail) table pairs, used alternately across resizes
+    int32_t* tail = C.r_head + C.rcap_max;
+    int32_t* head2 = C.r_head + 2 * C.rcap_max;
+    int32_t* tail2 = C.r_head + 3 * C.rcap_max;
+    for (int b = 0; b < rcap; b++) { head[b] = -1; tail[b] = -1; }
+    for (int i = 0; i < nr; i++) {
+        const int32_t id = C.ready[i];
+        const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(rcap - 1));
+        int len = 0;
+        for (int32_t k = head[b]; k >= 0; k = C.r_next[k]) len++;
+        if (len >= 7) treeified = 1;
+        C.r_next[id] = -1;
+        if (tail[b] >= 0) C.r_next[tail[b]] = id; else head[b] = id;
+        tail[b] = id;
+        if (++rsize > (int)(rcap * 0.75f)) {
+            const int ncap = rcap * 2;
+            HMK_CHECK(ncap <= C.rcap_max);
+            for (int b2 = 0; b2 < ncap; b2++) { head2[b2] = -1; tail2[b2] = -1; }
+            for (int b2 = 0; b2 < rcap; b2++)
+                for (int32_t k = head[b2], nx; k >= 0; k = nx) {
+                    nx = C.r_next[k];
+                    const int nb = (int)(hmk_cluster_hash(k) & (uint32_t)(ncap - 1));
+                    C.r_next[k] = -1;
+                    if (tail2[nb] >= 0) C.r_next[tail2[nb]] = k; else head2[nb] = k;
+                    tail2[nb] = k;
+                }
+            int32_t* t1 = head; head = head2; head2 = t1;
+            t1 = tail; tail = tail2; tail2 = t1;
+            rcap = ncap;
+        }
+    }
+    int o = 0, multi = 0;
+    for (int b = 0; b < rcap; b++)
+        for (int32_t id = head[b]; id >= 0; id = C.r_next[id]) { HMK_CHECK(o < nr); C.result_order[o++] = id; }
+    for (int i = 0; i < nr; i++) { const int s = C.slot_of[C.result_order[i]]; multi += C.mhead[s] != C.mtail[s]; }
+    C.out_scalars[0] = nr; C.out_scalars[1] = multi; C.out_scalars[2] = treeified; C.out_scalars[3] = searches;
+}
+
+// cluster_id / member_rank of every member of the nr returned clusters.  All threads, after a barrier.
+__device__ __forceinline__ void hmk_cl_members(const HmkClinkage& C, int nr) {
+    for (int i = threadIdx.x; i < nr; i += blockDim.x) {
+        const int32_t id = C.result_order[i];
+        int32_t rank = 0;
+        for (int32_t m = C.mhead[C.slot_of[id]]; m >= 0; m = C.mnext[m]) {
+            HMK_CHECK(m >= 0 && m < C.n);
+            C.cluster_id[m] = id; C.member_rank[m] = rank++;
+        }
+    }
+}
+
+// arg-max of the block's per-thread candidates under hmk_consider's order; the result is valid on thread 0 only.
+// r_*: [32] shared scratch.  Ends without a barrier (the caller's next one separates the reuse of r_*).
+__device__ __forceinline__ HmkBestCluster hmk_cl_block_best(HmkBestCluster bb, int32_t* r_score, int32_t* r_size, int32_t* r_id) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    hmk_best_reduce(bb);
+    if (lane == 0) { r_score[wid] = bb.slot >= 0 ? bb.score : HMK_JMIN; r_size[wid] = bb.size; r_id[wid] = bb.slot >= 0 ? bb.fid : -1; }
+    __syncthreads();
+    HmkBestCluster g;
+    g.score = HMK_JMIN; g.size = 0; g.fid = 0; g.slot = -1;
+    if (threadIdx.x == 0)
+        for (int w = 0; w < (int)(blockDim.x >> 5); w++)
+            if (r_id[w] >= 0) hmk_consider(g, r_score[w], r_size[w], r_id[w], w);
+    return g;
+}
+
+__global__ void __launch_bounds__(HMK_CL_THREADS, 1) hmk_clinkage_chain(const HmkClinkage C) {
     __shared__ int32_t r_score[32], r_size[32], r_id[32];
     __shared__ int32_t s_top, s_best, s_action, s_ts, s_bs;     // action: 0 ready, 1 merge, 2 push
     __shared__ int32_t s_first[32];
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     const int n = C.n;
     const unsigned FULL = 0xffffffffu;
-    // ---- the n singleton clusters, ids 1..n (:48-54)
-    for (int b = tid; b < C.acap; b += blockDim.x) { C.a_head[b] = -1; C.a_tail[b] = -1; }
-    for (int i = tid; i < n; i += blockDim.x) {
-        C.id_of[i] = i + 1; C.slot_of[i + 1] = i; C.size_of[i] = C.ab[i];
-        C.mhead[i] = i; C.mtail[i] = i; C.mnext[i] = -1;
-    }
-    __syncthreads();
     __shared__ int32_t sp, nr, nactive, cur_id, treeified, searches;
-    if (tid == 0) {
-        treeified = 0;
-        for (int id = 1; id <= n; id++) {            // insertion order = id order; chains are short (consecutive hash codes)
-            const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(C.acap - 1));
-            int len = 0;
-            for (int k = C.a_head[b]; k >= 0; k = C.a_next[k]) len++;
-            if (len >= 7) treeified = 1;
-            C.a_next[id] = -1; C.a_prev[id] = C.a_tail[b];
-            if (C.a_tail[b] >= 0) C.a_next[C.a_tail[b]] = id; else C.a_head[b] = id;
-            C.a_tail[b] = id;
-        }
-        sp = 0; nr = 0; nactive = n; cur_id = n + 1; searches = 0;
-    }
+    hmk_cl_init(C, treeified);
+    if (tid == 0) { sp = 0; nr = 0; nactive = n; cur_id = n + 1; searches = 0; }
     __syncthreads();
-    auto set_remove = [&](int32_t id) {               // thread 0
-        const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(C.acap - 1));
-        const int32_t p = C.a_prev[id], nx = C.a_next[id];
-        if (p >= 0) C.a_next[p] = nx; else C.a_head[b] = nx;
-        if (nx >= 0) C.a_prev[nx] = p; else C.a_tail[b] = p;
-        nactive--;
-    };
-    auto set_add = [&](int32_t id) {                  // thread 0
-        const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(C.acap - 1));
-        int len = 0;
-        for (int k = C.a_head[b]; k >= 0; k = C.a_next[k]) len++;
-        if (len >= 7) treeified = 1;
-        C.a_next[id] = -1; C.a_prev[id] = C.a_tail[b];
-        if (C.a_tail[b] >= 0) C.a_next[C.a_tail[b]] = id; else C.a_head[b] = id;
-        C.a_tail[b] = id;
-        nactive++;
-    };
     for (;;) {
         // ---- empty stack: activeClusters.iterator().next() -- the head of the first non-empty bin (:62-70)
         if (sp == 0) {
@@ -2479,21 +2584,16 @@ __global__ void __launch_bounds__(HMK_CL_THREADS) hmk_clinkage_chain(const HmkCl
             if (id < 0 || k == ts) continue;
             hmk_consider(bb, C.D[(size_t)ts * n + k], C.size_of[k], id, k);
         }
-        hmk_best_reduce(bb);
-        if (lane == 0) { r_score[wid] = bb.slot >= 0 ? bb.score : HMK_JMIN; r_size[wid] = bb.size; r_id[wid] = bb.slot >= 0 ? bb.fid : -1; }
-        __syncthreads();
+        const HmkBestCluster g = hmk_cl_block_best(bb, r_score, r_size, r_id);
         if (tid == 0) {
-            HmkBestCluster g;
-            g.score = HMK_JMIN; g.size = 0; g.fid = 0; g.slot = -1;
-            for (int w = 0; w < (int)(blockDim.x >> 5); w++)
-                if (r_id[w] >= 0) hmk_consider(g, r_score[w], r_size[w], r_id[w], w);
             const int32_t best = g.slot >= 0 ? g.fid : -1, bscore = g.slot >= 0 ? g.score : HMK_JMIN;
             s_best = best;
             HMK_CHECK(sp >= 1 && sp <= n && nr < n && ts >= 0 && ts < n);
             if (bscore < C.T) {                                           // :85-91
                 sp--;
                 C.ready[nr++] = top;
-                set_remove(top);
+                hmk_cl_set_remove(C, top);
+                nactive--;
                 C.id_of[ts] = -1;
                 s_action = 0;
             } else if (sp > 1 && C.stack[sp - 2] == best) {               // :95-109
@@ -2514,71 +2614,185 @@ __global__ void __launch_bounds__(HMK_CL_THREADS) hmk_clinkage_chain(const HmkCl
                 C.D[(size_t)k * n + ts] = m;
             }
             if (tid == 0) {
-                cur_id++;
-                HMK_CHECK(cur_id < 2 * n + 3 && bs >= 0 && bs < n && bs != ts);
                 sp -= 2;
-                set_remove(top);
-                set_remove(s_best);
-                // new Cluster(top.getSequences() ++ nearest.getSequences(), currentId) (:104-106)
-                C.mnext[C.mtail[ts]] = C.mhead[bs];
-                C.mtail[ts] = C.mtail[bs];
-                C.size_of[ts] = hmk_wadd(C.size_of[ts], C.size_of[bs]);
-                C.id_of[ts] = cur_id; C.id_of[bs] = -1;
-                C.slot_of[cur_id] = ts;
-                set_add(cur_id);
+                hmk_cl_merge(C, top, s_best, ts, bs, cur_id, treeified);
+                nactive--;
             }
         }
         __syncthreads();
     }
-    // ---- the last cluster is ready too (:116); then new ArrayList(readyClusters): bucket order of a table that grew with
-    // the set (capacity 16, doubled whenever the size exceeded 0.75 x capacity)
-    if (tid == 0) {
-        for (int b = 0; b < C.acap; b++)
-            if (C.a_head[b] >= 0) { C.ready[nr++] = C.a_head[b]; break; }
-        // the set as HashMap builds it: append at the bin's tail, double the table (bins split in order) whenever the size
-        // exceeds 0.75 x capacity
-        int rcap = 16, rsize = 0;
-        int32_t* head = C.r_head;                     // two (head, tail) table pairs, used alternately across resizes
-        int32_t* tail = C.r_head + C.rcap_max;
-        int32_t* head2 = C.r_head + 2 * C.rcap_max;
-        int32_t* tail2 = C.r_head + 3 * C.rcap_max;
-        for (int b = 0; b < rcap; b++) { head[b] = -1; tail[b] = -1; }
-        for (int i = 0; i < nr; i++) {
-            const int32_t id = C.ready[i];
-            const int b = (int)(hmk_cluster_hash(id) & (uint32_t)(rcap - 1));
-            int len = 0;
-            for (int32_t k = head[b]; k >= 0; k = C.r_next[k]) len++;
-            if (len >= 7) treeified = 1;
-            C.r_next[id] = -1;
-            if (tail[b] >= 0) C.r_next[tail[b]] = id; else head[b] = id;
-            tail[b] = id;
-            if (++rsize > (int)(rcap * 0.75f)) {
-                const int ncap = rcap * 2;
-                HMK_CHECK(ncap <= C.rcap_max);
-                for (int b2 = 0; b2 < ncap; b2++) { head2[b2] = -1; tail2[b2] = -1; }
-                for (int b2 = 0; b2 < rcap; b2++)
-                    for (int32_t k = head[b2], nx; k >= 0; k = nx) {
-                        nx = C.r_next[k];
-                        const int nb = (int)(hmk_cluster_hash(k) & (uint32_t)(ncap - 1));
-                        C.r_next[k] = -1;
-                        if (tail2[nb] >= 0) C.r_next[tail2[nb]] = k; else head2[nb] = k;
-                        tail2[nb] = k;
-                    }
-                int32_t* t1 = head; head = head2; head2 = t1;
-                t1 = tail; tail = tail2; tail2 = t1;
-                rcap = ncap;
+    if (tid == 0) hmk_cl_finish(C, nr, 0, treeified, searches);
+    __syncthreads();
+    hmk_cl_members(C, nr);
+}
+
+// ---- sparse chain: the same state machine on rows of valid entries only (sizes beyond the dense n x n matrix).
+// Exactness: a step either takes a neighbour scoring >= T or declares the top ready, so the arg-max over the valid entries
+// of active clusters is the dense scan's choice whenever it is used.  join's element-wise minimum with
+// min(x, BELOW) == BELOW makes the merged cluster's valid set the INTERSECTION of its parts' sets (scored by the minimum):
+// rows only shrink.  Entries of inactive slots are skipped lazily (a slot never becomes active again); entries that leave
+// an intersection are killed in place (score HMK_JMIN), so rows keep their layout and the twin positions stay valid.
+// Restarts take the head of the lowest non-empty bin from a cursor instead of scanning the acap bins: an add into a lower
+// bin moves it back, and it moves forward over emptied bins when a restart needs it.
+// Block shape: a step costs a few dependent global loads per row pass plus the barriers, so the block is sized from the
+// row lengths by the host (see Engine::clinkage).
+__device__ __forceinline__ int32_t hmk_cl_entry_score(uint64_t v) { return (int32_t)(uint32_t)v; }
+__device__ __forceinline__ int32_t hmk_cl_entry_slot(uint64_t v) { return (int32_t)(v >> 32); }
+
+__global__ void __launch_bounds__(HMK_CL_THREADS, 1) hmk_clinkage_chain_sparse(const HmkClinkage C) {
+    __shared__ int32_t r_score[32], r_size[32], r_id[32];
+    __shared__ int32_t s_top, s_best, s_action, s_ts, s_bs;     // action: 0 ready, 1 merge, 2 push
+    __shared__ int32_t sp, nr, nactive, cur_id, treeified, searches, cursor;
+    const int tid = threadIdx.x;
+    const int n = C.n;
+    const int lowest = hmk_cl_init(C, treeified);
+    if (tid == 0) { sp = 0; nr = 0; nactive = n; cur_id = n + 1; searches = 0; cursor = lowest; }
+    __syncthreads();
+    for (;;) {
+        if (sp == 0 && nactive <= 1) break;           // (uniform: shared variables, read after a barrier)
+        if (tid == 0) {
+            if (sp == 0) {                            // activeClusters.iterator().next() (:62-70)
+                while (C.a_head[cursor] < 0) { cursor++; HMK_CHECK(cursor < C.acap); }
+                C.stack[0] = C.a_head[cursor];
+                sp = 1;
+            }
+            s_top = C.stack[sp - 1]; s_ts = C.slot_of[s_top]; searches++;
+        }
+        __syncthreads();
+        const int32_t top = s_top, ts = s_ts;
+        HMK_CHECK(ts >= 0 && ts < n);
+        const int64_t e0 = C.row_off[ts], e1 = C.row_off[ts + 1];
+        // ---- nearest neighbour of `top` over its valid entries (:75-82)
+        HmkBestCluster bb;
+        bb.score = HMK_JMIN; bb.size = 0; bb.fid = 0; bb.slot = -1;
+        for (int64_t e = e0 + tid; e < e1; e += blockDim.x) {
+            const uint64_t v = C.rows[e];
+            const int32_t sc = hmk_cl_entry_score(v), k = hmk_cl_entry_slot(v);
+            if (sc < C.T) continue;
+            HMK_CHECK(k >= 0 && k < n && k != ts);
+            const int32_t id = C.id_of[k];
+            if (id < 0) continue;
+            hmk_consider(bb, sc, C.size_of[k], id, k);
+        }
+        const HmkBestCluster g = hmk_cl_block_best(bb, r_score, r_size, r_id);
+        if (tid == 0) {
+            const int32_t best = g.slot >= 0 ? g.fid : -1, bscore = g.slot >= 0 ? g.score : HMK_JMIN;
+            s_best = best;
+            HMK_CHECK(sp >= 1 && sp <= n && nr < n);
+            if (bscore < C.T) {                                           // :85-91
+                sp--;
+                C.ready[nr++] = top;
+                hmk_cl_set_remove(C, top);
+                nactive--;
+                C.id_of[ts] = -1;
+                s_action = 0;
+            } else if (sp > 1 && C.stack[sp - 2] == best) {               // :95-109
+                s_bs = C.slot_of[best];
+                s_action = 1;
+            } else {
+                C.stack[sp++] = best;                                     // :111
+                s_action = 2;
             }
         }
-        int o = 0, multi = 0;
-        for (int b = 0; b < rcap; b++)
-            for (int32_t id = head[b]; id >= 0; id = C.r_next[id]) C.result_order[o++] = id;
-        for (int i = 0; i < nr; i++) { const int s = C.slot_of[C.result_order[i]]; multi += C.mhead[s] != C.mtail[s]; }
-        C.out_scalars[0] = nr; C.out_scalars[1] = multi; C.out_scalars[2] = treeified; C.out_scalars[3] = searches;
+        __syncthreads();
+        if (s_action == 1) {
+            const int32_t bs = s_bs;
+            HMK_CHECK(bs >= 0 && bs < n && bs != ts);
+            const int64_t b0 = C.row_off[bs], b1 = C.row_off[bs + 1];
+            // row(ts) := row(ts) & row(bs), minimum score; the mirror entry in the neighbour's row follows.  Only row(bs)
+            // is searched, and no thread writes it (its entry for ts is not in row(ts) -- no self entries)
+            for (int64_t e = e0 + tid; e < e1; e += blockDim.x) {
+                const uint64_t v = C.rows[e];
+                const int32_t sc = hmk_cl_entry_score(v), k = hmk_cl_entry_slot(v);
+                if (sc < C.T) continue;
+                int32_t m = HMK_JMIN;
+                const bool live = k != bs && C.id_of[k] >= 0;
+                if (live) {
+                    int64_t lo = b0, hi = b1;                             // first entry of row(bs) with slot >= k
+                    while (lo < hi) {
+                        const int64_t mid = (lo + hi) >> 1;
+                        if (hmk_cl_entry_slot(C.rows[mid]) < k) lo = mid + 1; else hi = mid;
+                    }
+                    if (lo < b1) {
+                        const uint64_t w = C.rows[lo];
+                        const int32_t sb = hmk_cl_entry_score(w);
+                        if (hmk_cl_entry_slot(w) == k && sb >= C.T) m = sc < sb ? sc : sb;
+                    }
+                }
+                C.rows[e] = (v & 0xffffffff00000000ull) | (uint32_t)m;
+                if (live) {
+                    const int64_t t = C.row_off[k] + C.twin[e];
+                    HMK_CHECK(t >= C.row_off[k] && t < C.row_off[k + 1] && hmk_cl_entry_slot(C.rows[t]) == ts);
+                    C.rows[t] = ((uint64_t)(uint32_t)ts << 32) | (uint32_t)m;
+                }
+            }
+            if (tid == 0) {
+                sp -= 2;
+                const int b = hmk_cl_merge(C, top, s_best, ts, bs, cur_id, treeified);
+                nactive--;
+                if (b < cursor) cursor = b;
+            }
+        }
+        __syncthreads();
     }
+    if (tid == 0) hmk_cl_finish(C, nr, cursor, treeified, searches);
     __syncthreads();
-    for (int i = tid; i < nr; i += blockDim.x) {
-        const int32_t id = C.result_order[i];
-        int32_t rank = 0;
-        for (int32_t m = C.mhead[C.slot_of[id]]; m >= 0; m = C.mnext[m]) { C.cluster_id[m] = id; C.member_rank[m] = rank++; }
+    hmk_cl_members(C, nr);
+}
+
+// ---- sparse row build (Engine::clinkage): the bulk kernel's EMIT hits of one query batch, upper triangle only
+// (profile index p = query q0 + p, thread-side id > query).  Pass 1 counts the entries per row, pass 2 scatters both
+// directions behind per-row cursors (row order is fixed afterwards by a segmented sort).
+__global__ void hmk_cl_count_hits(const int4* __restrict__ hits, const unsigned int* __restrict__ count, unsigned int cap,
+                                  int32_t q0, int32_t n, unsigned long long* deg) {
+    const unsigned int m = min(*count, cap);
+    for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
+        const int4 h = hits[i];
+        const int32_t q = q0 + h.x;
+        HMK_CHECK(q >= 0 && q < n && h.y >= 0 && h.y < n);
+        if (h.y <= q) continue;
+        atomicAdd(deg + q, 1ull);
+        atomicAdd(deg + h.y, 1ull);
+    }
+}
+
+__global__ void hmk_cl_scatter_hits(const int4* __restrict__ hits, const unsigned int* __restrict__ count, unsigned int cap,
+                                    int32_t q0, int32_t n, const int64_t* __restrict__ row_off, unsigned long long* cur,
+                                    uint64_t* rows) {
+    const unsigned int m = min(*count, cap);
+    for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
+        const int4 h = hits[i];
+        const int32_t q = q0 + h.x;
+        if (h.y <= q) continue;
+        const int64_t pa = row_off[q] + (int64_t)atomicAdd(cur + q, 1ull);
+        const int64_t pb = row_off[h.y] + (int64_t)atomicAdd(cur + h.y, 1ull);
+        HMK_CHECK(pa < row_off[q + 1] && pb < row_off[h.y + 1]);
+        rows[pa] = ((uint64_t)(uint32_t)h.y << 32) | (uint32_t)h.z;
+        rows[pb] = ((uint64_t)(uint32_t)q << 32) | (uint32_t)h.z;
+    }
+}
+
+// rel[i] = row_off[r0 + i] - row_off[r0], i = 0..nr: int32 segment offsets of one sort group
+__global__ void hmk_cl_rel_offsets(const int64_t* __restrict__ row_off, int32_t r0, int32_t nr, int32_t* rel) {
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i <= nr; i += gridDim.x * blockDim.x)
+        rel[i] = (int32_t)(row_off[r0 + i] - row_off[r0]);
+}
+
+// twin[e] = position of e's mirror entry in the neighbour's row (relative to its start): binary search for the row's slot
+// in the neighbour's sorted row.  One warp per row.
+__global__ void hmk_cl_twins(const int64_t* __restrict__ row_off, const uint64_t* __restrict__ rows, int32_t n, int32_t* twin) {
+    const int lane = threadIdx.x & 31;
+    for (int64_t a = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; a < n; a += ((int64_t)gridDim.x * blockDim.x) >> 5) {
+        for (int64_t e = row_off[a] + lane; e < row_off[a + 1]; e += 32) {
+            const int32_t b = (int32_t)(rows[e] >> 32);
+            HMK_CHECK(b >= 0 && b < n && b != a);
+            int64_t lo = row_off[b], hi = row_off[b + 1];
+            while (lo < hi) {
+                const int64_t mid = (lo + hi) >> 1;
+                if ((int32_t)(rows[mid] >> 32) < (int32_t)a) lo = mid + 1; else hi = mid;
+            }
+            HMK_CHECK(lo < row_off[b + 1] && (int32_t)(rows[lo] >> 32) == (int32_t)a);
+            twin[e] = (int32_t)(lo - row_off[b]);
+        }
     }
 }

@@ -631,6 +631,28 @@ class GreedyContext:
         self._L.hmk_get_section_ms(self._h, buf, len(_lib.SECTIONS))
         return {k: float(buf[i]) for i, k in enumerate(_lib.SECTIONS)}
 
+    def clinkage(self, residues, offsets, abundance, matrix, threshold, max_shift, shift_penalty):
+        """hmk_clinkage_run: the exact complete-linkage clustering of clinkage_cluster_arrays on this context, so that its
+        options apply and stats() / section_ms() report the call (section slots 0, 1, 2 = scoring, sparse row build,
+        chain) -> (status, GreedyResult | None, message).  Replaces the uploaded sequences."""
+        residues = np.ascontiguousarray(residues, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int32)
+        abundance = np.ascontiguousarray(abundance, dtype=np.int32)
+        matrix = np.ascontiguousarray(matrix, dtype=np.int32).reshape(-1)
+        self._keep = (residues, offsets, abundance, matrix)
+        n = self.n = len(abundance)
+        cid = np.empty(max(n, 1), dtype=np.int32)
+        rank = np.empty(max(n, 1), dtype=np.int32)
+        order = np.empty(max(n, 1), dtype=np.int32)
+        gin = _lib.GreedyIn(n, _ptr(residues, C.c_uint8), _ptr(offsets, C.c_int32), _ptr(abundance, C.c_int32),
+                            _ptr(matrix, C.c_int32), int(threshold), int(max_shift), int(shift_penalty), 0)
+        out = _lib.GreedyOut(_ptr(cid, C.c_int32), _ptr(rank, C.c_int32), _ptr(order, C.c_int32), 0, 0, -1)
+        err = C.create_string_buffer(512)
+        rc = self._L.hmk_clinkage_run(self._h, C.byref(gin), C.byref(out), err, 512)
+        if rc:
+            return rc, None, err.value
+        return 0, GreedyResult(cid[:n], rank[:n], order[:out.n_result].copy(), int(out.n_multi), self.stats()), b""
+
     def score_block(self, first_ids, second_ids) -> np.ndarray:
         """scores[a, b] = ShiftedScorer.sequenceScore(seq1 = first_ids[a], seq2 = second_ids[b])."""
         f = np.ascontiguousarray(first_ids, dtype=np.int32)
@@ -760,7 +782,8 @@ class LimitedGreedySequenceClusterer:
 
 
 class UnsupportedInput(HammockException):
-    """hmk_clinkage_cluster: asymmetric matrix, too many sequences, or a treeified java.util.HashMap bin"""
+    """hmk_clinkage_cluster: asymmetric matrix, valid pairs beyond the free device memory, or a treeified java.util.HashMap
+    bin"""
 
 
 class ClinkageSequenceClusterer:

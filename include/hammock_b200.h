@@ -37,7 +37,7 @@ extern "C" {
 #define HMK_STATUS_BAD_RESIDUE 3   /* residue code >= 24                  UniqueSequence.java:51-54 */
 #define HMK_STATUS_CUDA 4          /* CUDA / NCCL failure (no CPU fallback) */
 #define HMK_STATUS_BAD_ARG 5
-#define HMK_STATUS_UNSUPPORTED 6   /* hmk_clinkage_cluster only, see there */
+#define HMK_STATUS_UNSUPPORTED 6   /* hmk_clinkage_cluster / hmk_clinkage_run only, see there */
 
 typedef struct {
     int32_t n;                /* sequences, ALREADY in clustering order                              */
@@ -112,10 +112,20 @@ int hmk_greedy_cluster_multi(const hmk_greedy_in* in, hmk_greedy_out* out, const
  * singletons, n + 2, n + 3, ... for merged clusters, in merge order), member_rank[i] = position in getSequences(),
  * result_order[0 .. n_result) = the ids of the returned list IN ITS ORDER, n_multi = clusters with more than one member.
  * The chain start and the order of the returned list come from java.util.HashSet iteration; they are reproduced for the
- * OpenJDK 8+ HashMap.  HMK_STATUS_UNSUPPORTED: asymmetric matrix (the reference's cached scores then depend on the thread
- * schedule), more than 32768 sequences, or a hash bin that the JDK would turn into a tree.  An empty input (the reference
+ * OpenJDK 8+ HashMap.  Any n: up to 32768 sequences (option clinkage_dense_max) the scores are kept as a dense n x n
+ * matrix, above that only the pairs scoring >= threshold are kept, as sparse rows in device memory (12 bytes per pair and
+ * direction); both give the same result.  HMK_STATUS_UNSUPPORTED: asymmetric matrix (the reference's cached scores then
+ * depend on the thread schedule), sparse rows that do not fit in the free device memory (errbuf then names the number of
+ * valid pairs and the bytes needed), or a hash bin that the JDK would turn into a tree.  An empty input (the reference
  * throws NoSuchElementException) returns HMK_STATUS_BAD_ARG. */
 int hmk_clinkage_cluster(const hmk_greedy_in* in, hmk_greedy_out* out, int device, char* errbuf, size_t errlen);
+/* hmk_clinkage_cluster on the caller's context: its options apply, and hmk_get_stats / hmk_get_section_ms report the call.
+ * Fields hmk_stats holds afterwards: bulk_pairs (pair scores executed; the sparse path scores the upper triangle twice,
+ * once to count and once to fill the rows), p1_steps (nearest-neighbour searches), total_ms = phase1_ms (device time of
+ * the call), bulk_kernel_ms (with option profile), bulk_launches, total_launches, fast_path, lane_bits; sparse path only:
+ * xhits_kept (directed valid pairs = entries of the rows) and xhits_capacity (entries the row storage holds).  The other
+ * fields are 0.  The context's uploaded sequences are replaced by `in`. */
+int hmk_clinkage_run(hmk_ctx* ctx, const hmk_greedy_in* in, hmk_greedy_out* out, char* errbuf, size_t errlen);
 /* Frees the contexts the two calls above keep.  Call it before the process unloads CUDA if the memory
  * matters; the library never tears them down from a static destructor. */
 void hmk_release_cached(void);
@@ -147,7 +157,10 @@ int hmk_timer_end(hmk_ctx* ctx, double* ms);
 int hmk_measure_peaks(hmk_ctx* ctx, double* out4, char* errbuf, size_t errlen);
 /* device time per section of the last run (only filled when option "profile" is 1):
  * p1_select, p1_partner, p1_cluster, p1_intra, p1_resolve, p2_setup, p2_filter, p2_check, p2_sort,
- * p2_base, p2_iterate, p2_commit, final */
+ * p2_base, p2_iterate, p2_commit, final
+ * After hmk_clinkage_run the first three slots hold the stages of the complete-linkage call instead: [0] scoring (dense:
+ * the n x n matrix; sparse: the counting pass), [1] sparse row build (the filling pass, row sort and twin index; 0 on the
+ * dense path), [2] nearest-neighbour chain; the others are 0. */
 #define HMK_NSECTIONS 13
 int hmk_get_section_ms(hmk_ctx* ctx, double* out, int n);
 /* tuning knobs; unknown names and out-of-range values return HMK_STATUS_BAD_ARG.  None of them changes the result.
@@ -168,6 +181,10 @@ int hmk_get_section_ms(hmk_ctx* ctx, double* out, int n);
  *   xhit_cap   entries of the buffer that keeps the phase-1 hits for phase 2 (0 = automatic: what the last run on this
  *              context needed, else 96 per sequence); an overflow is reported in hmk_stats.flags
  *   force_generic  1 = scalar kernel for everything (correctness path)
+ *   clinkage_dense_max  complete linkage: largest n that keeps the dense n x n score matrix (0..32768, default 32768);
+ *              larger inputs take the sparse path
+ *   clinkage_threads  complete linkage, sparse path: threads of the chain kernel (0 = automatic from the mean row length,
+ *              else a multiple of 32 up to 1024)
  *   profile    1 = time every bulk launch with CUDA events (hmk_stats.bulk_kernel_ms) */
 int hmk_set_option(hmk_ctx* ctx, const char* name, int64_t value);
 
