@@ -175,6 +175,8 @@ struct HmkCtl {
     int32_t steps, joins, creates, orphans;
     int32_t restarts;
     int32_t pad0, pad1;
+    int32_t discards;      // resolver exits that threw the prepared batches away (any status but CONTINUE / GROWHITS)
+    int32_t pad2;
     int64_t scalar_pairs;  // pair scores computed one at a time (resolvers, member checks)
     int64_t scalar_cells;
     int64_t dbg[8];        // resolver cycle counters (only filled when built with -DHMK_RESOLVE_TIMING)

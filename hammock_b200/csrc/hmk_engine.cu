@@ -194,7 +194,10 @@ public:
         CK(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
         CK(cudaStreamCreateWithPriority(&st_, cudaStreamNonBlocking, prio_hi));    // resolvers, small kernels
         CK(cudaStreamCreateWithPriority(&st2_, cudaStreamNonBlocking, prio_lo));   // look-ahead partner search
+        CK(cudaStreamCreateWithPriority(&st3_, cudaStreamNonBlocking, prio_hi));   // look-ahead tails (small kernels)
         for (auto& b : bb_) CK(cudaEventCreateWithFlags(&b.ready, cudaEventDisableTiming));
+        for (auto& b : bb_) CK(cudaEventCreateWithFlags(&b.searched, cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&part1_ev_, cudaEventDisableTiming));
         for (auto& a : aux_) CK(cudaStreamCreateWithPriority(&a, cudaStreamNonBlocking, prio_lo));
         CK(cudaEventCreateWithFlags(&fork_ev_, cudaEventDisableTiming));
         for (auto& e : join_ev_) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -220,9 +223,12 @@ public:
         if (h_p2flags_) cudaFreeHost(h_p2flags_);
         if (comm_) NcclApi::get().CommDestroy(comm_);
         for (auto& b : bb_) if (b.ready) cudaEventDestroy(b.ready);
+        for (auto& b : bb_) if (b.searched) cudaEventDestroy(b.searched);
+        if (part1_ev_) cudaEventDestroy(part1_ev_);
         for (auto& e : join_ev_) if (e) cudaEventDestroy(e);
         if (fork_ev_) cudaEventDestroy(fork_ev_);
         for (auto& a : aux_) if (a) cudaStreamDestroy(a);
+        if (st3_) cudaStreamDestroy(st3_);
         if (st2_) cudaStreamDestroy(st2_);
         if (st_) cudaStreamDestroy(st_);
     }
@@ -291,8 +297,8 @@ private:
     HmkCtl* h_ctl_ = nullptr;
     int32_t* h_scalars_ = nullptr;
     int32_t* h_p2flags_ = nullptr;
-    // ---- phase-1 per-batch buffers, double buffered: while batch i is resolved on the main stream the
-    // partner search of batch i+1 already runs on the side stream
+    // ---- phase-1 per-batch buffers, a ring: while batch i is resolved on the main stream the partner searches of
+    // batches i+1 and i+2 already run on the side stream, and their tails (merge, dense tables, masks) on the tail stream
     struct BatchBuf {
         DevBuf<int32_t> qid, gqid, nq_dev, tk_cnt, tk_ovf, bk_cnt, bk_ovf, gk_cnt, gk_ovf;
         DevBuf<uint64_t> tk_key, bk_key, gk_key;
@@ -311,16 +317,24 @@ private:
         // their scores against every batch query
         DevBuf<int32_t> ib, pcand, pd;
         DevBuf<uint32_t> ibm, ibm2;
-        cudaEvent_t ready = nullptr;
+        cudaEvent_t ready = nullptr;     // everything above is complete
+        cudaEvent_t searched = nullptr;  // the partner search is issued (qid final; the tail starts behind it)
         bool valid = false;      // partner search for the batch starting behind `after` has been issued
         int nq = 0;
         int batch_id = 0;
     };
     BatchBuf bb_[HMK_NBATCHBUF];
-    cudaStream_t st2_ = nullptr;
+    cudaStream_t st2_ = nullptr, st3_ = nullptr;
+    cudaEvent_t part1_ev_ = nullptr;
     cudaStream_t aux_[HMK_NAUX] = {nullptr};
     cudaEvent_t fork_ev_ = nullptr, join_ev_[HMK_NAUX] = {nullptr};
-    void stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32_t* start_after, int ncl_known, cudaStream_t s);
+    void stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32_t* start_after, int ncl_known, cudaStream_t s,
+                              cudaStream_t t);
+    void drain_lookahead() {
+        CK(cudaStreamSynchronize(st2_));
+        CK(cudaStreamSynchronize(st3_));
+        for (auto& b : bb_) b.valid = false;
+    }
     void founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf<int32_t>& sched);
     size_t hit_cap_ = 0;
     // ---- phase-1 scratch
@@ -386,8 +400,8 @@ private:
                          uint32_t* cells = nullptr, uint32_t* ops = nullptr);
     void plan_bulk(HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched = nullptr) const;
     void launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const int32_t* prof_ids, int prof_is_query, cudaStream_t s);
-    void launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int prof_is_query, cudaStream_t s = nullptr,
-                     BatchBuf* bb = nullptr, DevBuf<int32_t>* sched_buf = nullptr);
+    HmkBulkArgs launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int prof_is_query, cudaStream_t s = nullptr,
+                            BatchBuf* bb = nullptr, DevBuf<int32_t>* sched_buf = nullptr);
     cudaEvent_t next_event();
     // per-section device timers (only with opt.profile)
     std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> sections_;
@@ -760,11 +774,11 @@ void Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const
     bulk_launches_++;
 }
 
-// one-launch convenience for everything that is not a (possibly multi-bucket) partner search:
-// the uniform packed kernel when the whole input has one length <= 12, else the generic kernel
-void Engine::launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int prof_is_query, cudaStream_t s, BatchBuf* bb,
-                         DevBuf<int32_t>* sched_buf) {
-    if (a.nq <= 0 || a.ndb <= 0) return;
+// one-launch convenience: the uniform packed kernel when the whole input has one length <= 12, else the generic kernel.
+// Returns the planned arguments (a TOPK launch's per-stripe lists are merged by the caller, with hmk_topk_merge).
+HmkBulkArgs Engine::launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int prof_is_query, cudaStream_t s, BatchBuf* bb,
+                                DevBuf<int32_t>* sched_buf) {
+    if (a.nq <= 0 || a.ndb <= 0) return a;
     if (!s) s = st_;
     const HmkScheme* sch = fast_ ? &sc_ : nullptr;
     DevBuf<int32_t>& sched = sched_buf ? *sched_buf : (bb ? bb->sched : d_sched_);      // launches on different streams overlap: one each
@@ -777,13 +791,7 @@ void Engine::launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int p
         a.stripe_base = 0;
     }
     launch_planned(mode, a, sch, prof_ids, prof_is_query, s);
-    if (mode == HMK_MODE_TOPK) {
-        hmk_topk_merge<<<(a.nq * 32 + 255) / 256, 256, 0, s>>>(a.nq, a.nstripes, (int)opt.kb, bb->tk_key.p, bb->tk_cnt.p,
-                                                               bb->tk_ovf.p, bb->bk_key.p, bb->bk_cnt.p, bb->bk_ovf.p,
-                                                               a.sched ? a.sched + a.nqt : nullptr, a.qt);
-        CK(cudaGetLastError());
-        launches_++;
-    }
+    return a;
 }
 
 int Engine::compact_unassigned(int32_t* out) {
@@ -813,8 +821,6 @@ void Engine::sort_pairs(unsigned long long* keys, int32_t* vals, int n, int begi
 }
 
 // ---------------------------------------------------------------- phase 1
-// select the next batch, build its query profiles and run the partner search (+ the multi-GPU
-// best-hit exchange) on stream `s`; bb.ready fires when the merged lists are in bb.bk_*
 // founder filter of the cluster search for the clusters [from, to): appends (query index, founder id, score) to bb.hits
 void Engine::founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf<int32_t>& sched) {
     if (to <= from) return;
@@ -822,6 +828,7 @@ void Engine::founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf
     a.prof = bb.prof.p; a.nq = bb.nq;
     a.packed = d_packed_.p; a.db_ids = d_cf_.p + from; a.db_begin = 0; a.ndb = to - from;
     a.hits = bb.hits.p; a.hit_count = bb.hcount.p; a.hit_cap = (unsigned int)bb.hit_cap;
+    a.discards = &d_ctl_.p->discards; a.discards_seen = h_ctl_->discards;
     if (!mixed_ || max_len_ > HMK_MAXL1) { launch_bulk(HMK_MODE_EMIT, a, bb.qid.p, 1, s, nullptr, &sched); return; }
     // mixed lengths <= 12: the founders are split by length on the device (no host round trip: every bucket is launched
     // for the upper bound `to - from` and reads its real size on the device) and each bucket runs the packed kernel on
@@ -852,7 +859,13 @@ void Engine::founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf
     }
 }
 
-void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32_t* start_after, int ncl_known, cudaStream_t s) {
+// Selects the next batch, builds its query profiles and runs the partner search (+ the multi-GPU best-hit exchange) and
+// part 1 of the cluster search on stream `s`.  The rest of the batch's state-independent work -- merging the per-stripe
+// top-k lists, the intra-batch and partner-candidate score tables and their masks -- runs on stream `t` behind the
+// partner search, so that the next batch's partner search follows this one directly on `s`.  bb.ready fires when both
+// are complete; bb.searched when the query ids are final (the next batch starts behind the last of them).
+void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32_t* start_after, int ncl_known, cudaStream_t s,
+                                  cudaStream_t t) {
     const int kb = (int)opt.kb;
     bb.qid.reserve(HMK_MAXBATCH); bb.nq_dev.reserve(1);
     bb.bk_key.reserve((size_t)HMK_MAXBATCH * kb); bb.bk_cnt.reserve(HMK_MAXBATCH); bb.bk_ovf.reserve(HMK_MAXBATCH);
@@ -873,6 +886,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
     a.nq = nq;
     a.packed = d_packed_.p; a.slot = d_slot_.p; a.q_minid = bb.qid.p;
     a.tierank = identity_rank_ ? nullptr : d_tierank_.p;
+    a.discards = &d_ctl_.p->discards; a.discards_seen = h_ctl_->discards;
     bb.batch_id = ++batch_id_;
     bb.gmin.reserve(HMK_MAXBATCH);
     CK(cudaMemsetAsync(bb.gmin.p, 0, sizeof(unsigned long long) * nq, s));
@@ -880,6 +894,11 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
     if (reuse_) {
         a.xhits = d_xhits_.p; a.xhit_count = d_xcount_.p; a.xhit_cap = d_xhits_.cap; a.xbatch = bb.batch_id;
     }
+    // the per-stripe top-k lists of the partner search, merged into bb.bk_* (at world > 1 on `s`: the all-gather below
+    // needs this rank's merged lists, and every NCCL call stays on one stream, in the same order on every rank)
+    int merge_stripes = 0;
+    const int32_t* merge_slots = nullptr;
+    int merge_qt = 1;
     if (!mixed_) {
         if (fast_) launch_profiles(HMK_PROF_QUERY, bb.qid.p, nq, bb.prof.p, sc_, s);
         a.prof = bb.prof.p;
@@ -891,10 +910,10 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
             lo = (int)((int64_t)n_ * rank_ / world_); hi = (int)((int64_t)n_ * (rank_ + 1) / world_);
             a.db_ids = d_lsort_.p + lo; a.db_begin = 0; a.ndb = hi - lo; a.db_min_id = db_from;
         }
-        if (a.ndb > 0) launch_bulk(HMK_MODE_TOPK, a, bb.qid.p, 1, s, &bb);
-        else {
-            CK(cudaMemsetAsync(bb.bk_cnt.p, 0, sizeof(int32_t) * nq, s));
-            CK(cudaMemsetAsync(bb.bk_ovf.p, 0, sizeof(int32_t) * nq, s));
+        if (a.ndb > 0) {
+            const HmkBulkArgs p = launch_bulk(HMK_MODE_TOPK, a, bb.qid.p, 1, s, &bb);
+            merge_stripes = p.nstripes; merge_qt = p.qt;
+            merge_slots = p.sched ? p.sched + p.nqt : nullptr;
         }
     } else {
         // mixed lengths: one packed-kernel launch per length bucket of the later singletons (profiles are
@@ -917,10 +936,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
             total_stripes += p.a.nstripes;
             plans.push_back(p);
         }
-        if (plans.empty()) {
-            CK(cudaMemsetAsync(bb.bk_cnt.p, 0, sizeof(int32_t) * nq, s));
-            CK(cudaMemsetAsync(bb.bk_ovf.p, 0, sizeof(int32_t) * nq, s));
-        } else {
+        if (!plans.empty()) {
             const size_t slots = (size_t)total_stripes * nq;
             bb.tk_key.reserve(slots * kb); bb.tk_cnt.reserve(slots); bb.tk_ovf.reserve(slots);
             // the buckets are independent (own profiles, own output slots): fork them over the auxiliary streams so
@@ -944,13 +960,22 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
                 CK(cudaEventRecord(join_ev_[j], aux_[j]));
                 CK(cudaStreamWaitEvent(s, join_ev_[j], 0));
             }
-            hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, s>>>(nq, total_stripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
-                                                                 bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p);
-            CK(cudaGetLastError());
-            launches_++;
+            merge_stripes = total_stripes;
         }
     }
+    if (merge_stripes == 0) {
+        CK(cudaMemsetAsync(bb.bk_cnt.p, 0, sizeof(int32_t) * nq, s));
+        CK(cudaMemsetAsync(bb.bk_ovf.p, 0, sizeof(int32_t) * nq, s));
+    }
+    auto merge_stripe_lists = [&](cudaStream_t ms) {
+        if (merge_stripes == 0) return;
+        hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, ms>>>(nq, merge_stripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
+                                                              bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p, merge_slots, merge_qt);
+        CK(cudaGetLastError());
+        launches_++;
+    };
     if (world_ > 1) {
+        merge_stripe_lists(s);
         // best-hit exchange: every rank contributes its stripe's top-k per query (a few KB),
         // then every rank merges the same lists -> identical, replicated decisions
         bb.gk_key.reserve((size_t)world_ * nq * kb); bb.gk_cnt.reserve((size_t)world_ * nq); bb.gk_ovf.reserve((size_t)world_ * nq);
@@ -959,10 +984,17 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
         allgather(bb.bk_cnt.p, bb.gk_cnt.p, sizeof(int32_t) * nq, s);
         allgather(bb.bk_ovf.p, bb.gk_ovf.p, sizeof(int32_t) * nq, s);
         NK(NcclApi::get().GroupEnd());
-        hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, s>>>(nq, world_, kb, bb.gk_key.p, bb.gk_cnt.p, bb.gk_ovf.p,
+    }
+    // ---- tail, on `t`
+    CK(cudaEventRecord(bb.searched, s));
+    if (t != s) CK(cudaStreamWaitEvent(t, bb.searched, 0));
+    if (world_ > 1) {
+        hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, t>>>(nq, world_, kb, bb.gk_key.p, bb.gk_cnt.p, bb.gk_ovf.p,
                                                              bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p);
         CK(cudaGetLastError());
         launches_++;
+    } else {
+        merge_stripe_lists(t);
     }
     // intra-batch scores S(member = q_b2, query = q_b); row strides padded to 16 bytes for the TMA row prefetch
     const int ib_stride = (nq + 3) & ~3, pd_stride = (nq * kb + 3) & ~3, nw = (nq + 31) / 32;
@@ -970,7 +1002,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
     bb.pcand.reserve((size_t)nq * kb); bb.pd.reserve((size_t)nq * (pd_stride + 4));
     const bool dense_packed = mixed_ && fast_scalar_;      // mixed lengths <= 12: one thread per pair on the packed words
     if (dense_packed) {
-        hmk_dense_packed<<<std::min(sm_count_ * 8, (nq * nq + 255) / 256), 256, 0, s>>>(d_packed_.p, bb.qid.p, nq, bb.qid.p, nq, d_M_.p, X_, P_,
+        hmk_dense_packed<<<std::min(sm_count_ * 8, (nq * nq + 255) / 256), 256, 0, t>>>(d_packed_.p, bb.qid.p, nq, bb.qid.p, nq, d_M_.p, X_, P_,
                                                                                        bb.ib.p, ib_stride, d_pairctr_.p);
         launches_++;
     } else {
@@ -978,19 +1010,19 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
         d.prof = bb.prof.p; d.nq = nq;
         d.packed = d_packed_.p; d.db_ids = bb.qid.p; d.db_begin = 0; d.ndb = nq;
         d.dense = bb.ib.p; d.dense_stride = ib_stride;
-        launch_bulk(HMK_MODE_DENSE, d, bb.qid.p, 1, s);
+        launch_bulk(HMK_MODE_DENSE, d, bb.qid.p, 1, t);
     }
-    hmk_ib_mask<<<(nq * nw + 127) / 128, 128, 0, s>>>(nq, nw, T_, bb.ib.p, ib_stride, bb.ibm.p, kb, bb.bk_key.p, bb.bk_cnt.p, bb.ibm2.p);
+    hmk_ib_mask<<<(nq * nw + 127) / 128, 128, 0, t>>>(nq, nw, T_, bb.ib.p, ib_stride, bb.ibm.p, kb, bb.bk_key.p, bb.bk_cnt.p, bb.ibm2.p);
     launches_++;
     // S(partner candidate, query) for every candidate of the batch: clusters born inside the
     // batch have one of these as their second member
     {
         const int npc = nq * kb;
-        hmk_partner_ids<<<(npc + 127) / 128, 128, 0, s>>>(nq, kb, bb.bk_key.p, bb.bk_cnt.p,
+        hmk_partner_ids<<<(npc + 127) / 128, 128, 0, t>>>(nq, kb, bb.bk_key.p, bb.bk_cnt.p,
                                                           identity_rank_ ? nullptr : d_id_of_rank_.p, bb.qid.p, bb.pcand.p);
         launches_++;
         if (dense_packed) {
-            hmk_dense_packed<<<std::min(sm_count_ * 8, (nq * npc + 255) / 256), 256, 0, s>>>(d_packed_.p, bb.qid.p, nq, bb.pcand.p, npc, d_M_.p, X_,
+            hmk_dense_packed<<<std::min(sm_count_ * 8, (nq * npc + 255) / 256), 256, 0, t>>>(d_packed_.p, bb.qid.p, nq, bb.pcand.p, npc, d_M_.p, X_,
                                                                                             P_, bb.pd.p, pd_stride, d_pairctr_.p);
             launches_++;
         } else {
@@ -998,12 +1030,12 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
             d.prof = bb.prof.p; d.nq = nq;
             d.packed = d_packed_.p; d.db_ids = bb.pcand.p; d.db_begin = 0; d.ndb = npc;
             d.dense = bb.pd.p; d.dense_stride = pd_stride;
-            launch_bulk(HMK_MODE_DENSE, d, bb.qid.p, 1, s);
+            launch_bulk(HMK_MODE_DENSE, d, bb.qid.p, 1, t);
         }
     }
     CK(cudaGetLastError());
-    // cluster search, part 1 (state independent as well: founders never change): the clusters that exist now.  The ones
-    // created until the batch is resolved are added on the main stream (phase1)
+    // cluster search, part 1 (state independent as well: founders never change), on `s`: the clusters that exist now.  The
+    // ones created until the batch is resolved are added on the main stream (phase1)
     bb.nq = nq;
     bb.hit_cap = hit_cap_;
     bb.hits.reserve(bb.hit_cap); bb.hcount.reserve(4);
@@ -1011,7 +1043,11 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
     CK(cudaMemsetAsync(bb.hcount.p, 0, 4 * sizeof(unsigned int), s));
     bb.ncl_ahead = ncl_known;
     founder_hits(bb, 0, ncl_known, s, bb.sched2);
-    CK(cudaEventRecord(bb.ready, s));
+    if (t != s) {
+        CK(cudaEventRecord(part1_ev_, s));
+        CK(cudaStreamWaitEvent(t, part1_ev_, 0));
+    }
+    CK(cudaEventRecord(bb.ready, t));
     bb.valid = true;
 }
 
@@ -1055,7 +1091,7 @@ int Engine::phase1() {
         BatchBuf& cb = bb_[head];
         const int cur = h_ctl_->cur, ncl = h_ctl_->ncl;
         sec(SEC_P1_PARTNER);
-        if (!cb.valid) stage_partner_search(cb, std::min(B, h_ctl_->unproc_alive), cur, nullptr, ncl, st_);   // not prepared ahead
+        if (!cb.valid) stage_partner_search(cb, std::min(B, h_ctl_->unproc_alive), cur, nullptr, ncl, st_, st_);   // not prepared ahead
         else CK(cudaStreamWaitEvent(st_, cb.ready, 0));
         const int nq = cb.nq;
         const int32_t* d_qid = cb.qid.p;
@@ -1106,9 +1142,10 @@ int Engine::phase1() {
         CK(cudaGetLastError());
         launches_++;
         // look ahead: the partner searches of the next `depth` batches (and everything else that does not depend on
-        // the clustering state) run on the side stream while this batch is resolved; they are issued right behind
+        // the clustering state) run on the side streams while this batch is resolved; they are issued right behind
         // the resolver so that the resolver's CTA is placed first.  A batch only needs its predecessor's last query
         // id; whatever the batches before it consume in the meantime is filtered by the resolver's consumed set.
+        // A resolver that throws the prepared batches away bumps ctl.discards, and their persistent launches stop.
         sec(SEC_P1_INTRA);   // host time of issuing the look-ahead
         for (int d = 1; d <= depth; d++) {
             BatchBuf& prev = bb_[(head + d - 1) % HMK_NBATCHBUF];
@@ -1116,8 +1153,12 @@ int Engine::phase1() {
             if (nb.valid) continue;
             if (!prev.valid || prev.nq != B || h_ctl_->unproc_alive < nq + (2 + d) * B) break;
             plan_sms_ = sm_count_ - reserve;
-            CK(cudaStreamWaitEvent(st2_, prev.ready, 0));      // prev.qid is written on the stream that staged prev
-            stage_partner_search(nb, B, cur, prev.qid.p + (prev.nq - 1), ncl, st2_);
+            // the tail stream takes the tails of the packed kernels' batches; the generic scalar kernel's dense tables are
+            // long launches that slowed the main stream down at the tail stream's priority (7-30 mixed: 32.1 -> 33.6 ms),
+            // so on that path a batch is staged behind the whole previous one, as on a single side stream
+            const bool tail = fast_ || mixed_;
+            CK(cudaStreamWaitEvent(st2_, tail ? prev.searched : prev.ready, 0));   // prev.qid is written on the stream that staged prev
+            stage_partner_search(nb, B, cur, prev.qid.p + (prev.nq - 1), ncl, st2_, tail ? st3_ : st2_);
             plan_sms_ = 0;
         }
         sec(-1);
@@ -1139,10 +1180,7 @@ int Engine::phase1() {
         }
         stats.p1_batches++;
         cb.valid = false;
-        if (st != HMK_P1_CONTINUE) {     // the prepared batches do not follow this one after all
-            CK(cudaStreamSynchronize(st2_));
-            for (auto& b : bb_) b.valid = false;
-        }
+        if (st != HMK_P1_CONTINUE) drain_lookahead();    // the prepared batches do not follow this one after all
         if (st == HMK_P1_NPE) { error_step = h_ctl_->npe_step; stats.error_step = error_step; return HMK_ERR_NULL_CLUSTER; }
         if (st == HMK_P1_DONE) break;
         if (st == HMK_P1_GROW) {   // a query had more valid clusters than its arrays hold
@@ -1151,8 +1189,7 @@ int Engine::phase1() {
         }
         head = (head + 1) % HMK_NBATCHBUF;
     }
-    CK(cudaStreamSynchronize(st2_));
-    for (auto& b : bb_) b.valid = false;
+    drain_lookahead();      // phase 2 reads d_xcount_, which the look-ahead searches append to
     return HMK_OK;
 }
 

@@ -215,6 +215,10 @@ struct HmkBulkArgs {
     // (CTA x tile engagements) handed out for tile t; nstripes = slots per query in tk_* (>= CTAs)
     int32_t* sched;
     int32_t nchunks;
+    // optional, persistent mode: a phase-1 batch prepared ahead stops taking chunks once the resolver's discard counter
+    // (HmkCtl::discards) differs from the value the host knew when it staged the batch -- its results are thrown away
+    const int32_t* discards;
+    int32_t discards_seen;
     const int32_t* ndb_dev;   // optional: the real number of thread-side items (<= ndb, which then only sizes the grid)
     int32_t db_min_id;        // generic kernel with a length-sorted id list: ids below this are not scored at all
 };
@@ -629,10 +633,13 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
         } else {
             __syncthreads();            // everybody is done with s_next (and with the previous chunk)
             if (threadIdx.x == 0) {
-                int t = home, ch = atomicAdd(a.sched + t, 1);
-                for (int k = 1; ch >= a.nchunks && k < a.nqt; k++) {
-                    t = (home + k) % a.nqt;
-                    ch = __ldcg(a.sched + t) < a.nchunks ? atomicAdd(a.sched + t, 1) : a.nchunks;
+                int t = home, ch = a.nchunks;
+                if (!a.discards || __ldcg(a.discards) == a.discards_seen) {   // else the batch was thrown away: stop
+                    ch = atomicAdd(a.sched + t, 1);
+                    for (int k = 1; ch >= a.nchunks && k < a.nqt; k++) {
+                        t = (home + k) % a.nqt;
+                        ch = __ldcg(a.sched + t) < a.nchunks ? atomicAdd(a.sched + t, 1) : a.nchunks;
+                    }
                 }
                 if (ch >= a.nchunks) t = -1;
                 else if (t != cur_tile) s_next[2] = atomicAdd(a.sched + a.nqt + t, 1);
@@ -1816,6 +1823,7 @@ __global__ void __launch_bounds__(HMK_RESOLVE_THREADS) hmk_p1_resolve_kernel(con
         if (npe_step >= 0) ctl->npe_step = npe_step;
         ctl->steps = steps; ctl->joins = joins; ctl->creates = creates; ctl->orphans = orphans;
         if (status == HMK_P1_RESTART) ctl->restarts += 1;
+        if (status != HMK_P1_CONTINUE) ctl->discards += 1;     // cancels the partner searches prepared behind this batch
     }
 }
 

@@ -19,7 +19,8 @@ def main():
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     env = dict(os.environ, HMK_LIB=lib)
     cmd = [sys.executable, "-m", "pytest", "-m", "gpu", "-q", "-x", "tests/test_gpu_fuzz.py", "tests/test_gpu_boundary.py",
-           "tests/test_clinkage.py", "tests/test_clinkage_large.py", "tests/test_gpu_parity.py"] + sys.argv[1:]
+           "tests/test_clinkage.py", "tests/test_clinkage_large.py", "tests/test_gpu_parity.py",
+           "tests/test_p1_pipeline.py"] + sys.argv[1:]
     with open(os.path.join(ROOT, "gpurun_out", "checked_fuzz.log"), "w") as log:
         log.write("library: " + lib + "\n$ " + " ".join(cmd) + "\n")
         log.flush()
