@@ -617,8 +617,10 @@ int Engine::qt_max(const HmkScheme& sc) const {
     if (opt.qt > 0) return (int)opt.qt;
     const size_t pwb = (size_t)sc.prof_words * 4;
     const size_t per = pwb + (size_t)opt.kb * 8 + 8 + 12;
-    const size_t fixed = 128 + (HMK_BULK_THREADS / 32) * HMK_QCAP * 8 + (sc.filter ? 16 + (HMK_BULK_THREADS / 32) * HMK_CQCAP * 12 : 0);
-    return (int)std::min<size_t>(255, std::max<size_t>(1, (smem_optin_ - fixed) / per));
+    const size_t fixed = 128 + (HMK_BULK_THREADS / 32) * HMK_QCAP * 8;
+    // the filter kernel's tile stays at the 56 profiles the batch size and chunking were measured with (more would fit)
+    const size_t cap = sc.filter ? HMK_FILTER_QT : 255;
+    return (int)std::min<size_t>(cap, std::max<size_t>(1, (smem_optin_ - fixed) / per));
 }
 
 // scheme of a launch whose thread-side sequences all have length n
@@ -752,7 +754,6 @@ void Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const
     if (sch) {
         size_t smem = (((size_t)a.qt * sch->prof_words * 4 + 15) & ~(size_t)15) + 16 +
                       hmk_carve_bytes(a.qt, a.kb, sch->long_layout ? HMK_LONG_THREADS : HMK_BULK_THREADS, false);
-        if (sch->filter) smem += 16 + (size_t)(HMK_BULK_THREADS / 32) * HMK_CQCAP * 12;   // candidate queues
         if (mode == HMK_MODE_TOPK) launch_fast_mode<HMK_MODE_TOPK>(smem_cfg_, a, grid, smem, s);
         else if (mode == HMK_MODE_EMIT) launch_fast_mode<HMK_MODE_EMIT>(smem_cfg_, a, grid, smem, s);
         else launch_fast_mode<HMK_MODE_DENSE>(smem_cfg_, a, grid, smem, s);

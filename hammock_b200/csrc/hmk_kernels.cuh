@@ -25,7 +25,9 @@
 #define HMK_NWMAX 10           // most 32-bit words per profile entry (long kernel)
 #define HMK_LONG_THREADS 512
 #define HMK_FPW 868            // words per profile with the filter sub-table: 3 x 288 + 4 (the +16 B skews the tables over the banks)
-#define HMK_CQCAP 64           // filter kernel: candidate-queue entries per warp
+#define HMK_FILTER_QT 56       // filter kernel: most profiles per tile (Engine::qt_max)
+#define HMK_FGROUP 32          // filter kernel: queries whose filter results one lane keeps as bits before they are handed out
+                               // (four octets of one 32-bit mask per exact word; the kernel relies on 32)
 #ifndef HMK_BULK_THREADS
 #define HMK_BULK_THREADS 768
 #endif
@@ -550,19 +552,49 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_fast(const __gri
     }
 }
 
+// ---------------------------------------------------------------- filter candidates
+// whole warp: lane l holds row l of a 32 x 32 bit matrix (bit c = element (l, c)); returns column `lane`
+// (bit l = element (l, lane)).  Recursive block transpose, one exchange per halving of the block size.
+__device__ __forceinline__ uint32_t hmk_transpose32(uint32_t x, int lane) {
+    const uint32_t keep[5] = {0x0000ffffu, 0x00ff00ffu, 0x0f0f0f0fu, 0x33333333u, 0x55555555u};
+#pragma unroll
+    for (int i = 0, s = 16; i < 5; i++, s >>= 1) {
+        const uint32_t y = __shfl_xor_sync(0xffffffffu, x, s);
+        x = (lane & s) ? ((x & ~keep[i]) | ((y & ~keep[i]) >> s)) : ((x & keep[i]) | ((y & keep[i]) << s));
+    }
+    return x;
+}
+
+// position of the n-th (from 0) set bit of m; n < popc(m)
+__device__ __forceinline__ int hmk_nth_bit(uint32_t m, int n) {
+    int pos = 0;
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        const int c = __popc(m & ((1u << s) - 1u));
+        if (n >= c) { n -= c; m >>= s; pos += s; }
+    }
+    return pos;
+}
+
 // ---------------------------------------------------------------- filter + verify bulk kernel
 // The exact kernel needs 24 shared-memory look-ups per pair and is bound by that pipe.  Here every pair
 // first takes 12 look-ups in a FILTER table whose four u8 lanes bound PAIRS of neighbouring diagonals from
 // above (max of the two exact entries per position); only pairs where some bound reaches the threshold
-// (about 7 % for random 12-mers at T = 20, against 0.3 % real hits) are queued per warp and re-scored
-// exactly, 32 candidates at a time, one per lane.  No false negatives (sum of maxima >= each sum), exact
-// scores for everything that is reported.  u8 lanes, two exact words, lengths <= 12.
+// (about 4 % for the synthetic 12-mers at T = 20, against 0.3 % real hits) are re-scored exactly, 32
+// candidates at a time, one per lane.  No false negatives (sum of maxima >= each sum), exact scores for
+// everything that is reported.  u8 lanes, two exact words, lengths <= 12.
+// Candidates never go through shared memory: a lane keeps, for HMK_FGROUP queries, one bit per (query, half)
+// that passed for its own item.  At the end of the group the warp lists them query-major (lane minor) and
+// hands them out into a round of 32 held in registers, one candidate per lane, fetching the item's packed
+// word from the owning lane by shuffle; a part-filled round is carried into the next group and is verified
+// when it is full or when the chunk ends.
 // LT: compile-time length (0 = use sc.L; then the twelve look-ups are predicated, which costs issue slots)
 template <int MODE, int LT>
 __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __grid_constant__ HmkBulkArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr uint32_t PWB = HMK_FPW * 4;
     constexpr uint32_t SUB = HMK_MAXL1 * HMK_ROWB;   // bytes of one sub-table
+    constexpr int OCT_UNROLL = LT ? 2 : 1;
     __shared__ int s_next[3];                         // persistent mode: (tile, chunk, output slot) of the next piece of work
     const int L = LT ? LT : a.sc.L;
     size_t o = ((size_t)a.qt * PWB + 15) & ~(size_t)15;
@@ -571,12 +603,6 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
     HmkTopkSmem tk;
     HmkHitQueue hq;
     hmk_carve(smem_raw + o, a.qt, a.kb, false, tk, hq);
-    o += hmk_carve_bytes(a.qt, a.kb, HMK_BULK_THREADS, false);
-    // candidate queue of this warp: packed word of the database item + entry word (see verify)
-    uint64_t* cqw = reinterpret_cast<uint64_t*>(smem_raw + ((o + 15) & ~(size_t)15)) + (threadIdx.x >> 5) * HMK_CQCAP;
-    uint32_t* cq = reinterpret_cast<uint32_t*>(smem_raw + ((o + 15) & ~(size_t)15) + (size_t)(HMK_BULK_THREADS / 32) * HMK_CQCAP * 8) +
-                   (threadIdx.x >> 5) * HMK_CQCAP;
-    int ccnt = 0;   // warp-uniform
 
     if (threadIdx.x == 0) hmk_mbar_init(bar, 1);
     __syncthreads();
@@ -585,24 +611,28 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
     const int32_t dec = a.sc.T - a.sc.half;
     const unsigned char* sbase = smem_raw;
     const int lane = threadIdx.x & 31;
-    const unsigned ltmask = (1u << lane) - 1u;
     const bool persistent = a.sched != nullptr;
     int cur_tile = -1, slot = 0, q0 = 0, qn = 0, home = blockIdx.x % a.nqt;
     uint32_t bar_phase = 0;
     int i_begin = 0, i_end = 0;
 
-    // exact re-scoring of up to 32 queued candidates, one per lane.  entry: bits 24..31 = t, bit 7 / bit 23 =
-    // "a filter byte of exact word 0 / word 1 passed", the other 22 bits = offset in the chunk.  Only the
-    // exact word(s) whose filter bytes passed are summed (both: rare, handled in a divergent tail)
+    // the round: lanes below rfill hold a candidate -- the item's packed word rw and the entry re: bits 24..31 =
+    // tile-local query, bit 22 / bit 23 = "a filter byte of exact word 0 / word 1 passed", the low 22 bits = the
+    // item's offset in the chunk.  Free lanes keep rw = 0 and re = bit 22, so their look-ups hit the row everybody
+    // else reads in profile 0.
+    int rfill = 0;   // warp-uniform
+    uint32_t re = 1u << 22;
+    uint64_t rw = 0ull;
+
+    // exact re-scoring of the round.  Only the exact word(s) whose filter bytes passed are summed (both: rare,
+    // handled in a divergent tail)
     auto verify = [&]() {
-        const int n = ccnt < 32 ? ccnt : 32, base = ccnt - n;
-        const bool have = lane < n;
-        const uint32_t ent = have ? cq[base + lane] : 0u;
-        const int t = (int)(ent >> 24);
-        const uint32_t halves = ((ent >> 7) & 1u) | ((ent >> 22) & 2u);
-        const int32_t i = i_begin + (int32_t)((ent & 0x7fu) | ((ent & 0x7fff00u) >> 1));
+        const bool have = lane < rfill;
+        const int t = (int)(re >> 24);
+        const uint32_t halves = (re >> 22) & 3u;
+        const int32_t i = i_begin + (int32_t)(re & 0x3fffffu);
         HMK_CHECK(!have || (t < qn && i >= i_begin && i < i_end && halves != 0u));
-        const uint64_t w = have ? cqw[base + lane] : 0ull;
+        const uint64_t w = rw;
         const unsigned char* pb = sbase + (uint32_t)t * PWB + ((halves & 1u) ? 0u : SUB);
         uint32_t acc0 = 0, acc1 = 0;
 #pragma unroll
@@ -615,7 +645,7 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
         }
         __syncwarp();
         const bool hit = have && ((acc0 | acc1) & 0x80808080u) != 0;
-        ccnt = base;
+        rfill = 0; re = 1u << 22; rw = 0ull;
         const uint32_t mx = __vmaxu4(acc0, acc1);
         const uint32_t m2 = __vmaxu4(mx, mx >> 16);
         const uint32_t m1 = (m2 & 0xffu) > ((m2 >> 8) & 0xffu) ? (m2 & 0xffu) : ((m2 >> 8) & 0xffu);
@@ -651,8 +681,8 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
             HMK_CHECK(tile < a.nqt && chunk_idx >= 0 && chunk_idx < a.nchunks);
         }
         if (tile != cur_tile) {
-            if (cur_tile >= 0) {        // leave the previous tile: everything queued belongs to it
-                while (ccnt > 0) verify();
+            if (cur_tile >= 0) {        // leave the previous tile: the round was verified at the end of the chunk
+                HMK_CHECK(rfill == 0);
                 if (hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
                 if (MODE == HMK_MODE_TOPK) { __syncthreads(); hmk_topk_flush(a, tk, q0, qn, slot); }
                 __syncthreads();
@@ -689,13 +719,8 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
             if (valid && a.slot && a.slot[id] >= 0) valid = false;
             if (!__any_sync(0xffffffffu, valid)) continue;
             const uint64_t w = valid ? a.packed[id] : 0ull;
-            const unsigned char* rowp[HMK_MAXL1];   // &filter[0][j][residue_j]
-#pragma unroll
-            for (int j = 0; j < HMK_MAXL1; j++)
-                rowp[j] = sbase + 2 * SUB + j * HMK_ROWB + (uint32_t)((w >> (5 * j)) & 31u) * 4u;
+            const unsigned char* rowp[HMK_MAXL1];   // &filter[t][j][residue_j]
             if (valid) scored += qn;
-            const uint32_t ilocal = (uint32_t)(i - i_begin);
-            uint32_t tI = (ilocal & 0x7fu) | ((ilocal >> 7) << 8);
 
             auto bound = [&](const int tu) -> uint32_t {
                 uint32_t f = 0;
@@ -704,40 +729,96 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
                     if (j < L) f += *reinterpret_cast<const uint32_t*>(rowp[j] + tu * PWB);
                 return f;
             };
-            auto enqueue = [&](const uint32_t tu, const uint32_t f) {
-                // lanes without an item look up residue 0 (same row as everybody else: no bank conflict) and are masked here
-                const uint32_t top = valid ? f & 0x80808080u : 0u;
-                const unsigned m = __ballot_sync(0xffffffffu, top != 0);
-                if (m) {
-                    if (top) {
-                        const int sl = ccnt + __popc(m & ltmask);
-                        HMK_CHECK(sl >= 0 && sl < HMK_CQCAP && ilocal < (1u << 22) && (tI >> 24) + tu < 256u);
-                        cq[sl] = (tI + (tu << 24)) | ((top | (top >> 8)) & 0x00800080u);
-                        cqw[sl] = w;
+            // bit k of m0 / m1: a filter byte of exact word 0 / word 1 passed against query g0 + k.  They are built an
+            // octet of queries at a time: x = (x >> 1) | (f & 0x80808080) over c <= 8 queries leaves query q's top bit
+            // of filter byte b at bit 8b + q + 8 - c (two instructions per query; no bit crosses into the byte below
+            // before the eighth shift), and `octet` moves the bytes of the two exact words into the top of m0 / m1
+            uint32_t m0 = 0, m1 = 0;
+            auto octet = [&](uint32_t x, const int c) {
+                x >>= 8 - c;
+                const uint32_t y = x | (x >> 8);            // byte 0: exact word 0, byte 2: exact word 1
+                m0 = __funnelshift_r(m0, y, 8);
+                m1 = __funnelshift_r(m1, y >> 16, 8);
+            };
+            // hand the group's candidates out into the round, query-major with the lane as the minor key
+            auto resolve = [&](const int g0) {
+                // lanes without an item looked up residue 0 (same row as everybody else: no bank conflict); drop them here
+                const uint32_t pm = valid ? (m0 | m1) : 0u;
+                if (!__any_sync(0xffffffffu, pm != 0u)) return;
+                const uint32_t col = hmk_transpose32(pm, lane);   // lanes with a candidate against query g0 + lane
+                const int cnt = __popc(col);
+                int incl = cnt;                                    // candidates of queries g0 .. g0 + lane
+#pragma unroll
+                for (int s = 1; s < 32; s <<= 1) {
+                    const int v = __shfl_up_sync(0xffffffffu, incl, s);
+                    if (lane >= s) incl += v;
+                }
+                const int n = __shfl_sync(0xffffffffu, incl, 31);
+                for (int base = 0; base < n;) {
+                    const int take = min(32 - rfill, n - base);
+                    const int g = base + lane - rfill;            // this lane's candidate in the group's list
+                    const int gq = min(max(g, 0), n - 1);
+                    int k = 0;                                     // its query: the first k with incl[k] > gq
+#pragma unroll
+                    for (int s = 16; s > 0; s >>= 1)
+                        if (__shfl_sync(0xffffffffu, incl, k + s - 1) <= gq) k += s;
+                    const uint32_t ck = __shfl_sync(0xffffffffu, col, k);
+                    const int first = __shfl_sync(0xffffffffu, incl - cnt, k);
+                    const int src = hmk_nth_bit(ck, gq - first); // the lane that owns the item
+                    const uint64_t ws = __shfl_sync(0xffffffffu, w, src);
+                    const uint32_t h = (__shfl_sync(0xffffffffu, m0, src) >> k & 1u) |
+                                       (__shfl_sync(0xffffffffu, m1, src) >> k & 1u) << 1;
+                    if (lane >= rfill && g < base + take) {
+                        HMK_CHECK(k < HMK_FGROUP && g0 + k < qn && src >= 0 && src < 32 && (ck >> src & 1u) && h != 0u &&
+                                  ib + src - i_begin < (1 << 22));
+                        re = (uint32_t)(g0 + k) << 24 | h << 22 | (uint32_t)(ib + src - i_begin);
+                        rw = ws;
                     }
-                    ccnt += __popc(m);
-                    __syncwarp();
-                    if (ccnt >= 32) verify();
+                    rfill += take;
+                    base += take;
+                    if (rfill == 32) verify();
                 }
             };
 
             int t = 0;
-            for (; t + 4 <= qn; t += 4) {
-                const uint32_t f0 = bound(0), f1 = bound(1), f2 = bound(2), f3 = bound(3);
-                enqueue(0, f0); enqueue(1, f1); enqueue(2, f2); enqueue(3, f3);
-                tI += 4u << 24;
+            for (int g0 = 0; g0 < qn; g0 += HMK_FGROUP) {
+                const int gend = min(qn, g0 + HMK_FGROUP);
+                // set up per group, so that the pointers are not live while the group's candidates are handed out
 #pragma unroll
-                for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += 4 * PWB;
-            }
-            for (; t < qn; t++) {
-                const uint32_t f0 = bound(0);
-                enqueue(0, f0);
-                tI += 1u << 24;
+                for (int j = 0; j < HMK_MAXL1; j++)
+                    rowp[j] = sbase + (uint32_t)g0 * PWB + 2 * SUB + j * HMK_ROWB + (uint32_t)((w >> (5 * j)) & 31u) * 4u;
+                for (; t + 8 <= gend; t += 8) {
+                    uint32_t x = 0;
+                    // two blocks of four queries; unrolled only at a fixed length, where the predicate-free look-ups
+                    // leave the registers for it (the general-length build would spill)
+#pragma unroll OCT_UNROLL
+                    for (int u = 0; u < 2; u++) {
+                        const uint32_t f0 = bound(0), f1 = bound(1), f2 = bound(2), f3 = bound(3);
+                        x = (x >> 1) | (f0 & 0x80808080u); x = (x >> 1) | (f1 & 0x80808080u);
+                        x = (x >> 1) | (f2 & 0x80808080u); x = (x >> 1) | (f3 & 0x80808080u);
 #pragma unroll
-                for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += PWB;
+                        for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += 4 * PWB;
+                    }
+                    octet(x, 8);
+                }
+                if (t < gend) {                             // last, part-filled octet of the group
+                    const int c = gend - t;
+                    uint32_t x = 0;
+                    for (; t < gend; t++) {
+                        x = (x >> 1) | (bound(0) & 0x80808080u);
+#pragma unroll
+                        for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += PWB;
+                    }
+                    octet(x, c);
+                }
+                const int octets = (gend - g0 + 7) >> 3;     // the first octet sits in the lowest byte
+                m0 >>= 8 * (4 - octets);
+                m1 >>= 8 * (4 - octets);
+                resolve(g0);
+                m0 = 0; m1 = 0;
             }
         }
-        while (ccnt > 0) verify();      // the queued offsets are relative to this chunk
+        if (rfill) verify();      // the round must be empty before the tile (and with it q0) can change
     }
     if (cur_tile >= 0 && qn > 0) {
         if (hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
