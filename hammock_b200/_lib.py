@@ -43,7 +43,7 @@ class Stats(C.Structure):
 
 
 EXPORTS = ["hmk_abi_version", "hmk_greedy_cluster", "hmk_greedy_cluster_multi", "hmk_clinkage_cluster", "hmk_clinkage_run", "hmk_create", "hmk_destroy", "hmk_upload", "hmk_run",
-           "hmk_download", "hmk_get_stats", "hmk_get_section_ms", "hmk_set_option", "hmk_score_block",
+           "hmk_download", "hmk_get_stats", "hmk_get_section_ms", "hmk_set_option", "hmk_score_block", "hmk_bulk_probe",
            "hmk_timer_begin", "hmk_timer_end", "hmk_measure_peaks", "hmk_nccl_unique_id", "hmk_init_distributed", "hmk_release_cached"]
 SECTIONS = ["p1_select", "p1_partner", "p1_cluster", "p1_intra", "p1_resolve", "p2_setup", "p2_filter", "p2_check",
             "p2_sort", "p2_base", "p2_iterate", "p2_commit", "final"]
@@ -102,5 +102,8 @@ def load():
     L.hmk_set_option.argtypes = [vp, cp, C.c_int64]
     L.hmk_score_block.restype = C.c_int
     L.hmk_score_block.argtypes = [vp, i32p, C.c_int32, i32p, C.c_int32, i32p, cp, sz]
+    L.hmk_bulk_probe.restype = C.c_int
+    L.hmk_bulk_probe.argtypes = [vp, C.c_int32, i32p, C.c_int32, i32p, C.c_int32, C.c_int32, C.POINTER(C.c_uint8),
+                                 C.POINTER(C.c_uint64), i32p, i32p, i32p, C.c_int64, C.POINTER(C.c_int64), i32p, cp, sz]
     _lib = L
     return L

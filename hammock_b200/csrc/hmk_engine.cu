@@ -239,6 +239,9 @@ public:
     int run();
     void download(hmk_greedy_out* out);
     void score_block(const int32_t* first, int32_t nf, const int32_t* second, int32_t ns, int32_t* scores);
+    void bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t* db_ids, int32_t db_begin, int32_t ndb,
+                    const uint8_t* clustered, uint64_t* keys, int32_t* cnt, int32_t* ovf, int32_t* hits, int64_t hit_cap,
+                    int64_t* hit_count, int32_t* kernel);
     int clinkage(const hmk_greedy_in* in, hmk_greedy_out* out);
     std::string status_msg;      // details of the last non-zero status, when there are any
     hmk_stats stats{};
@@ -1610,6 +1613,104 @@ void Engine::score_block(const int32_t* first, int32_t nf, const int32_t* second
     }
 }
 
+// One bulk launch with the context's scheme and options, for the kernel tests (hmk_bulk_probe).  Mode 0 is the partner
+// search of stage_partner_search's uniform-length branch: only ids > qids[t] qualify, the per-stripe lists are merged
+// with hmk_topk_merge and every qualifying hit is kept.  Mode 1 emits every hit.
+void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t* db_ids, int32_t db_begin, int32_t ndb,
+                        const uint8_t* clustered, uint64_t* keys, int32_t* cnt, int32_t* ovf, int32_t* hits, int64_t hit_cap,
+                        int64_t* hit_count, int32_t* kernel) {
+    CK(cudaSetDevice(device_));
+    if (!uploaded_) throw std::invalid_argument("hmk_bulk_probe before hmk_upload");
+    if ((mode != 0 && mode != 1) || nq < 0 || ndb < 0 || hit_cap < 0 || (nq && !qids) || (nq && mode == 0 && (!keys || !cnt || !ovf)) ||
+        (hit_cap && !hits) || !hit_count || !kernel)
+        throw std::invalid_argument("hmk_bulk_probe: bad argument");
+    for (int32_t t = 0; t < nq; t++)
+        if (qids[t] < 0 || qids[t] >= n_) throw std::invalid_argument("hmk_bulk_probe: query id out of range");
+    for (int32_t i = 0; i < ndb; i++) {
+        const int64_t id = db_ids ? db_ids[i] : (int64_t)db_begin + i;
+        if (id < 0 || id >= n_) throw std::invalid_argument("hmk_bulk_probe: thread-side id out of range");
+    }
+    const int kb = (int)opt.kb;
+    DevBuf<int32_t> d_q, d_db, d_slot;
+    BatchBuf bb;
+    d_q.reserve(std::max(nq, 1));
+    if (nq) CK(cudaMemcpyAsync(d_q.p, qids, sizeof(int32_t) * nq, cudaMemcpyHostToDevice, st_));
+    HmkBulkArgs a{};
+    a.nq = nq;
+    a.packed = d_packed_.p;
+    a.db_begin = db_begin; a.ndb = ndb;
+    if (db_ids) {
+        d_db.reserve(std::max(ndb, 1));
+        if (ndb) CK(cudaMemcpyAsync(d_db.p, db_ids, sizeof(int32_t) * ndb, cudaMemcpyHostToDevice, st_));
+        a.db_ids = d_db.p; a.db_begin = 0;
+    }
+    std::vector<int32_t> h_slot;
+    if (clustered) {
+        h_slot.resize(std::max(n_, 1));
+        for (int i = 0; i < n_; i++) h_slot[i] = clustered[i] ? 0 : -1;
+        d_slot.reserve(h_slot.size());
+        CK(cudaMemcpyAsync(d_slot.p, h_slot.data(), sizeof(int32_t) * h_slot.size(), cudaMemcpyHostToDevice, st_));
+        a.slot = d_slot.p;
+    }
+    if (fast_) {
+        bb.prof.reserve((size_t)std::max(nq, 1) * sc_.prof_words);
+        launch_profiles(HMK_PROF_QUERY, d_q.p, nq, bb.prof.p, sc_, st_);
+        a.prof = bb.prof.p;
+    }
+    DevBuf<int4> d_hits;
+    DevBuf<unsigned long long> d_count;
+    d_hits.reserve(std::max<int64_t>(hit_cap, 1));
+    d_count.reserve(2);
+    CK(cudaMemsetAsync(d_count.p, 0, 2 * sizeof(unsigned long long), st_));
+    HmkBulkArgs p = a;
+    if (mode == 0) {
+        a.q_minid = d_q.p;
+        a.tierank = identity_rank_ ? nullptr : d_tierank_.p;
+        bb.gmin.reserve(std::max(nq, 1));
+        CK(cudaMemsetAsync(bb.gmin.p, 0, sizeof(unsigned long long) * std::max(nq, 1), st_));
+        a.tk_gmin = bb.gmin.p;
+        a.xhits = d_hits.p; a.xhit_count = d_count.p; a.xhit_cap = (unsigned long long)hit_cap;
+        p = launch_bulk(HMK_MODE_TOPK, a, d_q.p, 1, st_, &bb);
+        bb.bk_key.reserve((size_t)std::max(nq, 1) * kb); bb.bk_cnt.reserve(std::max(nq, 1)); bb.bk_ovf.reserve(std::max(nq, 1));
+        if (nq && ndb) {
+            hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, st_>>>(nq, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
+                                                                  bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p,
+                                                                  p.sched ? p.sched + p.nqt : nullptr, p.qt);
+            CK(cudaGetLastError());
+            launches_++;
+            CK(cudaMemcpyAsync(keys, bb.bk_key.p, sizeof(uint64_t) * nq * kb, cudaMemcpyDeviceToHost, st_));
+            CK(cudaMemcpyAsync(cnt, bb.bk_cnt.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
+            CK(cudaMemcpyAsync(ovf, bb.bk_ovf.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
+        } else {
+            for (int t = 0; t < nq; t++) { cnt[t] = 0; ovf[t] = 0; }
+        }
+    } else {
+        a.hits = d_hits.p; a.hit_count = reinterpret_cast<unsigned int*>(d_count.p);
+        a.hit_cap = (unsigned int)std::min<int64_t>(hit_cap, UINT32_MAX);
+        p = launch_bulk(HMK_MODE_EMIT, a, d_q.p, 1, st_);
+    }
+    CK(cudaMemcpyAsync(h_scalars_, d_count.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
+    CK(cudaStreamSynchronize(st_));
+    unsigned long long total;
+    if (mode == 0) total = *reinterpret_cast<unsigned long long*>(h_scalars_);
+    else total = *reinterpret_cast<unsigned int*>(h_scalars_);
+    *hit_count = (int64_t)total;
+    const size_t stored = (size_t)std::min<unsigned long long>(total, (unsigned long long)hit_cap);
+    if (stored) {
+        std::vector<int4> h((size_t)stored);
+        CK(cudaMemcpy(h.data(), d_hits.p, sizeof(int4) * stored, cudaMemcpyDeviceToHost));
+        for (size_t e = 0; e < stored; e++) { hits[3 * e] = h[e].x; hits[3 * e + 1] = h[e].y; hits[3 * e + 2] = h[e].z; }
+    }
+    // which kernel ran: kind (0 generic, 1 hmk_bulk_fast, 2 hmk_bulk_filter, 3 hmk_bulk_long), the filter kernel's
+    // compile-time length (12 or 0, else -1), words per profile entry, lane bits, persistent grid
+    const bool ran = nq > 0 && ndb > 0;
+    kernel[0] = !fast_ ? 0 : sc_.long_layout ? 3 : sc_.filter ? 2 : 1;
+    kernel[1] = kernel[0] == 2 ? (sc_.L == 12 ? 12 : 0) : -1;
+    kernel[2] = fast_ ? sc_.nw : 0;
+    kernel[3] = fast_ ? (sc_.lane16 ? 16 : 8) : 32;
+    kernel[4] = ran && p.sched ? 1 : 0;
+}
+
 // ---------------------------------------------------------------- exact complete-linkage clustering (SURVEY.md 8f N1)
 // ClinkageSequenceClusterer.cluster (ClinkageSequenceClusterer.java:43-124).  n <= opt.clinkage_dense_max: dense pair
 // scores from the bulk kernel, nearest-neighbour chain in hmk_clinkage_chain.  Larger n: the entries scoring >= T only
@@ -2075,6 +2176,18 @@ int hmk_score_block(hmk_ctx* ctx, const int32_t* first_ids, int32_t n_first, con
     if (!ctx) return HMK_STATUS_BAD_ARG;
     return guarded(errbuf, errlen, [&] {
         ctx->engine.score_block(first_ids, n_first, second_ids, n_second, scores);
+        return HMK_STATUS_OK;
+    });
+}
+
+int hmk_bulk_probe(hmk_ctx* ctx, int32_t mode, const int32_t* query_ids, int32_t n_query, const int32_t* db_ids,
+                   int32_t db_begin, int32_t n_db, const uint8_t* clustered, uint64_t* keys, int32_t* counts,
+                   int32_t* overflow, int32_t* hits, int64_t hit_cap, int64_t* hit_count, int32_t* kernel, char* errbuf,
+                   size_t errlen) {
+    if (!ctx) return HMK_STATUS_BAD_ARG;
+    return guarded(errbuf, errlen, [&] {
+        ctx->engine.bulk_probe(mode, query_ids, n_query, db_ids, db_begin, n_db, clustered, keys, counts, overflow, hits,
+                               hit_cap, hit_count, kernel);
         return HMK_STATUS_OK;
     });
 }

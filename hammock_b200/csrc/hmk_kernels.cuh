@@ -239,14 +239,16 @@ struct HmkTopkSmem {
     int* ovf;         // [qt]
 };
 
+// A packed-path hit has T <= score <= T + (top - half) of its lanes, at most T + 32767 with 16-bit lanes, so the queue
+// stores score - T as an unsigned 16-bit number (a signed 16-bit score would wrap above 32767).
 struct HmkHitQueue {
-    uint64_t* q;      // this warp's HMK_QCAP entries: (tile-local query << 48) | (score16 << 32) | item
+    uint64_t* q;      // this warp's HMK_QCAP entries: (tile-local query << 48) | ((score - T) as u16 << 32) | item
     int32_t* s32;     // generic kernel only: full int32 scores (NULL on the packed path)
     int cnt;          // warp-uniform
 };
 
-__device__ __forceinline__ uint64_t hmk_hit_pack(int tl, int32_t score, int32_t i) {
-    return ((uint64_t)(uint32_t)tl << 48) | ((uint64_t)(uint16_t)(int16_t)score << 32) | (uint32_t)i;
+__device__ __forceinline__ uint64_t hmk_hit_pack(int tl, uint32_t over, int32_t i) {
+    return ((uint64_t)(uint32_t)tl << 48) | ((uint64_t)(uint16_t)over << 32) | (uint32_t)i;
 }
 
 // executed by ONE lane of a warp at a time (the others wait at a ballot), so the spin only
@@ -300,7 +302,7 @@ __device__ __noinline__ void hmk_queue_drain(const HmkBulkArgs& a, const HmkTopk
         for (int e = lane; e < n; e += 32) {
             const uint64_t v = hq.q[e];
             const unsigned int pos = base + e;
-            const int32_t sc = hq.s32 ? hq.s32[e] : (int32_t)(int16_t)(uint16_t)(v >> 32);
+            const int32_t sc = hq.s32 ? hq.s32[e] : a.sc.T + (int32_t)(uint16_t)(v >> 32);
             const int32_t i = (int32_t)(uint32_t)v;
             HMK_CHECK(i >= 0 && i < a.ndb && (int)(v >> 48) < a.qt);
             const int32_t id = a.db_ids ? a.db_ids[i] : a.db_begin + i;
@@ -319,7 +321,7 @@ __device__ __noinline__ void hmk_queue_drain(const HmkBulkArgs& a, const HmkTopk
                 const int32_t i = (int32_t)(uint32_t)v;
                 HMK_CHECK(i >= 0 && i < a.ndb && tl < a.qt && q0 + tl < a.nq);
                 id = a.db_ids ? a.db_ids[i] : a.db_begin + i;
-                sc = hq.s32 ? hq.s32[e] : (int32_t)(int16_t)(uint16_t)(v >> 32);
+                sc = hq.s32 ? hq.s32[e] : a.sc.T + (int32_t)(uint16_t)(v >> 32);
                 pending = !(a.q_minid && id <= a.q_minid[q0 + tl]);   // initialList[index+1 ..] only
             }
             if (a.xhits) {   // keep every qualifying hit for phase 2
@@ -368,8 +370,9 @@ __device__ __forceinline__ void hmk_queue_push(const HmkBulkArgs& a, const HmkTo
         const int lane = threadIdx.x & 31;
         if (hit) {
             const int pos = hq.cnt + __popc(m & ((1u << lane) - 1u));
-            HMK_CHECK(pos >= 0 && pos < HMK_QCAP);
-            hq.q[pos] = hmk_hit_pack(tl, score, i);
+            const uint32_t over = (uint32_t)score - (uint32_t)a.sc.T;   // 0 .. 0xffff on the packed path
+            HMK_CHECK(pos >= 0 && pos < HMK_QCAP && (hq.s32 || over <= 0xffffu));
+            hq.q[pos] = hmk_hit_pack(tl, over, i);
             if (hq.s32) hq.s32[pos] = score;
         }
         hq.cnt += __popc(m);

@@ -534,12 +534,15 @@ class GreedyContext:
             _raise_status(rc, err.value)
         self._keep = None
         self.n = 0
+        self._kb = 8        # option kb (the engine's default): row length of bulk_probe's key lists
         for k, v in options.items():
             self.set_option(k, v)
 
     def set_option(self, name: str, value: int):
         if self._L.hmk_set_option(self._h, name.encode(), int(value)):
             raise ValueError(f"unknown option {name}")
+        if name == "kb":
+            self._kb = int(value)
 
     def close(self):
         if self._h:
@@ -663,6 +666,45 @@ class GreedyContext:
                                      _ptr(out, C.c_int32), err, 512)
         if rc:
             _raise_status(rc, err.value)
+        return out
+
+    _KERNELS = {0: "generic", 1: "fast", 2: "filter", 3: "long"}
+
+    def bulk_probe(self, mode: int, query_ids, db=None, db_range=None, clustered=None, hit_cap: int = 0):
+        """hmk_bulk_probe: one bulk launch (the kernel tests' hook).  The thread side is the id list `db` or the id range
+        `db_range` = (begin, count); `clustered` (optional, bool per uploaded sequence) skips those items.
+        -> dict with "hits" (int32 [k, 3]: query id (mode 0) or query index (mode 1), thread-side
+        id, score), "hit_count" (what the kernel found; may exceed hit_cap), "kernel" (kind, filter_lt, nw, lane_bits,
+        persistent) and, in mode 0, "keys" (uint64 [nq, kb]), "cnt", "ovf"."""
+        q = np.ascontiguousarray(query_ids, dtype=np.int32)
+        nq = len(q)
+        if (db is None) == (db_range is None):
+            raise ValueError("give exactly one of db and db_range")
+        if db is not None:
+            dbi = np.ascontiguousarray(db, dtype=np.int32)
+            dbp, begin, ndb = _ptr(dbi, C.c_int32), 0, len(dbi)
+        else:
+            dbi = None
+            dbp, (begin, ndb) = None, (int(db_range[0]), int(db_range[1]))
+        cl = None if clustered is None else np.ascontiguousarray(clustered, dtype=np.uint8)
+        keys = np.zeros((max(nq, 1), self._kb), dtype=np.uint64)
+        cnt = np.zeros(max(nq, 1), dtype=np.int32)
+        ovf = np.zeros(max(nq, 1), dtype=np.int32)
+        hits = np.zeros((max(hit_cap, 1), 3), dtype=np.int32)
+        hcount = C.c_int64(0)
+        kern = np.zeros(5, dtype=np.int32)
+        err = C.create_string_buffer(512)
+        rc = self._L.hmk_bulk_probe(self._h, int(mode), _ptr(q, C.c_int32), nq, dbp, begin, ndb,
+                                    None if cl is None else _ptr(cl, C.c_uint8), _ptr(keys, C.c_uint64),
+                                    _ptr(cnt, C.c_int32), _ptr(ovf, C.c_int32), _ptr(hits, C.c_int32), int(hit_cap),
+                                    C.byref(hcount), _ptr(kern, C.c_int32), err, 512)
+        if rc:
+            _raise_status(rc, err.value)
+        out = {"hits": hits[:min(hcount.value, hit_cap)], "hit_count": int(hcount.value),
+               "kernel": {"kind": self._KERNELS[int(kern[0])], "filter_lt": int(kern[1]), "nw": int(kern[2]),
+                          "lane_bits": int(kern[3]), "persistent": int(kern[4])}}
+        if mode == 0:
+            out.update(keys=keys[:nq], cnt=cnt[:nq], ovf=ovf[:nq])
         return out
 
 

@@ -194,6 +194,23 @@ int hmk_set_option(hmk_ctx* ctx, const char* name, int64_t value);
 int hmk_score_block(hmk_ctx* ctx, const int32_t* first_ids, int32_t n_first, const int32_t* second_ids,
                     int32_t n_second, int32_t* scores, char* errbuf, size_t errlen);
 
+/* One bulk scoring launch over the uploaded sequences with the context's scheme and options.  Used by the kernel tests.
+ * Profile side: query_ids[0 .. n_query), as seq2.  Thread side (seq1): db_ids[0 .. n_db), or with db_ids NULL the ids
+ * db_begin .. db_begin + n_db - 1.  clustered (optional, one byte per uploaded sequence): non-zero items are skipped.
+ *   mode 0, partner search: a thread-side id qualifies for query t when it is > query_ids[t] and scores >= threshold.
+ *     keys[t * kb ..] (kb = option kb) = the merged best-hit list in descending key order (score, then the tie-break rank
+ *     (abundance desc, id asc)), counts[t] = its length, overflow[t] = 1 when more than kb ids qualified.  hits receives
+ *     every qualifying hit as (query id, thread-side id, score).
+ *   mode 1, hits: hits receives every pair scoring >= threshold as (query index, thread-side id, score).
+ * hits holds hit_cap triples; *hit_count = the hits the kernel found (may exceed hit_cap; then hit_cap are stored).
+ * kernel[5] = the kernel that ran: kind (0 hmk_bulk_generic, 1 hmk_bulk_fast, 2 hmk_bulk_filter, 3 hmk_bulk_long),
+ * hmk_bulk_filter's compile-time length (12 or 0; else -1), 32-bit words per profile entry, lane bits (32: generic),
+ * persistent grid (1) or static grid (0). */
+int hmk_bulk_probe(hmk_ctx* ctx, int32_t mode, const int32_t* query_ids, int32_t n_query, const int32_t* db_ids,
+                   int32_t db_begin, int32_t n_db, const uint8_t* clustered, uint64_t* keys, int32_t* counts,
+                   int32_t* overflow, int32_t* hits, int64_t hit_cap, int64_t* hit_count, int32_t* kernel, char* errbuf,
+                   size_t errlen);
+
 #ifdef __cplusplus
 }
 #endif
