@@ -144,6 +144,15 @@ struct SmemConfig {
     }
 };
 
+// the bulk kernel a launch runs (Engine::launch_planned); `kind` numbers as in hmk_bulk_probe's kernel array
+struct BulkKernel {
+    enum Kind { GENERIC = 0, FAST = 1, FILTER = 2, LONG = 3 };
+    int kind;
+    int lt;            // hmk_bulk_filter's compile-time length (12 or 0); -1 for the other kernels
+    int threads;
+    const void* fn;    // takes HmkGenericArgs (GENERIC) or HmkBulkArgs
+};
+
 enum { HMK_MAXTILES_PERSISTENT = 1024 };   // profile tiles a persistent bulk launch schedules (more: static grid)
 enum { HMK_FB_STRIDE = 1 << 16 };   // founders per slice of the per-length split of the cluster search
 enum { HMK_NAUX = 6 };         // auxiliary streams for launches that are independent of each other (length buckets)
@@ -401,10 +410,11 @@ private:
     HmkScheme scheme_for(int n) const;
     void launch_profiles(int mode, const int32_t* ids, int nq, uint32_t* prof, const HmkScheme& sc, cudaStream_t s,
                          uint32_t* cells = nullptr, uint32_t* ops = nullptr);
-    void plan_bulk(HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched = nullptr) const;
-    void launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const int32_t* prof_ids, int prof_is_query, cudaStream_t s);
+    void plan_bulk(int mode, HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched = nullptr) const;
+    BulkKernel launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const int32_t* prof_ids, int prof_is_query,
+                              cudaStream_t s);
     HmkBulkArgs launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int prof_is_query, cudaStream_t s = nullptr,
-                            BatchBuf* bb = nullptr, DevBuf<int32_t>* sched_buf = nullptr);
+                            BatchBuf* bb = nullptr, DevBuf<int32_t>* sched_buf = nullptr, BulkKernel* ran = nullptr);
     cudaEvent_t next_event();
     // per-section device timers (only with opt.profile)
     std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> sections_;
@@ -618,9 +628,10 @@ cudaEvent_t Engine::next_event() {
 
 int Engine::qt_max(const HmkScheme& sc) const {
     if (opt.qt > 0) return (int)opt.qt;
-    const size_t pwb = (size_t)sc.prof_words * 4;
-    const size_t per = pwb + (size_t)opt.kb * 8 + 8 + 12;
-    const size_t fixed = 128 + (HMK_BULK_THREADS / 32) * HMK_QCAP * 8;
+    // a profile with its share of the carve-up, beside the hit queues of a 768-thread block and 128 bytes for the barrier
+    // and alignment.  The 512-thread long kernel is sized the same way: its tiles are the ones it was measured with.
+    const size_t per = (size_t)sc.prof_words * 4 + hmk_carve_bytes(1, (int)opt.kb, 0, false);
+    const size_t fixed = 128 + hmk_carve_bytes(0, (int)opt.kb, HMK_BULK_THREADS, false);
     // the filter kernel's tile stays at the 56 profiles the batch size and chunking were measured with (more would fit)
     const size_t cap = sc.filter ? HMK_FILTER_QT : 255;
     return (int)std::min<size_t>(cap, std::max<size_t>(1, (smem_optin_ - fixed) / per));
@@ -643,58 +654,35 @@ void Engine::launch_profiles(int mode, const int32_t* ids, int nq, uint32_t* pro
     launches_++;
 }
 
-template <int NW, int MODE>
-static void launch_fast_inst(SmemConfig& cfg, const HmkBulkArgs& a, int grid, size_t smem, cudaStream_t st) {
-    cfg.ensure(hmk_bulk_fast<NW, MODE>, smem);
-    hmk_bulk_fast<NW, MODE><<<grid, HMK_BULK_THREADS, smem, st>>>(a);
-}
-
+// the bulk kernel of a (MODE, scheme) pair; `sch` NULL: the generic kernel
 template <int MODE>
-static void launch_long_mode(SmemConfig& cfg, const HmkBulkArgs& a, int grid, size_t smem, cudaStream_t st) {
-    cfg.ensure(hmk_bulk_long<MODE>, smem);
-    hmk_bulk_long<MODE><<<grid, HMK_LONG_THREADS, smem, st>>>(a);
-}
-
-template <int MODE>
-static void launch_filter_mode(SmemConfig& cfg, const HmkBulkArgs& a, int grid, size_t smem, cudaStream_t st) {
-    if (MODE == HMK_MODE_DENSE) {      // every score is wanted: exact kernel on the filter-layout profiles
-        cfg.ensure(hmk_bulk_fast<2, HMK_MODE_DENSE, true>, smem);
-        hmk_bulk_fast<2, HMK_MODE_DENSE, true><<<grid, HMK_BULK_THREADS, smem, st>>>(a);
-    } else {
-        constexpr int M2 = MODE == HMK_MODE_DENSE ? HMK_MODE_EMIT : MODE;
-        if (a.sc.L == 12) {
-            cfg.ensure(hmk_bulk_filter<M2, 12>, smem);
-            hmk_bulk_filter<M2, 12><<<grid, HMK_BULK_THREADS, smem, st>>>(a);
-        } else {
-            cfg.ensure(hmk_bulk_filter<M2, 0>, smem);
-            hmk_bulk_filter<M2, 0><<<grid, HMK_BULK_THREADS, smem, st>>>(a);
-        }
+static BulkKernel pick_bulk_kernel(const HmkScheme* sch) {
+    constexpr int FM = MODE == HMK_MODE_DENSE ? HMK_MODE_EMIT : MODE;   // hmk_bulk_filter has no DENSE form
+    if (!sch) return {BulkKernel::GENERIC, -1, HMK_GENERIC_THREADS, (const void*)hmk_bulk_generic<MODE>};
+    if (sch->long_layout) return {BulkKernel::LONG, -1, HMK_LONG_THREADS, (const void*)hmk_bulk_long<MODE>};
+    if (sch->filter) {
+        if (MODE == HMK_MODE_DENSE)    // every score is wanted: exact kernel on the filter-layout profiles
+            return {BulkKernel::FAST, -1, HMK_BULK_THREADS, (const void*)hmk_bulk_fast<2, HMK_MODE_DENSE, true>};
+        if (sch->L == 12) return {BulkKernel::FILTER, 12, HMK_BULK_THREADS, (const void*)hmk_bulk_filter<FM, 12>};
+        return {BulkKernel::FILTER, 0, HMK_BULK_THREADS, (const void*)hmk_bulk_filter<FM, 0>};
+    }
+    switch (sch->nw) {
+        case 1: return {BulkKernel::FAST, -1, HMK_BULK_THREADS, (const void*)hmk_bulk_fast<1, MODE>};
+        case 2: return {BulkKernel::FAST, -1, HMK_BULK_THREADS, (const void*)hmk_bulk_fast<2, MODE>};
+        case 3: return {BulkKernel::FAST, -1, HMK_BULK_THREADS, (const void*)hmk_bulk_fast<3, MODE>};
+        default: return {BulkKernel::FAST, -1, HMK_BULK_THREADS, (const void*)hmk_bulk_fast<4, MODE>};
     }
 }
-
-template <int MODE>
-static void launch_fast_mode(SmemConfig& cfg, const HmkBulkArgs& a, int grid, size_t smem, cudaStream_t st) {
-    if (a.sc.long_layout) { launch_long_mode<MODE>(cfg, a, grid, smem, st); return; }
-    if (a.sc.filter) { launch_filter_mode<MODE>(cfg, a, grid, smem, st); return; }
-    switch (a.sc.nw) {
-        case 1: launch_fast_inst<1, MODE>(cfg, a, grid, smem, st); break;
-        case 2: launch_fast_inst<2, MODE>(cfg, a, grid, smem, st); break;
-        case 3: launch_fast_inst<3, MODE>(cfg, a, grid, smem, st); break;
-        default: launch_fast_inst<4, MODE>(cfg, a, grid, smem, st); break;
-    }
-}
-
-template <int MODE>
-static void launch_generic_mode(SmemConfig& cfg, const HmkGenericArgs& g, int grid, size_t smem, cudaStream_t st) {
-    cfg.ensure(hmk_bulk_generic<MODE>, smem);
-    hmk_bulk_generic<MODE><<<grid, HMK_GENERIC_THREADS, smem, st>>>(g);
+static BulkKernel bulk_kernel(int mode, const HmkScheme* sch) {
+    return mode == HMK_MODE_TOPK ? pick_bulk_kernel<HMK_MODE_TOPK>(sch)
+         : mode == HMK_MODE_EMIT ? pick_bulk_kernel<HMK_MODE_EMIT>(sch) : pick_bulk_kernel<HMK_MODE_DENSE>(sch);
 }
 
 // tiling of a bulk launch: nqt profile tiles x nstripes database stripes; the grid is an exact
 // multiple of the SM count whenever the database is large enough (one CTA per SM is resident:
 // the profile tile fills shared memory)
-void Engine::plan_bulk(HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched) const {
-    const int threads = sch ? (sch->long_layout ? HMK_LONG_THREADS : HMK_BULK_THREADS) : HMK_GENERIC_THREADS;
+void Engine::plan_bulk(int mode, HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched) const {
+    const int threads = bulk_kernel(mode, sch).threads;
     const int sms = plan_sms_ > 0 ? plan_sms_ : sm_count_;
     int qmax = sch ? qt_max(*sch) : 128;
     if (!sch) {     // generic kernel: a thread scores its item against the whole tile, one pair after the other -- small
@@ -745,56 +733,55 @@ void Engine::plan_bulk(HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched) con
 
 // launches a planned bulk pass.  `sch` non-NULL: packed SWAR kernel with that scheme (a.prof holds
 // matching profiles); NULL: generic scalar kernel (prof_ids / prof_is_query name the profile side).
-void Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const int32_t* prof_ids, int prof_is_query,
-                            cudaStream_t s) {
+BulkKernel Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const int32_t* prof_ids, int prof_is_query,
+                                  cudaStream_t s) {
     a.sc = sch ? *sch : sc_;
     a.pair_counter = d_pairctr_.p;
     a.kb = (int)opt.kb;
     const int grid = a.sched ? a.nstripes : a.nqt * a.nstripes;
     if (a.sched) CK(cudaMemsetAsync(a.sched, 0, sizeof(int32_t) * 2 * a.nqt, s));
-    cudaEvent_t e0 = nullptr, e1 = nullptr;
-    if (opt.profile) { e0 = next_event(); e1 = next_event(); CK(cudaEventRecord(e0, s)); }
+    const BulkKernel k = bulk_kernel(mode, sch);
+    HmkGenericArgs g;
+    size_t smem;
+    void* args[1];
     if (sch) {
-        size_t smem = (((size_t)a.qt * sch->prof_words * 4 + 15) & ~(size_t)15) + 16 +
-                      hmk_carve_bytes(a.qt, a.kb, sch->long_layout ? HMK_LONG_THREADS : HMK_BULK_THREADS, false);
-        if (mode == HMK_MODE_TOPK) launch_fast_mode<HMK_MODE_TOPK>(smem_cfg_, a, grid, smem, s);
-        else if (mode == HMK_MODE_EMIT) launch_fast_mode<HMK_MODE_EMIT>(smem_cfg_, a, grid, smem, s);
-        else launch_fast_mode<HMK_MODE_DENSE>(smem_cfg_, a, grid, smem, s);
+        smem = hmk_packed_smem(a.qt, (uint32_t)sch->prof_words * 4, a.kb, k.threads).total;
+        args[0] = &a;
     } else {
-        HmkGenericArgs g;
         g.b = a; g.prof_ids = prof_ids; g.prof_is_query = prof_is_query;
         g.res = d_res_.p; g.off = d_off_.p; g.M = d_M_.p; g.maxlen = std::max(max_len_, 1);
         g.db_smem = g.maxlen <= 128 ? 1 : 0;
-        size_t smem = HMK_NRES * HMK_NRES * 4 + hmk_carve_bytes(a.qt, a.kb, HMK_GENERIC_THREADS, true) +
-                      (size_t)a.qt * 4 + (((size_t)a.qt * g.maxlen + 15) & ~(size_t)15) +
-                      (g.db_smem ? (size_t)g.maxlen * HMK_GENERIC_THREADS : 0) + 16;
-        if (mode == HMK_MODE_TOPK) launch_generic_mode<HMK_MODE_TOPK>(smem_cfg_, g, grid, smem, s);
-        else if (mode == HMK_MODE_EMIT) launch_generic_mode<HMK_MODE_EMIT>(smem_cfg_, g, grid, smem, s);
-        else launch_generic_mode<HMK_MODE_DENSE>(smem_cfg_, g, grid, smem, s);
+        smem = hmk_generic_smem(a.qt, a.kb, g.maxlen, g.db_smem).total;
+        args[0] = &g;
     }
-    CK(cudaGetLastError());
+    smem_cfg_.ensure(k.fn, smem);
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    if (opt.profile) { e0 = next_event(); e1 = next_event(); CK(cudaEventRecord(e0, s)); }
+    CK(cudaLaunchKernel(k.fn, dim3(grid), dim3(k.threads), args, smem, s));
     if (opt.profile) { CK(cudaEventRecord(e1, s)); bulk_events_.push_back({e0, e1}); }
     launches_++;
     bulk_launches_++;
+    return k;
 }
 
 // one-launch convenience: the uniform packed kernel when the whole input has one length <= 12, else the generic kernel.
 // Returns the planned arguments (a TOPK launch's per-stripe lists are merged by the caller, with hmk_topk_merge).
 HmkBulkArgs Engine::launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids, int prof_is_query, cudaStream_t s, BatchBuf* bb,
-                                DevBuf<int32_t>* sched_buf) {
+                                DevBuf<int32_t>* sched_buf, BulkKernel* ran) {
     if (a.nq <= 0 || a.ndb <= 0) return a;
     if (!s) s = st_;
     const HmkScheme* sch = fast_ ? &sc_ : nullptr;
     DevBuf<int32_t>& sched = sched_buf ? *sched_buf : (bb ? bb->sched : d_sched_);      // launches on different streams overlap: one each
     sched.reserve(2 * HMK_MAXTILES_PERSISTENT);
-    plan_bulk(a, sch, mode == HMK_MODE_DENSE ? nullptr : sched.p);
+    plan_bulk(mode, a, sch, mode == HMK_MODE_DENSE ? nullptr : sched.p);
     if (mode == HMK_MODE_TOPK) {
         const size_t slots = (size_t)a.nstripes * a.nq;
         bb->tk_key.reserve(slots * opt.kb); bb->tk_cnt.reserve(slots); bb->tk_ovf.reserve(slots);
         a.tk_key = bb->tk_key.p; a.tk_cnt = bb->tk_cnt.p; a.tk_ovf = bb->tk_ovf.p;
         a.stripe_base = 0;
     }
-    launch_planned(mode, a, sch, prof_ids, prof_is_query, s);
+    const BulkKernel k = launch_planned(mode, a, sch, prof_ids, prof_is_query, s);
+    if (ran) *ran = k;
     return a;
 }
 
@@ -857,7 +844,7 @@ void Engine::founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf
             HmkBulkArgs b = a;
             b.prof = pf.p; b.prof_cells = bb.pcells[L].p; b.prof_ops = bb.pops[L].p;
             b.db_ids = bb.fb_ids.p + (size_t)L * HMK_FB_STRIDE; b.ndb = fn; b.ndb_dev = bb.fb_cnt.p + L;
-            plan_bulk(b, &sch);
+            plan_bulk(HMK_MODE_EMIT, b, &sch);
             launch_planned(HMK_MODE_EMIT, b, &sch, bb.qid.p, 1, s);
         }
     }
@@ -935,7 +922,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
             Plan p;
             p.L = L; p.sc = scheme_for(L); p.a = a;
             p.a.db_ids = d_bucket_[L].p + lo; p.a.db_begin = 0; p.a.ndb = hi - lo;
-            plan_bulk(p.a, &p.sc);
+            plan_bulk(HMK_MODE_TOPK, p.a, &p.sc);
             p.a.stripe_base = total_stripes;
             total_stripes += p.a.nstripes;
             plans.push_back(p);
@@ -1232,7 +1219,7 @@ void Engine::phase2() {
             a.packed = d_packed_.p; a.db_ids = ids + c0; a.db_begin = 0; a.ndb = cn;
             a.hits = d_hits_.p; a.hit_count = d_counts_.p; a.hit_cap = (unsigned int)hit_cap;
             if (sch && mixed_) { a.prof_cells = d_pcells_.p; a.prof_ops = d_pops_.p; }
-            plan_bulk(a, sch);
+            plan_bulk(HMK_MODE_EMIT, a, sch);
             launch_planned(HMK_MODE_EMIT, a, sch, d_cf_.p, 0, st_);
             sec(SEC_P2_CHECK);
             CK(cudaMemcpyAsync(h_scalars_, d_counts_.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st_));
@@ -1663,6 +1650,7 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
     d_count.reserve(2);
     CK(cudaMemsetAsync(d_count.p, 0, 2 * sizeof(unsigned long long), st_));
     HmkBulkArgs p = a;
+    BulkKernel k{-1, -1, 0, nullptr};
     if (mode == 0) {
         a.q_minid = d_q.p;
         a.tierank = identity_rank_ ? nullptr : d_tierank_.p;
@@ -1670,7 +1658,7 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
         CK(cudaMemsetAsync(bb.gmin.p, 0, sizeof(unsigned long long) * std::max(nq, 1), st_));
         a.tk_gmin = bb.gmin.p;
         a.xhits = d_hits.p; a.xhit_count = d_count.p; a.xhit_cap = (unsigned long long)hit_cap;
-        p = launch_bulk(HMK_MODE_TOPK, a, d_q.p, 1, st_, &bb);
+        p = launch_bulk(HMK_MODE_TOPK, a, d_q.p, 1, st_, &bb, nullptr, &k);
         bb.bk_key.reserve((size_t)std::max(nq, 1) * kb); bb.bk_cnt.reserve(std::max(nq, 1)); bb.bk_ovf.reserve(std::max(nq, 1));
         if (nq && ndb) {
             hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, st_>>>(nq, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
@@ -1687,7 +1675,7 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
     } else {
         a.hits = d_hits.p; a.hit_count = reinterpret_cast<unsigned int*>(d_count.p);
         a.hit_cap = (unsigned int)std::min<int64_t>(hit_cap, UINT32_MAX);
-        p = launch_bulk(HMK_MODE_EMIT, a, d_q.p, 1, st_);
+        p = launch_bulk(HMK_MODE_EMIT, a, d_q.p, 1, st_, nullptr, nullptr, &k);
     }
     CK(cudaMemcpyAsync(h_scalars_, d_count.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st_));
     CK(cudaStreamSynchronize(st_));
@@ -1701,14 +1689,14 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
         CK(cudaMemcpy(h.data(), d_hits.p, sizeof(int4) * stored, cudaMemcpyDeviceToHost));
         for (size_t e = 0; e < stored; e++) { hits[3 * e] = h[e].x; hits[3 * e + 1] = h[e].y; hits[3 * e + 2] = h[e].z; }
     }
-    // which kernel ran: kind (0 generic, 1 hmk_bulk_fast, 2 hmk_bulk_filter, 3 hmk_bulk_long), the filter kernel's
-    // compile-time length (12 or 0, else -1), words per profile entry, lane bits, persistent grid
-    const bool ran = nq > 0 && ndb > 0;
-    kernel[0] = !fast_ ? 0 : sc_.long_layout ? 3 : sc_.filter ? 2 : 1;
-    kernel[1] = kernel[0] == 2 ? (sc_.L == 12 ? 12 : 0) : -1;
-    kernel[2] = fast_ ? sc_.nw : 0;
-    kernel[3] = fast_ ? (sc_.lane16 ? 16 : 8) : 32;
-    kernel[4] = ran && p.sched ? 1 : 0;
+    // which kernel ran (kind -1: none, the launch was empty): kind, the filter kernel's compile-time length, words per
+    // profile entry, lane bits, persistent grid
+    const bool packed = k.kind > BulkKernel::GENERIC;
+    kernel[0] = k.kind;
+    kernel[1] = k.lt;
+    kernel[2] = packed ? sc_.nw : 0;
+    kernel[3] = packed ? (sc_.lane16 ? 16 : 8) : k.fn ? 32 : 0;
+    kernel[4] = k.fn && p.sched ? 1 : 0;
 }
 
 // ---------------------------------------------------------------- exact complete-linkage clustering (SURVEY.md 8f N1)

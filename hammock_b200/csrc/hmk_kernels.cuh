@@ -1,8 +1,10 @@
 // hmk_kernels.cuh -- sm_100a kernels of the greedy-clustering engine.
 //
-// Hot kernel: hmk_bulk_fast<NW, MODE>.  One thread owns one database peptide (5-bit packed,
-// one 64-bit word, <= 12 residues) and scores it against a tile of "profile" sequences held
-// in shared memory.  A profile is the substitution matrix pre-arranged per diagonal:
+// Hot kernel: hmk_bulk_filter<MODE, LT>, the partner search and founder filter on sequences of
+// <= 12 residues; it screens pairs with an upper-bound table and re-scores the survivors with
+// the exact scheme of hmk_bulk_fast<NW, MODE>.  There one thread owns one database peptide
+// (5-bit packed, one 64-bit word, <= 12 residues) and scores it against a tile of "profile"
+// sequences held in shared memory.  A profile is the substitution matrix pre-arranged per diagonal:
 // entry[h][j][r] (32 bit) holds, for database position j carrying residue r, the
 // contributions to 4 (u8 lanes) or 2 (s16 lanes) of the 2X+1 shift diagonals.  One pair score
 // = L x NW conflict-free LDS.32 + 3-input adds on packed lanes; lanes are biased so that
@@ -30,9 +32,6 @@
                                // (four octets of one 32-bit mask per exact word; the kernel relies on 32)
 #ifndef HMK_BULK_THREADS
 #define HMK_BULK_THREADS 768
-#endif
-#ifndef HMK_LFIX
-#define HMK_LFIX 0               // 12: compile the packed kernel for length-12 data only (no length predicates)
 #endif
 
 enum { HMK_MODE_TOPK = 0, HMK_MODE_EMIT = 1, HMK_MODE_DENSE = 2 };
@@ -437,6 +436,89 @@ __host__ __device__ inline size_t hmk_carve_bytes(int qt, int kb, int threads, b
     return (size_t)qt * kb * 8 + (size_t)qt * 8 + (size_t)(threads / 32) * HMK_QCAP * (wide ? 12 : 8) + (size_t)qt * 12;
 }
 
+// ---------------------------------------------------------------- pieces shared by the bulk kernels
+// Packed kernels' shared memory: the profile tile (qt profiles of pwb bytes) from offset 0, the TMA barrier at `bar`,
+// the carve-up for `threads` threads at `carve`; `total` is a launch's dynamic size.
+struct HmkPackedSmem { size_t bar, carve, total; };
+__host__ __device__ inline HmkPackedSmem hmk_packed_smem(int qt, uint32_t pwb, int kb, int threads) {
+    const size_t bar = ((size_t)qt * pwb + 15) & ~(size_t)15;
+    return {bar, bar + 16, bar + 16 + hmk_carve_bytes(qt, kb, threads, false)};
+}
+
+// carves a packed kernel's shared memory and initialises the tile barrier (visible after the next __syncthreads)
+__device__ __forceinline__ uint64_t* hmk_packed_carve(unsigned char* smem, const HmkBulkArgs& a, uint32_t pwb, HmkTopkSmem& tk,
+                                                      HmkHitQueue& hq) {
+    const HmkPackedSmem ly = hmk_packed_smem(a.qt, pwb, a.kb, blockDim.x);
+    hmk_carve(smem + ly.carve, a.qt, a.kb, false, tk, hq);
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + ly.bar);
+    if (threadIdx.x == 0) hmk_mbar_init(bar, 1);
+    return bar;
+}
+
+// stages profiles q0 .. q0 + qn - 1 (pwb bytes each) at the start of shared memory with the TMA bulk-copy engine and
+// waits for them (barrier parity `phase`); TOPK first clears the tile's lists
+template <int MODE>
+__device__ __forceinline__ void hmk_stage_tile(unsigned char* smem, uint64_t* bar, uint32_t phase, const HmkBulkArgs& a,
+                                               const HmkTopkSmem& tk, int q0, int qn, uint32_t pwb) {
+    if (MODE == HMK_MODE_TOPK) hmk_topk_init(tk, qn, a.kb);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const uint32_t total = (uint32_t)qn * pwb;
+        hmk_mbar_expect_tx(bar, total);
+        const unsigned char* src = reinterpret_cast<const unsigned char*>(a.prof) + (size_t)q0 * pwb;
+        uint32_t done = 0;
+        while (done < total) {
+            uint32_t n = min(total - done, 32768u);
+            hmk_bulk_g2s(smem + done, src + done, n, bar);
+            done += n;
+        }
+    }
+    hmk_mbar_wait(bar, phase);
+}
+
+// end of the thread-side items of the chunk that starts at i_begin: ndb, or *ndb_dev when given
+__device__ __forceinline__ int hmk_items_end(const HmkBulkArgs& a, int i_begin) {
+    return min(a.ndb_dev ? min(a.ndb, __ldg(a.ndb_dev)) : a.ndb, i_begin + a.chunk);
+}
+
+// thread-side item i: its sequence id (0 past the end) and whether it is scored -- before i_end, not below min_id and
+// still a singleton.  The packed kernels pass min_id = 0: ids are >= 0, so the unsigned test folds away (a runtime
+// a.db_min_id there costs registers); the generic kernel passes a.db_min_id, tested before the slot load.
+__device__ __forceinline__ bool hmk_item(const HmkBulkArgs& a, int i, int i_end, int32_t min_id, int32_t& id) {
+    bool valid = i < i_end;
+    id = valid ? (a.db_ids ? a.db_ids[i] : a.db_begin + i) : 0;
+    if (valid && ((uint32_t)id < (uint32_t)min_id || (a.slot && a.slot[id] >= 0))) valid = false;
+    return valid;
+}
+
+// end of a tile: the warp's last queued hits, then (TOPK) the tile's lists into output slot `slot`
+template <int MODE>
+__device__ __forceinline__ void hmk_tile_end(const HmkBulkArgs& a, const HmkTopkSmem& tk, int q0, int qn, HmkHitQueue& hq,
+                                             int slot) {
+    if (MODE != HMK_MODE_DENSE && hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
+    if (MODE == HMK_MODE_TOPK) {
+        __syncthreads();
+        hmk_topk_flush(a, tk, q0, qn, slot);
+    }
+}
+
+// pair accounting: the pairs this warp scored; with prof_cells (mixed lengths: the items of a launch share one length,
+// cells differ per profile of the tile q0 .. q0 + qn - 1, qn > 0) also their cells and int ops.  prof_cells needs a
+// CTA that scores one tile: hmk_bulk_filter, which may move between tiles, never gets it
+__device__ __forceinline__ void hmk_count_scored(const HmkBulkArgs& a, unsigned long long scored, int q0, int qn) {
+    if (!a.pair_counter) return;
+    for (int s = 16; s > 0; s >>= 1) scored += __shfl_xor_sync(0xffffffffu, scored, s);
+    if ((threadIdx.x & 31) == 0 && scored) {
+        atomicAdd(a.pair_counter, scored);
+        if (a.prof_cells) {
+            unsigned long long tc = 0, to = 0;
+            for (int t = 0; t < qn; t++) { tc += a.prof_cells[q0 + t]; to += a.prof_ops[q0 + t]; }
+            atomicAdd(a.pair_counter + 1, scored / qn * tc);
+            atomicAdd(a.pair_counter + 2, scored / qn * to);
+        }
+    }
+}
+
 // ---------------------------------------------------------------- fast bulk kernel
 #define HMK_ROWB (HMK_NRES * 4)                    // bytes of one (h, j) row: 24 residues x u32
 
@@ -448,33 +530,14 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_fast(const __gri
     const int q0 = qtile * a.qt;
     const int qn = min(a.qt, a.nq - q0);
     if (qn <= 0) return;
-    const int L = HMK_LFIX ? HMK_LFIX : a.sc.L;
-    size_t o = ((size_t)a.qt * PWB + 15) & ~(size_t)15;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + o);
-    o += 16;
+    const int L = a.sc.L;
     HmkTopkSmem tk;
     HmkHitQueue hq;
-    hmk_carve(smem_raw + o, a.qt, a.kb, false, tk, hq);
-
-    // ---- stage the profile tile with the TMA bulk-copy engine
-    if (threadIdx.x == 0) hmk_mbar_init(bar, 1);
-    if (MODE == HMK_MODE_TOPK) hmk_topk_init(tk, qn, a.kb);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const uint32_t total = (uint32_t)qn * PWB;
-        hmk_mbar_expect_tx(bar, total);
-        const unsigned char* src = reinterpret_cast<const unsigned char*>(a.prof) + (size_t)q0 * PWB;
-        uint32_t done = 0;
-        while (done < total) {
-            uint32_t n = min(total - done, 32768u);
-            hmk_bulk_g2s(smem_raw + done, src + done, n, bar);
-            done += n;
-        }
-    }
-    hmk_mbar_wait(bar, 0);
+    uint64_t* bar = hmk_packed_carve(smem_raw, a, PWB, tk, hq);
+    hmk_stage_tile<MODE>(smem_raw, bar, 0, a, tk, q0, qn, PWB);
 
     const int i_begin = stripe * a.chunk;
-    const int i_end = min(a.ndb_dev ? min(a.ndb, __ldg(a.ndb_dev)) : a.ndb, i_begin + a.chunk);
+    const int i_end = hmk_items_end(a, i_begin);
     unsigned long long scored = 0;
     const uint32_t topmask = a.sc.lane16 ? 0x80008000u : 0x80808080u;
     const int32_t dec = a.sc.T - a.sc.half;
@@ -484,9 +547,8 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_fast(const __gri
     // compute on a dummy item and are masked out of the hit test
     for (int ib = i_begin + (threadIdx.x & ~31); ib < i_end; ib += blockDim.x) {
         const int i = ib + (threadIdx.x & 31);
-        bool valid = i < i_end;
-        const int32_t id = valid ? (a.db_ids ? a.db_ids[i] : a.db_begin + i) : 0;
-        if (valid && a.slot && a.slot[id] >= 0) valid = false;
+        int32_t id;
+        const bool valid = hmk_item(a, i, i_end, 0, id);
         if (!__any_sync(0xffffffffu, valid)) continue;
         const uint64_t w = valid ? a.packed[id] : 0ull;
         // rowp[j] = &profile[0][h=0][j][residue_j]; later profiles/halves are immediates away
@@ -536,23 +598,8 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_fast(const __gri
             for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += PWB;
         }
     }
-    if (MODE != HMK_MODE_DENSE && hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
-    if (a.pair_counter) {
-        for (int s = 16; s > 0; s >>= 1) scored += __shfl_xor_sync(0xffffffffu, scored, s);
-        if ((threadIdx.x & 31) == 0 && scored) {
-            atomicAdd(a.pair_counter, scored);
-            if (a.prof_cells) {   // mixed lengths: cells differ per profile; items of this launch share one length
-                unsigned long long tc = 0, to = 0;
-                for (int t = 0; t < qn; t++) { tc += a.prof_cells[q0 + t]; to += a.prof_ops[q0 + t]; }
-                atomicAdd(a.pair_counter + 1, scored / qn * tc);
-                atomicAdd(a.pair_counter + 2, scored / qn * to);
-            }
-        }
-    }
-    if (MODE == HMK_MODE_TOPK) {
-        __syncthreads();
-        hmk_topk_flush(a, tk, q0, qn, stripe);
-    }
+    hmk_count_scored(a, scored, q0, qn);
+    hmk_tile_end<MODE>(a, tk, q0, qn, hq, stripe);
 }
 
 // ---------------------------------------------------------------- filter candidates
@@ -600,14 +647,10 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
     constexpr int OCT_UNROLL = LT ? 2 : 1;
     __shared__ int s_next[3];                         // persistent mode: (tile, chunk, output slot) of the next piece of work
     const int L = LT ? LT : a.sc.L;
-    size_t o = ((size_t)a.qt * PWB + 15) & ~(size_t)15;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + o);
-    o += 16;
+    HMK_CHECK(!a.prof_cells);                         // a CTA may score several tiles (hmk_count_scored)
     HmkTopkSmem tk;
     HmkHitQueue hq;
-    hmk_carve(smem_raw + o, a.qt, a.kb, false, tk, hq);
-
-    if (threadIdx.x == 0) hmk_mbar_init(bar, 1);
+    uint64_t* bar = hmk_packed_carve(smem_raw, a, PWB, tk, hq);
     __syncthreads();
 
     unsigned long long scored = 0;
@@ -686,8 +729,7 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
         if (tile != cur_tile) {
             if (cur_tile >= 0) {        // leave the previous tile: the round was verified at the end of the chunk
                 HMK_CHECK(rfill == 0);
-                if (hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
-                if (MODE == HMK_MODE_TOPK) { __syncthreads(); hmk_topk_flush(a, tk, q0, qn, slot); }
+                hmk_tile_end<MODE>(a, tk, q0, qn, hq, slot);
                 __syncthreads();
             }
             if (persistent) { slot = s_next[2]; home = tile; }
@@ -695,31 +737,16 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
             q0 = tile * a.qt;
             qn = min(a.qt, a.nq - q0);
             if (qn <= 0) { if (persistent) continue; else return; }
-            // ---- stage the profile tile with the TMA bulk-copy engine
-            if (MODE == HMK_MODE_TOPK) hmk_topk_init(tk, qn, a.kb);
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                const uint32_t total = (uint32_t)qn * PWB;
-                hmk_mbar_expect_tx(bar, total);
-                const unsigned char* src = reinterpret_cast<const unsigned char*>(a.prof) + (size_t)q0 * PWB;
-                uint32_t done = 0;
-                while (done < total) {
-                    uint32_t n = min(total - done, 32768u);
-                    hmk_bulk_g2s(smem_raw + done, src + done, n, bar);
-                    done += n;
-                }
-            }
-            hmk_mbar_wait(bar, bar_phase);
+            hmk_stage_tile<MODE>(smem_raw, bar, bar_phase, a, tk, q0, qn, PWB);
             bar_phase ^= 1u;
         }
         i_begin = chunk_idx * a.chunk;
-        i_end = min(a.ndb, i_begin + a.chunk);
+        i_end = hmk_items_end(a, i_begin);
 
         for (int ib = i_begin + (threadIdx.x & ~31); ib < i_end; ib += blockDim.x) {
             const int i = ib + lane;
-            bool valid = i < i_end;
-            const int32_t id = valid ? (a.db_ids ? a.db_ids[i] : a.db_begin + i) : 0;
-            if (valid && a.slot && a.slot[id] >= 0) valid = false;
+            int32_t id;
+            const bool valid = hmk_item(a, i, i_end, 0, id);
             if (!__any_sync(0xffffffffu, valid)) continue;
             const uint64_t w = valid ? a.packed[id] : 0ull;
             const unsigned char* rowp[HMK_MAXL1];   // &filter[t][j][residue_j]
@@ -823,17 +850,8 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
         }
         if (rfill) verify();      // the round must be empty before the tile (and with it q0) can change
     }
-    if (cur_tile >= 0 && qn > 0) {
-        if (hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
-        if (MODE == HMK_MODE_TOPK) {
-            __syncthreads();
-            hmk_topk_flush(a, tk, q0, qn, slot);
-        }
-    }
-    if (a.pair_counter) {
-        for (int s = 16; s > 0; s >>= 1) scored += __shfl_xor_sync(0xffffffffu, scored, s);
-        if ((threadIdx.x & 31) == 0 && scored) atomicAdd(a.pair_counter, scored);
-    }
+    if (cur_tile >= 0 && qn > 0) hmk_tile_end<MODE>(a, tk, q0, qn, hq, slot);
+    hmk_count_scored(a, scored, q0, qn);
 }
 
 // ---------------------------------------------------------------- long bulk kernel
@@ -850,30 +868,13 @@ __global__ void __launch_bounds__(HMK_LONG_THREADS, 1) hmk_bulk_long(const __gri
     if (qn <= 0) return;
     const int L = a.sc.L, nw = a.sc.nw, W = a.sc.words;
     const uint32_t PWB = (uint32_t)a.sc.prof_words * 4u;
-    size_t o = ((size_t)a.qt * PWB + 15) & ~(size_t)15;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + o);
-    o += 16;
     HmkTopkSmem tk;
     HmkHitQueue hq;
-    hmk_carve(smem_raw + o, a.qt, a.kb, false, tk, hq);
-    if (threadIdx.x == 0) hmk_mbar_init(bar, 1);
-    if (MODE == HMK_MODE_TOPK) hmk_topk_init(tk, qn, a.kb);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const uint32_t total = (uint32_t)qn * PWB;
-        hmk_mbar_expect_tx(bar, total);
-        const unsigned char* src = reinterpret_cast<const unsigned char*>(a.prof) + (size_t)q0 * PWB;
-        uint32_t done = 0;
-        while (done < total) {
-            uint32_t n = min(total - done, 32768u);
-            hmk_bulk_g2s(smem_raw + done, src + done, n, bar);
-            done += n;
-        }
-    }
-    hmk_mbar_wait(bar, 0);
+    uint64_t* bar = hmk_packed_carve(smem_raw, a, PWB, tk, hq);
+    hmk_stage_tile<MODE>(smem_raw, bar, 0, a, tk, q0, qn, PWB);
 
     const int i_begin = stripe * a.chunk;
-    const int i_end = min(a.ndb, i_begin + a.chunk);
+    const int i_end = hmk_items_end(a, i_begin);
     unsigned long long scored = 0;
     const uint32_t topmask = a.sc.lane16 ? 0x80008000u : 0x80808080u;
     const int32_t dec = a.sc.T - a.sc.half;
@@ -881,9 +882,8 @@ __global__ void __launch_bounds__(HMK_LONG_THREADS, 1) hmk_bulk_long(const __gri
 
     for (int ib = i_begin + (threadIdx.x & ~31); ib < i_end; ib += blockDim.x) {
         const int i = ib + (threadIdx.x & 31);
-        bool valid = i < i_end;
-        const int32_t id = valid ? (a.db_ids ? a.db_ids[i] : a.db_begin + i) : 0;
-        if (valid && a.slot && a.slot[id] >= 0) valid = false;
+        int32_t id;
+        const bool valid = hmk_item(a, i, i_end, 0, id);
         if (!__any_sync(0xffffffffu, valid)) continue;
         uint64_t w[3] = {0ull, 0ull, 0ull};
 #pragma unroll
@@ -907,6 +907,7 @@ __global__ void __launch_bounds__(HMK_LONG_THREADS, 1) hmk_bulk_long(const __gri
                     rowp[j] += PWB;
                 }
             }
+            // both lane widths, then a select: hmk_lane_max's branch on lane16 would let the compiler duplicate this loop
             uint32_t any = 0, m2 = 0, m4 = 0;
 #pragma unroll
             for (int h = 0; h < HMK_NWMAX; h++)
@@ -926,23 +927,8 @@ __global__ void __launch_bounds__(HMK_LONG_THREADS, 1) hmk_bulk_long(const __gri
             }
         }
     }
-    if (MODE != HMK_MODE_DENSE && hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
-    if (a.pair_counter) {
-        for (int s = 16; s > 0; s >>= 1) scored += __shfl_xor_sync(0xffffffffu, scored, s);
-        if ((threadIdx.x & 31) == 0 && scored) {
-            atomicAdd(a.pair_counter, scored);
-            if (a.prof_cells) {
-                unsigned long long tc = 0, to = 0;
-                for (int t = 0; t < qn; t++) { tc += a.prof_cells[q0 + t]; to += a.prof_ops[q0 + t]; }
-                atomicAdd(a.pair_counter + 1, scored / qn * tc);
-                atomicAdd(a.pair_counter + 2, scored / qn * to);
-            }
-        }
-    }
-    if (MODE == HMK_MODE_TOPK) {
-        __syncthreads();
-        hmk_topk_flush(a, tk, q0, qn, stripe);
-    }
+    hmk_count_scored(a, scored, q0, qn);
+    hmk_tile_end<MODE>(a, tk, q0, qn, hq, stripe);
 }
 
 // ---------------------------------------------------------------- generic bulk kernel
@@ -962,26 +948,39 @@ struct HmkGenericArgs {
 
 #define HMK_GENERIC_THREADS 256
 
+// generic kernel's shared memory: the matrix from offset 0, the carve-up at `carve`, the profile lengths at `slen`, the
+// profile residues ([qt][maxlen]) at `sres`, with db_smem the thread-side residues at `sdb`; `total` is a launch's size
+struct HmkGenericSmem { size_t carve, slen, sres, sdb, total; };
+__host__ __device__ inline HmkGenericSmem hmk_generic_smem(int qt, int kb, int maxlen, bool db_smem) {
+    HmkGenericSmem l;
+    l.carve = HMK_NRES * HMK_NRES * 4;
+    l.slen = l.carve + hmk_carve_bytes(qt, kb, HMK_GENERIC_THREADS, true);
+    l.sres = l.slen + (size_t)qt * 4;
+    l.sdb = l.sres + (((size_t)qt * maxlen + 15) & ~(size_t)15);
+    l.total = l.sdb + (db_smem ? (size_t)maxlen * HMK_GENERIC_THREADS : 0) + 16;
+    return l;
+}
+
+// EMIT and DENSE: five CTAs per SM (48 registers); left free, the compiler takes 64 there, which allows only four.
+// TOPK needs its 64.
 template <int MODE>
-__global__ void __launch_bounds__(HMK_GENERIC_THREADS) hmk_bulk_generic(const __grid_constant__ HmkGenericArgs g) {
+__global__ void __launch_bounds__(HMK_GENERIC_THREADS, MODE == HMK_MODE_TOPK ? 4 : 5) hmk_bulk_generic(const __grid_constant__ HmkGenericArgs g) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const HmkBulkArgs& a = g.b;
     const int qtile = blockIdx.x % a.nqt, stripe = blockIdx.x / a.nqt;
     const int q0 = qtile * a.qt;
     const int qn = min(a.qt, a.nq - q0);
     if (qn <= 0) return;
+    const HmkGenericSmem ly = hmk_generic_smem(a.qt, a.kb, g.maxlen, g.db_smem);
     int32_t* sM = reinterpret_cast<int32_t*>(smem_raw);
-    size_t o = HMK_NRES * HMK_NRES * 4;
     HmkTopkSmem tk;
     HmkHitQueue hq;
-    hmk_carve(smem_raw + o, a.qt, a.kb, true, tk, hq);
-    o += hmk_carve_bytes(a.qt, a.kb, HMK_GENERIC_THREADS, true);
-    int32_t* slen = reinterpret_cast<int32_t*>(smem_raw + o); o += (size_t)a.qt * 4;
-    uint8_t* sres = smem_raw + o;   // [qt][maxlen]
-    o += (((size_t)a.qt * g.maxlen + 15) & ~(size_t)15);
+    hmk_carve(smem_raw + ly.carve, a.qt, a.kb, true, tk, hq);
+    int32_t* slen = reinterpret_cast<int32_t*>(smem_raw + ly.slen);
+    uint8_t* sres = smem_raw + ly.sres;
     // the thread-side sequences of the current iteration, position-major ([j][thread]): the inner loops then read shared
     // memory only, conflict free, instead of one global byte per cell and lane
-    uint8_t* sdb = smem_raw + o;    // [maxlen][HMK_GENERIC_THREADS]
+    uint8_t* sdb = smem_raw + ly.sdb;
     for (int i = threadIdx.x; i < HMK_NRES * HMK_NRES; i += blockDim.x) sM[i] = g.M[i];
     for (int t = threadIdx.x; t < qn; t += blockDim.x) {
         int32_t id = g.prof_ids[q0 + t];
@@ -992,13 +991,12 @@ __global__ void __launch_bounds__(HMK_GENERIC_THREADS) hmk_bulk_generic(const __
     if (MODE == HMK_MODE_TOPK) hmk_topk_init(tk, qn, a.kb);
     __syncthreads();
     const int i_begin = stripe * a.chunk;
-    const int i_end = min(a.ndb, i_begin + a.chunk);
+    const int i_end = hmk_items_end(a, i_begin);
     unsigned long long scored = 0;
     for (int ib = i_begin + (threadIdx.x & ~31); ib < i_end; ib += blockDim.x) {
         const int i = ib + (threadIdx.x & 31);
-        bool valid = i < i_end;
-        const int32_t id = valid ? (a.db_ids ? a.db_ids[i] : a.db_begin + i) : 0;
-        if (valid && (id < a.db_min_id || (a.slot && a.slot[id] >= 0))) valid = false;
+        int32_t id;
+        const bool valid = hmk_item(a, i, i_end, a.db_min_id, id);
         if (!__any_sync(0xffffffffu, valid)) continue;
         const uint8_t* dres = g.res + g.off[id];
         const int dlen = valid ? g.off[id + 1] - g.off[id] : 0;
@@ -1021,15 +1019,8 @@ __global__ void __launch_bounds__(HMK_GENERIC_THREADS) hmk_bulk_generic(const __
             else hmk_queue_push<MODE>(a, tk, q0, hq, valid && s >= a.sc.T, t, s, i);
         }
     }
-    if (MODE != HMK_MODE_DENSE && hq.cnt) hmk_queue_drain<MODE>(a, tk, q0, hq);
-    if (a.pair_counter) {
-        for (int s = 16; s > 0; s >>= 1) scored += __shfl_xor_sync(0xffffffffu, scored, s);
-        if ((threadIdx.x & 31) == 0 && scored) atomicAdd(a.pair_counter, scored);
-    }
-    if (MODE == HMK_MODE_TOPK) {
-        __syncthreads();
-        hmk_topk_flush(a, tk, q0, qn, stripe);
-    }
+    hmk_count_scored(a, scored, q0, qn);
+    hmk_tile_end<MODE>(a, tk, q0, qn, hq, stripe);
 }
 
 // ---------------------------------------------------------------- top-k merge across stripes

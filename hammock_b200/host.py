@@ -668,7 +668,7 @@ class GreedyContext:
             _raise_status(rc, err.value)
         return out
 
-    _KERNELS = {0: "generic", 1: "fast", 2: "filter", 3: "long"}
+    _KERNELS = {-1: "none", 0: "generic", 1: "fast", 2: "filter", 3: "long"}
 
     def bulk_probe(self, mode: int, query_ids, db=None, db_range=None, clustered=None, hit_cap: int = 0):
         """hmk_bulk_probe: one bulk launch (the kernel tests' hook).  The thread side is the id list `db` or the id range

@@ -203,9 +203,9 @@ int hmk_score_block(hmk_ctx* ctx, const int32_t* first_ids, int32_t n_first, con
  *     every qualifying hit as (query id, thread-side id, score).
  *   mode 1, hits: hits receives every pair scoring >= threshold as (query index, thread-side id, score).
  * hits holds hit_cap triples; *hit_count = the hits the kernel found (may exceed hit_cap; then hit_cap are stored).
- * kernel[5] = the kernel that ran: kind (0 hmk_bulk_generic, 1 hmk_bulk_fast, 2 hmk_bulk_filter, 3 hmk_bulk_long),
- * hmk_bulk_filter's compile-time length (12 or 0; else -1), 32-bit words per profile entry, lane bits (32: generic),
- * persistent grid (1) or static grid (0). */
+ * kernel[5] = the kernel that ran: kind (0 hmk_bulk_generic, 1 hmk_bulk_fast, 2 hmk_bulk_filter, 3 hmk_bulk_long; -1 when
+ * n_query or n_db is 0 and nothing was launched), hmk_bulk_filter's compile-time length (12 or 0; else -1), 32-bit words
+ * per profile entry, lane bits (32: generic; 0: nothing launched), persistent grid (1) or static grid (0). */
 int hmk_bulk_probe(hmk_ctx* ctx, int32_t mode, const int32_t* query_ids, int32_t n_query, const int32_t* db_ids,
                    int32_t db_begin, int32_t n_db, const uint8_t* clustered, uint64_t* keys, int32_t* counts,
                    int32_t* overflow, int32_t* hits, int64_t hit_cap, int64_t* hit_count, int32_t* kernel, char* errbuf,
