@@ -42,8 +42,18 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+class BatchProbeOut(C.Structure):
+    _fields_ = [("nq_out", C.c_int32), ("qid", C.POINTER(C.c_int32)), ("bk_key", C.POINTER(C.c_uint64)),
+                ("bk_cnt", C.POINTER(C.c_int32)), ("bk_ovf", C.POINTER(C.c_int32)), ("ib", C.POINTER(C.c_int32)),
+                ("ibm", C.POINTER(C.c_uint32)), ("ibm2", C.POINTER(C.c_uint32)), ("pcand", C.POINTER(C.c_int32)),
+                ("pd", C.POINTER(C.c_int32)), ("fhits", C.POINTER(C.c_int32)), ("fhit_cap", C.c_int64),
+                ("fhit_count", C.c_int64), ("ac_cnt", C.POINTER(C.c_int32)), ("ac_slot", C.POINTER(C.c_int32)),
+                ("ac_score", C.POINTER(C.c_int32)), ("ac_best", C.POINTER(C.c_int32)), ("kernel", C.c_int32 * 11)]
+
+
 EXPORTS = ["hmk_abi_version", "hmk_greedy_cluster", "hmk_greedy_cluster_multi", "hmk_clinkage_cluster", "hmk_clinkage_run", "hmk_create", "hmk_destroy", "hmk_upload", "hmk_run",
            "hmk_download", "hmk_get_stats", "hmk_get_section_ms", "hmk_set_option", "hmk_score_block", "hmk_bulk_probe",
+           "hmk_batch_probe",
            "hmk_timer_begin", "hmk_timer_end", "hmk_measure_peaks", "hmk_nccl_unique_id", "hmk_init_distributed", "hmk_release_cached"]
 SECTIONS = ["p1_select", "p1_partner", "p1_cluster", "p1_intra", "p1_resolve", "p2_setup", "p2_filter", "p2_check",
             "p2_sort", "p2_base", "p2_iterate", "p2_commit", "final"]
@@ -105,5 +115,8 @@ def load():
     L.hmk_bulk_probe.restype = C.c_int
     L.hmk_bulk_probe.argtypes = [vp, C.c_int32, i32p, C.c_int32, i32p, C.c_int32, C.c_int32, C.POINTER(C.c_uint8),
                                  C.POINTER(C.c_uint64), i32p, i32p, i32p, C.c_int64, C.POINTER(C.c_int64), i32p, cp, sz]
+    L.hmk_batch_probe.restype = C.c_int
+    L.hmk_batch_probe.argtypes = [vp, i32p, i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                  C.POINTER(BatchProbeOut), cp, sz]
     _lib = L
     return L

@@ -251,6 +251,8 @@ public:
     void bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t* db_ids, int32_t db_begin, int32_t ndb,
                     const uint8_t* clustered, uint64_t* keys, int32_t* cnt, int32_t* ovf, int32_t* hits, int64_t hit_cap,
                     int64_t* hit_count, int32_t* kernel);
+    void batch_probe(const int32_t* member_off, const int32_t* members, int32_t ncl, int32_t cur, int32_t nq, int32_t capq,
+                     int32_t tail_stream, hmk_batch_probe_out* out);
     int clinkage(const hmk_greedy_in* in, hmk_greedy_out* out);
     std::string status_msg;      // details of the last non-zero status, when there are any
     hmk_stats stats{};
@@ -348,6 +350,15 @@ private:
         for (auto& b : bb_) b.valid = false;
     }
     void founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf<int32_t>& sched);
+    void check_members(const BatchBuf& cb, int ncl, int capq);
+    // bulk launches per mode (HMK_MODE_*) while a batch probe runs: the last kernel launched and how many launches
+    struct LaunchLog {
+        BulkKernel last[3] = {{-1, -1, 0, nullptr}, {-1, -1, 0, nullptr}, {-1, -1, 0, nullptr}};
+        int count[3] = {0, 0, 0};
+        bool persistent = false;
+        int member_check = -1;   // scorer of the member check: 0 hmk_state_score, 1 hmk_packed_pair_score, 2 hmk_score12x3
+    };
+    LaunchLog* launch_log_ = nullptr;
     size_t hit_cap_ = 0;
     // ---- phase-1 scratch
     DevBuf<int32_t> d_qid_, d_nq_,
@@ -761,6 +772,11 @@ BulkKernel Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch,
     if (opt.profile) { CK(cudaEventRecord(e1, s)); bulk_events_.push_back({e0, e1}); }
     launches_++;
     bulk_launches_++;
+    if (launch_log_) {
+        launch_log_->last[mode] = k;
+        launch_log_->count[mode]++;
+        if (mode == HMK_MODE_TOPK && a.sched) launch_log_->persistent = true;
+    }
     return k;
 }
 
@@ -1042,6 +1058,31 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
     bb.valid = true;
 }
 
+// Cluster search, part 2, on the main stream: the linked member check of batch cb's founder hits against the clusters
+// [0, ncl) (ac_cnt / ac_slot / ac_score, capq rows per query), then each query's candidate records and best candidate
+void Engine::check_members(const BatchBuf& cb, int ncl, int capq) {
+    const int nq = cb.nq;
+    CK(cudaMemsetAsync(d_ac_cnt_.p, 0, sizeof(int32_t) * nq, st_));
+    if (ncl > 0) {
+        HmkCheckArgs c{};
+        c.S = state(); c.hits = cb.hits.p; c.hit_count = cb.hcount.p; c.hit_cap = (unsigned int)cb.hit_cap;
+        c.hit_t_is_query = 1; c.qids = cb.qid.p; c.sidx = nullptr;
+        c.ac_cnt = d_ac_cnt_.p; c.ac_slot = d_ac_slot_.p; c.ac_score = d_ac_score_.p; c.capq = capq;
+        c.cand_count = cb.hcount.p + 1; c.cand_cap = 0; c.linked = 1;
+        c.packed = fast_scalar_ ? d_packed_.p : nullptr; c.L = max_len_; c.pair_parts = d_pairparts_.p;
+        const bool fast = scalar12x3();
+        if (fast) hmk_member_check<true><<<sm_count_ * 2, 256, 0, st_>>>(c);
+        else hmk_member_check<false><<<sm_count_ * 2, 256, 0, st_>>>(c);
+        CK(cudaGetLastError());
+        launches_++;
+        if (launch_log_) launch_log_->member_check = fast ? 2 : c.packed ? 1 : 0;
+    }
+    hmk_p1_prepare_candidates<<<(nq * 32 + 255) / 256, 256, 0, st_>>>(state(), nq, capq, d_ac_cnt_.p, d_ac_slot_.p, d_ac_score_.p,
+                                                                     d_ac_full_.p, d_ac_best_.p);
+    CK(cudaGetLastError());
+    launches_++;
+}
+
 int Engine::phase1() {
     int B = (int)opt.batch;
     if (B <= 0) B = fast_ ? (sc_.filter ? 8 : 3) * qt_max() : 192;   // measured optimum on the 1 M workload
@@ -1070,7 +1111,12 @@ int Engine::phase1() {
         CK(cudaMemsetAsync(d_qbatch_.p, 0xff, sizeof(int32_t) * n_, st_));
     }
     hit_cap_ = (size_t)opt.hit_cap;
-    for (auto& b : bb_) b.valid = false;
+    // batch ids restart at 1, so per-length profiles that an earlier run or a batch probe built must not be taken for
+    // this run's batches of the same id
+    for (auto& b : bb_) {
+        b.valid = false;
+        std::fill(std::begin(b.prof_len_batch), std::end(b.prof_len_batch), 0);
+    }
     const int depth = (int)std::max<int64_t>(0, std::min<int64_t>(opt.lookahead, HMK_NBATCHBUF - 1));
     // SMs the side stream's bulk launches leave alone while the main stream works on a batch: one for the resolver,
     // the others for the small kernels around it (new founders, member check), which then never wait for a CTA of a
@@ -1089,27 +1135,12 @@ int Engine::phase1() {
         // A: clusters whose founder scores >= T (part 1 came with the batch; part 2 = the clusters created since), then
         // complete linkage over their members
         sec(SEC_P1_CLUSTER);
-        CK(cudaMemsetAsync(d_ac_cnt_.p, 0, sizeof(int32_t) * nq, st_));
-        if (ncl > 0) {
-            if (ncl > cb.ncl_ahead) {
-                plan_sms_ = (fast_ && reserve > 1) ? reserve - 1 : 0;      // while a prepared partner search holds the other SMs
-                founder_hits(cb, cb.ncl_ahead, ncl, st_, d_sched_);
-                plan_sms_ = 0;
-            }
-            HmkCheckArgs c{};
-            c.S = state(); c.hits = cb.hits.p; c.hit_count = cb.hcount.p; c.hit_cap = (unsigned int)cb.hit_cap;
-            c.hit_t_is_query = 1; c.qids = d_qid; c.sidx = nullptr;
-            c.ac_cnt = d_ac_cnt_.p; c.ac_slot = d_ac_slot_.p; c.ac_score = d_ac_score_.p; c.capq = (int32_t)capq;
-            c.cand_count = cb.hcount.p + 1; c.cand_cap = 0; c.linked = 1;
-            c.packed = fast_scalar_ ? d_packed_.p : nullptr; c.L = max_len_; c.pair_parts = d_pairparts_.p;
-            if (scalar12x3()) hmk_member_check<true><<<sm_count_ * 2, 256, 0, st_>>>(c);
-            else hmk_member_check<false><<<sm_count_ * 2, 256, 0, st_>>>(c);
-            CK(cudaGetLastError());
-            launches_++;
+        if (ncl > cb.ncl_ahead) {
+            plan_sms_ = (fast_ && reserve > 1) ? reserve - 1 : 0;      // while a prepared partner search holds the other SMs
+            founder_hits(cb, cb.ncl_ahead, ncl, st_, d_sched_);
+            plan_sms_ = 0;
         }
-        hmk_p1_prepare_candidates<<<(nq * 32 + 255) / 256, 256, 0, st_>>>(state(), nq, (int)capq, d_ac_cnt_.p, d_ac_slot_.p, d_ac_score_.p,
-                                                                         d_ac_full_.p, d_ac_best_.p);
-        launches_++;
+        check_members(cb, ncl, (int)capq);
         const int ib_stride = (nq + 3) & ~3, pd_stride = (nq * (int)opt.kb + 3) & ~3;
         const int nw = (nq + 31) / 32;
         HmkP1Batch pb{};
@@ -1699,6 +1730,123 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
     kernel[4] = k.fn && p.sched ? 1 : 0;
 }
 
+// Phase 1's per-batch work on a clustering state given by the caller (hmk_batch_probe): the state goes into the
+// context's own buffers, then stage_partner_search and check_members run as phase1 calls them, on the first batch
+// buffer.  Whatever of this a run reads, run() and phase1() set again: the clustering state, the control block, the
+// batch buffers' validity and profile ids, the batch counter, the hit capacity and the pair counters.
+void Engine::batch_probe(const int32_t* member_off, const int32_t* members, int32_t ncl, int32_t cur, int32_t nq, int32_t capq,
+                         int32_t tail_stream, hmk_batch_probe_out* out) {
+    CK(cudaSetDevice(device_));
+    if (!uploaded_ || n_ <= 0 || bad_residue_) throw std::invalid_argument("hmk_batch_probe needs an uploaded, valid input");
+    if (!out || ncl < 0 || ncl > K_ || (ncl && (!member_off || !members)) || cur < 0 || cur > n_ || nq < 1 ||
+        nq > HMK_MAXBATCH || capq < 0 || (out->fhit_cap && !out->fhits) || out->fhit_cap < 0 || !out->qid || !out->bk_key ||
+        !out->bk_cnt || !out->bk_ovf || !out->ib || !out->ibm || !out->ibm2 || !out->pcand || !out->pd || !out->ac_cnt ||
+        !out->ac_slot || !out->ac_score || !out->ac_best)
+        throw std::invalid_argument("hmk_batch_probe: bad argument");
+    if (X_ >= min_len_) throw std::invalid_argument("hmk_batch_probe: max shift not below the shortest length");
+    // ---- the clustering state
+    std::vector<int32_t> ab(n_), slot(n_, -1), rank(n_, 0), next(n_, -1), cf(ncl), cs(ncl), cc(ncl), ct(ncl);
+    CK(cudaMemcpy(ab.data(), d_ab_.p, sizeof(int32_t) * n_, cudaMemcpyDeviceToHost));
+    for (int c = 0; c < ncl; c++) {
+        const int32_t b = member_off[c], e = member_off[c + 1];
+        if (b < 0 || e <= b) throw std::invalid_argument("hmk_batch_probe: member_off must rise, every cluster non-empty");
+        uint32_t size = 0;      // Cluster.size(): Java int sum of the abundances
+        for (int32_t i = b; i < e; i++) {
+            const int32_t m = members[i];
+            if (m < 0 || m >= n_ || slot[m] >= 0) throw std::invalid_argument("hmk_batch_probe: member id out of range or repeated");
+            slot[m] = c; rank[m] = i - b;
+            if (i + 1 < e) next[m] = members[i + 1];
+            size += (uint32_t)ab[m];
+        }
+        cf[c] = members[b]; cs[c] = (int32_t)size; cc[c] = e - b; ct[c] = members[e - 1];
+    }
+    int32_t unproc = 0;
+    for (int i = cur; i < n_; i++) unproc += slot[i] < 0;
+    if (unproc == 0) throw std::invalid_argument("hmk_batch_probe: no singleton at or after cur");
+    CK(cudaMemcpyAsync(d_slot_.p, slot.data(), sizeof(int32_t) * n_, cudaMemcpyHostToDevice, st_));
+    CK(cudaMemcpyAsync(d_rank_.p, rank.data(), sizeof(int32_t) * n_, cudaMemcpyHostToDevice, st_));
+    CK(cudaMemcpyAsync(d_next_.p, next.data(), sizeof(int32_t) * n_, cudaMemcpyHostToDevice, st_));
+    if (ncl) {
+        CK(cudaMemcpyAsync(d_cf_.p, cf.data(), sizeof(int32_t) * ncl, cudaMemcpyHostToDevice, st_));
+        CK(cudaMemcpyAsync(d_cs_.p, cs.data(), sizeof(int32_t) * ncl, cudaMemcpyHostToDevice, st_));
+        CK(cudaMemcpyAsync(d_cc_.p, cc.data(), sizeof(int32_t) * ncl, cudaMemcpyHostToDevice, st_));
+        CK(cudaMemcpyAsync(d_ct_.p, ct.data(), sizeof(int32_t) * ncl, cudaMemcpyHostToDevice, st_));
+    }
+    HmkCtl c0{};
+    c0.cur = cur; c0.ncl = ncl; c0.unproc_alive = unproc; c0.status = HMK_P1_CONTINUE; c0.npe_step = -1;
+    *h_ctl_ = c0;
+    CK(cudaMemcpyAsync(d_ctl_.p, h_ctl_, sizeof(HmkCtl), cudaMemcpyHostToDevice, st_));
+    d_pairparts_.reserve(HMK_PAIR_SHARDS * 16);
+    CK(cudaStreamSynchronize(st_));      // the side streams start from here
+    // ---- one batch, as phase1 runs it (no kept hits for phase 2, every SM for the bulk launches)
+    opt.kb = std::max<int64_t>(1, std::min<int64_t>(opt.kb, 32));      // as phase1
+    const int kb = (int)opt.kb;
+    const int cq = capq > 0 ? capq : (int)std::max<int64_t>(1, opt.capq);
+    nq = std::min(nq, unproc);
+    reuse_ = false;
+    plan_sms_ = 0;
+    hit_cap_ = (size_t)opt.hit_cap;
+    d_ac_cnt_.reserve(nq); d_ac_slot_.reserve((size_t)nq * cq); d_ac_score_.reserve((size_t)nq * cq);
+    d_ac_full_.reserve((size_t)nq * cq); d_ac_best_.reserve(nq);
+    LaunchLog log;
+    struct Unset { LaunchLog*& p; ~Unset() { p = nullptr; } } unset{launch_log_};
+    launch_log_ = &log;
+    BatchBuf& bb = bb_[0];
+    if (tail_stream) stage_partner_search(bb, nq, cur, nullptr, ncl, st2_, st3_);
+    else stage_partner_search(bb, nq, cur, nullptr, ncl, st_, st_);
+    bb.valid = false;
+    CK(cudaStreamWaitEvent(st_, bb.ready, 0));
+    check_members(bb, ncl, cq);
+    // ---- results
+    const int nw = (nq + 31) / 32, ib_stride = (nq + 3) & ~3, pd_stride = (nq * kb + 3) & ~3;
+    std::vector<int32_t> ib((size_t)nq * ib_stride), pd((size_t)nq * pd_stride);
+    std::vector<int4> best(nq);
+    unsigned int hcount = 0;
+    CK(cudaMemcpyAsync(out->qid, bb.qid.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->bk_key, bb.bk_key.p, sizeof(uint64_t) * nq * kb, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->bk_cnt, bb.bk_cnt.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->bk_ovf, bb.bk_ovf.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(ib.data(), bb.ib.p, sizeof(int32_t) * ib.size(), cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->ibm, bb.ibm.p, sizeof(uint32_t) * nq * nw, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->ibm2, bb.ibm2.p, sizeof(uint32_t) * nq * nw, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->pcand, bb.pcand.p, sizeof(int32_t) * nq * kb, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(pd.data(), bb.pd.p, sizeof(int32_t) * pd.size(), cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(&hcount, bb.hcount.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->ac_cnt, d_ac_cnt_.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->ac_slot, d_ac_slot_.p, sizeof(int32_t) * nq * cq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(out->ac_score, d_ac_score_.p, sizeof(int32_t) * nq * cq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(best.data(), d_ac_best_.p, sizeof(int4) * nq, cudaMemcpyDeviceToHost, st_));
+    CK(cudaStreamSynchronize(st_));
+    out->nq_out = nq;
+    for (int b = 0; b < nq; b++) {
+        std::copy_n(&ib[(size_t)b * ib_stride], nq, out->ib + (size_t)b * nq);
+        std::copy_n(&pd[(size_t)b * pd_stride], nq * kb, out->pd + (size_t)b * nq * kb);
+        const int4 r = best[b];
+        out->ac_best[4 * b] = r.x; out->ac_best[4 * b + 1] = r.y; out->ac_best[4 * b + 2] = r.z; out->ac_best[4 * b + 3] = r.w;
+    }
+    out->fhit_count = hcount;
+    const size_t stored = std::min<size_t>({(size_t)hcount, bb.hit_cap, (size_t)out->fhit_cap});
+    if (stored) {
+        std::vector<int4> h(stored);
+        CK(cudaMemcpy(h.data(), bb.hits.p, sizeof(int4) * stored, cudaMemcpyDeviceToHost));
+        for (size_t e = 0; e < stored; e++) { out->fhits[3 * e] = h[e].x; out->fhits[3 * e + 1] = h[e].y; out->fhits[3 * e + 2] = h[e].z; }
+    }
+    const BulkKernel& k = log.last[HMK_MODE_TOPK];
+    const bool packed = k.kind > BulkKernel::GENERIC;
+    int32_t* kr = out->kernel;
+    kr[0] = k.kind;
+    kr[1] = k.lt;
+    kr[2] = packed ? sc_.nw : 0;
+    kr[3] = packed ? (sc_.lane16 ? 16 : 8) : k.fn ? 32 : 0;
+    kr[4] = log.persistent ? 1 : 0;
+    kr[5] = log.count[HMK_MODE_TOPK];
+    kr[6] = log.last[HMK_MODE_DENSE].kind;
+    kr[7] = log.count[HMK_MODE_DENSE];
+    kr[8] = log.last[HMK_MODE_EMIT].kind;
+    kr[9] = log.count[HMK_MODE_EMIT];
+    kr[10] = log.member_check;
+}
+
 // ---------------------------------------------------------------- exact complete-linkage clustering (SURVEY.md 8f N1)
 // ClinkageSequenceClusterer.cluster (ClinkageSequenceClusterer.java:43-124).  n <= opt.clinkage_dense_max: dense pair
 // scores from the bulk kernel, nearest-neighbour chain in hmk_clinkage_chain.  Larger n: the entries scoring >= T only
@@ -2176,6 +2324,15 @@ int hmk_bulk_probe(hmk_ctx* ctx, int32_t mode, const int32_t* query_ids, int32_t
     return guarded(errbuf, errlen, [&] {
         ctx->engine.bulk_probe(mode, query_ids, n_query, db_ids, db_begin, n_db, clustered, keys, counts, overflow, hits,
                                hit_cap, hit_count, kernel);
+        return HMK_STATUS_OK;
+    });
+}
+
+int hmk_batch_probe(hmk_ctx* ctx, const int32_t* member_off, const int32_t* members, int32_t ncl, int32_t cur, int32_t nq,
+                    int32_t capq, int32_t tail_stream, hmk_batch_probe_out* out, char* errbuf, size_t errlen) {
+    if (!ctx) return HMK_STATUS_BAD_ARG;
+    return guarded(errbuf, errlen, [&] {
+        ctx->engine.batch_probe(member_off, members, ncl, cur, nq, capq, tail_stream, out);
         return HMK_STATUS_OK;
     });
 }

@@ -535,6 +535,7 @@ class GreedyContext:
         self._keep = None
         self.n = 0
         self._kb = 8        # option kb (the engine's default): row length of bulk_probe's key lists
+        self._capq = 256    # option capq (the engine's default): rows of batch_probe's candidate arrays
         for k, v in options.items():
             self.set_option(k, v)
 
@@ -543,6 +544,8 @@ class GreedyContext:
             raise ValueError(f"unknown option {name}")
         if name == "kb":
             self._kb = int(value)
+        if name == "capq":
+            self._capq = int(value)
 
     def close(self):
         if self._h:
@@ -705,6 +708,49 @@ class GreedyContext:
                           "lane_bits": int(kern[3]), "persistent": int(kern[4])}}
         if mode == 0:
             out.update(keys=keys[:nq], cnt=cnt[:nq], ovf=ovf[:nq])
+        return out
+
+    def batch_probe(self, clusters, cur: int, nq: int, capq: int = 0, tail_stream: bool = False, fhit_cap: int = 1 << 20):
+        """hmk_batch_probe: phase 1's per-batch inputs of the resolver on the clustering state `clusters` (a list of member
+        id lists in chain order, founder first; everything else is a singleton), batch = the first nq singletons with id
+        >= cur (the kernel tests' hook).  -> dict with "qid", "keys" (uint64 [nq, kb]), "cnt", "ovf", "ib" [nq, nq],
+        "ibm", "ibm2" (uint32 [nq, nw]), "pcand" [nq, kb], "pd" [nq, nq * kb], "fhits" (int32 [k, 3]: query index,
+        founder id, score), "fhit_count", "ac_cnt", "ac_slot", "ac_score" [nq, capq], "ac_best" [nq, 4] and "kernel"."""
+        off = np.zeros(len(clusters) + 1, dtype=np.int32)
+        off[1:] = np.cumsum([len(c) for c in clusters])
+        mem = np.ascontiguousarray(np.concatenate([np.asarray(c, dtype=np.int32) for c in clusters]) if clusters
+                                   else np.zeros(1, dtype=np.int32), dtype=np.int32)
+        kb, nw = self._kb, (nq + 31) // 32
+        cq = capq if capq > 0 else self._capq
+        a = dict(qid=np.zeros(nq, np.int32), keys=np.zeros((nq, kb), np.uint64), cnt=np.zeros(nq, np.int32),
+                 ovf=np.zeros(nq, np.int32), ib=np.zeros((nq, nq), np.int32), ibm=np.zeros((nq, nw), np.uint32),
+                 ibm2=np.zeros((nq, nw), np.uint32), pcand=np.zeros((nq, kb), np.int32), pd=np.zeros((nq, nq * kb), np.int32),
+                 fhits=np.zeros((max(fhit_cap, 1), 3), np.int32), ac_cnt=np.zeros(nq, np.int32),
+                 ac_slot=np.zeros((nq, cq), np.int32), ac_score=np.zeros((nq, cq), np.int32),
+                 ac_best=np.zeros((nq, 4), np.int32))
+        i32, u32 = C.c_int32, C.c_uint32
+        o = _lib.BatchProbeOut(0, _ptr(a["qid"], i32), _ptr(a["keys"], C.c_uint64), _ptr(a["cnt"], i32), _ptr(a["ovf"], i32),
+                               _ptr(a["ib"], i32), _ptr(a["ibm"], u32), _ptr(a["ibm2"], u32), _ptr(a["pcand"], i32),
+                               _ptr(a["pd"], i32), _ptr(a["fhits"], i32), int(fhit_cap), 0, _ptr(a["ac_cnt"], i32),
+                               _ptr(a["ac_slot"], i32), _ptr(a["ac_score"], i32), _ptr(a["ac_best"], i32))
+        err = C.create_string_buffer(512)
+        rc = self._L.hmk_batch_probe(self._h, _ptr(off, i32), _ptr(mem, i32), len(clusters), int(cur), int(nq), int(capq),
+                                     int(bool(tail_stream)), C.byref(o), err, 512)
+        if rc:
+            _raise_status(rc, err.value)
+        n = o.nq_out
+        out = {k: v[:n] for k, v in a.items() if k != "fhits"}
+        out["ib"] = a["ib"].reshape(-1)[:n * n].reshape(n, n)
+        nwn = (n + 31) // 32
+        out["ibm"], out["ibm2"] = (a[k].reshape(-1)[:n * nwn].reshape(n, nwn) for k in ("ibm", "ibm2"))
+        out["pd"] = a["pd"].reshape(-1)[:n * n * kb].reshape(n, n * kb)
+        out["fhits"] = a["fhits"][:min(o.fhit_count, fhit_cap)]
+        out["fhit_count"] = int(o.fhit_count)
+        k = list(o.kernel)
+        out["kernel"] = {"kind": self._KERNELS[k[0]], "filter_lt": k[1], "nw": k[2], "lane_bits": k[3], "persistent": k[4],
+                         "search_launches": k[5], "tables": "dense_packed" if k[6] == -1 else self._KERNELS[k[6]],
+                         "table_launches": k[7], "founder": self._KERNELS[k[8]], "founder_launches": k[9],
+                         "member_check": {-1: "none", 0: "state", 1: "packed", 2: "score12x3"}[k[10]]}
         return out
 
 

@@ -211,6 +211,45 @@ int hmk_bulk_probe(hmk_ctx* ctx, int32_t mode, const int32_t* query_ids, int32_t
                    int32_t* overflow, int32_t* hits, int64_t hit_cap, int64_t* hit_count, int32_t* kernel, char* errbuf,
                    size_t errlen);
 
+/* What hmk_batch_probe returns.  Host arrays owned by the caller, sized for the nq it asks for (kb = option kb,
+ * nw = (nq + 31) / 32, capq as passed or option capq); the first nq_out rows are filled, rows packed without padding. */
+typedef struct {
+    int32_t nq_out;      /* queries of the batch: the first nq singletons with id >= cur, fewer when fewer remain          */
+    int32_t* qid;        /* [nq] their ids, ascending                                                                    */
+    uint64_t* bk_key;    /* [nq][kb] merged partner lists over the later singletons, hmk_bulk_probe's key order          */
+    int32_t* bk_cnt;     /* [nq] list lengths                                                                            */
+    int32_t* bk_ovf;     /* [nq] 1 = more later singletons scored >= threshold than the list holds                      */
+    int32_t* ib;         /* [nq][nq] ib[b][b2] = score(member = qid[b2], query = qid[b])                                 */
+    uint32_t* ibm;       /* [nq][nw] bit b2 (word b2 / 32, bit b2 % 32): b2 < b and ib[b][b2] >= threshold              */
+    uint32_t* ibm2;      /* [nq][nw] bits of ibm whose ib also reaches the lowest score of b's list (none: empty list)   */
+    int32_t* pcand;      /* [nq][kb] ids of the partner lists, padded with the query's own id                           */
+    int32_t* pd;         /* [nq][nq * kb] pd[b][e] = score(member = pcand[e], query = qid[b])                             */
+    int32_t* fhits;      /* [fhit_cap][3] founder hits: (query index, founder id, score >= threshold)                    */
+    int64_t fhit_cap;
+    int64_t fhit_count;  /* founder hits found (may exceed fhit_cap; then fhit_cap are stored)                           */
+    int32_t* ac_cnt;     /* [nq] clusters whose founder hit and every other member score >= threshold (may exceed capq) */
+    int32_t* ac_slot;    /* [nq][capq] the first min(ac_cnt, capq) of them, in no particular order                       */
+    int32_t* ac_score;   /* [nq][capq] their complete-linkage score: the minimum over all members                        */
+    int32_t* ac_best;    /* [nq][4] the best of them as (score, abundance-weighted size, founder id, cluster); -1: none  */
+    /* kernels that ran: [0..4] the partner search as hmk_bulk_probe's kernel[5], [5] partner-search launches (one per
+     * length bucket with later singletons on mixed lengths), [6] kind of the bulk kernel that made ib and pd (-1: the
+     * one-thread-per-pair hmk_dense_packed), [7] its launches, [8] kind of the founder filter (-1: none ran), [9] its
+     * launches, [10] scorer of the member check: 0 hmk_state_score, 1 hmk_packed_pair_score, 2 hmk_score12x3, -1 none */
+    int32_t kernel[11];
+} hmk_batch_probe_out;
+
+/* Phase 1's per-batch work on a given clustering state, for the kernel tests.  Writes the state into the context --
+ * members[member_off[c] .. member_off[c + 1]) are cluster c's members in chain order, founder first, for ncl <=
+ * max_clusters clusters; every other sequence is a singleton -- with cur as the first unvisited id.  Then runs what a
+ * run runs for one batch: the partner search with its tail (merged lists, score tables and masks) and the founder filter
+ * on one stream (tail_stream 0) or the tail on a second stream (tail_stream 1), then the member check and the candidate
+ * records.  capq: rows of the candidate arrays per query (0 = option capq).  A later hmk_run starts from a clean state.
+ * Unlike a run, the bulk launches are planned for every SM (a run's look-ahead leaves some to the resolver), and
+ * tail_stream 1 always puts the tail on the tail stream (a run's look-ahead does so on the packed paths; on the generic
+ * path it stages a whole batch on one side stream). */
+int hmk_batch_probe(hmk_ctx* ctx, const int32_t* member_off, const int32_t* members, int32_t ncl, int32_t cur, int32_t nq,
+                    int32_t capq, int32_t tail_stream, hmk_batch_probe_out* out, char* errbuf, size_t errlen);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1,5 +1,5 @@
 """Builds the library with -DHMK_CHECKED (in-kernel bounds assertions, hmk_common.h) next to the normal one and runs the
-bulk-kernel tests, the randomised differential tier, the boundary tests and the clinkage tests (dense and sparse path) against it (HMK_LIB selects the library the
+bulk-kernel and batch-table tests, the randomised differential tier, the boundary tests and the clinkage tests (dense and sparse path) against it (HMK_LIB selects the library the
 host layer loads).  A failing assertion prints `file:line: ... Assertion ... failed` from the device and the call
 returns HMK_STATUS_CUDA, so the test fails with the line in the log.  compute-sanitizer is not available on the pool.
 
@@ -18,7 +18,8 @@ def main():
     hb_build.build(force=True, defines=["HMK_CHECKED"], out=lib)
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     env = dict(os.environ, HMK_LIB=lib)
-    cmd = [sys.executable, "-m", "pytest", "-m", "gpu", "-q", "-x", "tests/test_bulk_kernels.py", "tests/test_gpu_fuzz.py",
+    cmd = [sys.executable, "-m", "pytest", "-m", "gpu", "-q", "-x", "tests/test_bulk_kernels.py", "tests/test_batch_tables.py",
+           "tests/test_gpu_fuzz.py",
            "tests/test_gpu_boundary.py", "tests/test_clinkage.py", "tests/test_clinkage_large.py", "tests/test_gpu_parity.py",
            "tests/test_p1_pipeline.py"] + sys.argv[1:]
     with open(os.path.join(ROOT, "gpurun_out", "checked_fuzz.log"), "w") as log:
