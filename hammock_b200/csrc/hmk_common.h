@@ -146,6 +146,18 @@ HMK_UNROLL
     for (int j = 0; j < HMK_MAXL1; j++) qrow[j] = (int32_t)((uint32_t)(wq >> (5 * j)) & 31u) * HMK_NRES;
 }
 
+// Residue prefix shared by a warp's items (hmk_bulk_filter).  The filter bound is a u32 sum over positions, so where
+// every scored lane of a warp holds the same residues 0 .. HMK_PREFIX_RES - 1, their rows are summed once per query for
+// the warp instead of once per lane.  The warp reduces the lanes' prefix keys to their least (hmk_prefix_lo) and
+// greatest (hmk_prefix_hi) value; a lane whose item is not scored adds the neutral value of each reduction, so the two
+// agree exactly when the scored lanes share the prefix, and never for a warp without a scored lane.
+#define HMK_PREFIX_RES 3
+HMK_HD uint32_t hmk_prefix_key(uint64_t w) { return (uint32_t)w & ((1u << (5 * HMK_PREFIX_RES)) - 1u); }
+HMK_HD uint32_t hmk_prefix_lo(uint64_t w, bool scored) { return scored ? hmk_prefix_key(w) : 0xffffffffu; }
+HMK_HD uint32_t hmk_prefix_hi(uint64_t w, bool scored) { return scored ? hmk_prefix_key(w) : 0u; }
+// residues shared (HMK_PREFIX_RES or 0) given kmin = min over the warp of hmk_prefix_lo, kmax = max of hmk_prefix_hi
+HMK_HD int hmk_prefix_shared(uint32_t kmin, uint32_t kmax) { return kmin == kmax ? HMK_PREFIX_RES : 0; }
+
 // status codes of the engine / C ABI (include/hammock_b200.h)
 enum {
     HMK_OK = 0,

@@ -641,8 +641,10 @@ int Engine::qt_max(const HmkScheme& sc) const {
     if (opt.qt > 0) return (int)opt.qt;
     // a profile with its share of the carve-up, beside the hit queues of a 768-thread block and 128 bytes for the barrier
     // and alignment.  The 512-thread long kernel is sized the same way: its tiles are the ones it was measured with.
-    const size_t per = (size_t)sc.prof_words * 4 + hmk_carve_bytes(1, (int)opt.kb, 0, false);
-    const size_t fixed = 128 + hmk_carve_bytes(0, (int)opt.kb, HMK_BULK_THREADS, false);
+    // The filter kernel adds a prefix sum per profile and warp (hmk_packed_smem), with up to 12 bytes of alignment per warp.
+    const size_t warps = HMK_BULK_THREADS / 32;
+    const size_t per = (size_t)sc.prof_words * 4 + hmk_carve_bytes(1, (int)opt.kb, 0, false) + (sc.filter ? warps * 4 : 0);
+    const size_t fixed = 128 + hmk_carve_bytes(0, (int)opt.kb, HMK_BULK_THREADS, false) + (sc.filter ? 16 + warps * 12 : 0);
     // the filter kernel's tile stays at the 56 profiles the batch size and chunking were measured with (more would fit)
     const size_t cap = sc.filter ? HMK_FILTER_QT : 255;
     return (int)std::min<size_t>(cap, std::max<size_t>(1, (smem_optin_ - fixed) / per));
@@ -756,7 +758,7 @@ BulkKernel Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch,
     size_t smem;
     void* args[1];
     if (sch) {
-        smem = hmk_packed_smem(a.qt, (uint32_t)sch->prof_words * 4, a.kb, k.threads).total;
+        smem = hmk_packed_smem(a.qt, (uint32_t)sch->prof_words * 4, a.kb, k.threads, k.kind == BulkKernel::FILTER).total;
         args[0] = &a;
     } else {
         g.b = a; g.prof_ids = prof_ids; g.prof_is_query = prof_is_query;

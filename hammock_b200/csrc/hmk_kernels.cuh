@@ -17,6 +17,7 @@
 // (cp.async.bulk + mbarrier; SASS UBLKCP).
 #pragma once
 #include <cooperative_groups.h>
+#include <type_traits>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -438,17 +439,21 @@ __host__ __device__ inline size_t hmk_carve_bytes(int qt, int kb, int threads, b
 
 // ---------------------------------------------------------------- pieces shared by the bulk kernels
 // Packed kernels' shared memory: the profile tile (qt profiles of pwb bytes) from offset 0, the TMA barrier at `bar`,
-// the carve-up for `threads` threads at `carve`; `total` is a launch's dynamic size.
-struct HmkPackedSmem { size_t bar, carve, total; };
-__host__ __device__ inline HmkPackedSmem hmk_packed_smem(int qt, uint32_t pwb, int kb, int threads) {
+// the carve-up for `threads` threads at `carve`, and for the filter kernel the warps' prefix sums at `pfx`
+// (hmk_pfx_words(qt) u32 per warp, 16-byte aligned); `total` is a launch's dynamic size.
+struct HmkPackedSmem { size_t bar, carve, pfx, total; };
+__host__ __device__ inline int hmk_pfx_words(int qt) { return (qt + 3) & ~3; }
+__host__ __device__ inline HmkPackedSmem hmk_packed_smem(int qt, uint32_t pwb, int kb, int threads, bool filter) {
     const size_t bar = ((size_t)qt * pwb + 15) & ~(size_t)15;
-    return {bar, bar + 16, bar + 16 + hmk_carve_bytes(qt, kb, threads, false)};
+    const size_t end = bar + 16 + hmk_carve_bytes(qt, kb, threads, false);
+    const size_t pfx = (end + 15) & ~(size_t)15;
+    return {bar, bar + 16, pfx, filter ? pfx + (size_t)(threads / 32) * hmk_pfx_words(qt) * 4 : end};
 }
 
 // carves a packed kernel's shared memory and initialises the tile barrier (visible after the next __syncthreads)
 __device__ __forceinline__ uint64_t* hmk_packed_carve(unsigned char* smem, const HmkBulkArgs& a, uint32_t pwb, HmkTopkSmem& tk,
                                                       HmkHitQueue& hq) {
-    const HmkPackedSmem ly = hmk_packed_smem(a.qt, pwb, a.kb, blockDim.x);
+    const HmkPackedSmem ly = hmk_packed_smem(a.qt, pwb, a.kb, blockDim.x, false);
     hmk_carve(smem + ly.carve, a.qt, a.kb, false, tk, hq);
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem + ly.bar);
     if (threadIdx.x == 0) hmk_mbar_init(bar, 1);
@@ -638,6 +643,9 @@ __device__ __forceinline__ int hmk_nth_bit(uint32_t m, int n) {
 // hands them out into a round of 32 held in registers, one candidate per lane, fetching the item's packed
 // word from the owning lane by shuffle; a part-filled round is carried into the next group and is verified
 // when it is full or when the chunk ends.
+// At the fixed length, an item block whose scored lanes share residues 0..2 (three warps in four on the clustering-order
+// walk) takes the sum of those three filter rows per query from a per-warp array instead: 9 look-ups plus a quarter of
+// a broadcast LDS.128 per query, against 12.
 // LT: compile-time length (0 = use sc.L; then the twelve look-ups are predicated, which costs issue slots)
 template <int MODE, int LT>
 __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __grid_constant__ HmkBulkArgs a) {
@@ -645,6 +653,9 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
     constexpr uint32_t PWB = HMK_FPW * 4;
     constexpr uint32_t SUB = HMK_MAXL1 * HMK_ROWB;   // bytes of one sub-table
     constexpr int OCT_UNROLL = LT ? 2 : 1;
+    // shared residue prefixes (below) in the partner search (TOPK) at a fixed length only: with them the general-length
+    // TOPK build spills at 80 registers, and the founder filter's launches (EMIT, a few profiles per tile) got slower
+    constexpr bool PREFIX = MODE == HMK_MODE_TOPK && LT >= HMK_PREFIX_RES;
     __shared__ int s_next[3];                         // persistent mode: (tile, chunk, output slot) of the next piece of work
     const int L = LT ? LT : a.sc.L;
     HMK_CHECK(!a.prof_cells);                         // a CTA may score several tiles (hmk_count_scored)
@@ -657,6 +668,9 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
     const int32_t dec = a.sc.T - a.sc.half;
     const unsigned char* sbase = smem_raw;
     const int lane = threadIdx.x & 31;
+    // this warp's prefix sums: pfx[t] = the filter rows 0 .. HMK_PREFIX_RES - 1 of query t at the residues its items share
+    uint32_t* pfx = reinterpret_cast<uint32_t*>(smem_raw + hmk_packed_smem(a.qt, PWB, a.kb, blockDim.x, true).pfx) +
+                    (threadIdx.x >> 5) * hmk_pfx_words(a.qt);
     const bool persistent = a.sched != nullptr;
     int cur_tile = -1, slot = 0, q0 = 0, qn = 0, home = blockIdx.x % a.nqt;
     uint32_t bar_phase = 0;
@@ -749,16 +763,28 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
             const bool valid = hmk_item(a, i, i_end, 0, id);
             if (!__any_sync(0xffffffffu, valid)) continue;
             const uint64_t w = valid ? a.packed[id] : 0ull;
-            const unsigned char* rowp[HMK_MAXL1];   // &filter[t][j][residue_j]
             if (valid) scored += qn;
-
-            auto bound = [&](const int tu) -> uint32_t {
-                uint32_t f = 0;
+            // Items are walked in id order, the clustering order (abundance, then sequence, descending), so the scored
+            // lanes of most warps share their first residues.  Then the filter rows of those positions are summed once
+            // per query into pfx (lane l: queries l, l + 32, ...) and the query loop below looks up the other rows only.
+            // u32 addition is associative: every bound is bit for bit the full twelve-row sum.
+            bool shared = false;
+            if (PREFIX) {
+                const uint32_t kmin = __reduce_min_sync(0xffffffffu, hmk_prefix_lo(w, valid));
+                const uint32_t kmax = __reduce_max_sync(0xffffffffu, hmk_prefix_hi(w, valid));
+                shared = hmk_prefix_shared(kmin, kmax) == HMK_PREFIX_RES;
+                if (shared) {
+                    for (int t = lane; t < qn; t += 32) {
+                        const unsigned char* pt = sbase + (uint32_t)t * PWB + 2 * SUB;
+                        uint32_t f = 0;
 #pragma unroll
-                for (int j = 0; j < HMK_MAXL1; j++)
-                    if (j < L) f += *reinterpret_cast<const uint32_t*>(rowp[j] + tu * PWB);
-                return f;
-            };
+                        for (int j = 0; j < HMK_PREFIX_RES; j++)
+                            f += *reinterpret_cast<const uint32_t*>(pt + j * HMK_ROWB + ((kmin >> (5 * j)) & 31u) * 4u);
+                        pfx[t] = f;
+                    }
+                    __syncwarp();
+                }
+            }
             // bit k of m0 / m1: a filter byte of exact word 0 / word 1 passed against query g0 + k.  They are built an
             // octet of queries at a time: x = (x >> 1) | (f & 0x80808080) over c <= 8 queries leaves query q's top bit
             // of filter byte b at bit 8b + q + 8 - c (two instructions per query; no bit crosses into the byte below
@@ -810,43 +836,61 @@ __global__ void __launch_bounds__(HMK_BULK_THREADS, 1) hmk_bulk_filter(const __g
                 }
             };
 
-            int t = 0;
-            for (int g0 = 0; g0 < qn; g0 += HMK_FGROUP) {
-                const int gend = min(qn, g0 + HMK_FGROUP);
-                // set up per group, so that the pointers are not live while the group's candidates are handed out
+            // the queries of the tile; U = residues whose rows come from pfx (a compile-time 0 or HMK_PREFIX_RES: a row
+            // predicated off at run time would still take an issue slot)
+            auto scan = [&](auto prefix) {
+                constexpr int U = decltype(prefix)::value;
+                const unsigned char* rowp[HMK_MAXL1];   // &filter[t][j][residue_j], j >= U
+                // f = pfx[t + tu] (p, when U > 0) + the rows j >= U of query t + tu
+                auto bound = [&](const int tu, const uint32_t p) -> uint32_t {
+                    uint32_t f = U ? p : 0u;
 #pragma unroll
-                for (int j = 0; j < HMK_MAXL1; j++)
-                    rowp[j] = sbase + (uint32_t)g0 * PWB + 2 * SUB + j * HMK_ROWB + (uint32_t)((w >> (5 * j)) & 31u) * 4u;
-                for (; t + 8 <= gend; t += 8) {
-                    uint32_t x = 0;
-                    // two blocks of four queries; unrolled only at a fixed length, where the predicate-free look-ups
-                    // leave the registers for it (the general-length build would spill)
+                    for (int j = U; j < HMK_MAXL1; j++)
+                        if (j < L) f += *reinterpret_cast<const uint32_t*>(rowp[j] + tu * PWB);
+                    return f;
+                };
+                int t = 0;
+                for (int g0 = 0; g0 < qn; g0 += HMK_FGROUP) {
+                    const int gend = min(qn, g0 + HMK_FGROUP);
+                    // set up per group, so that the pointers are not live while the group's candidates are handed out
+#pragma unroll
+                    for (int j = U; j < HMK_MAXL1; j++)
+                        rowp[j] = sbase + (uint32_t)g0 * PWB + 2 * SUB + j * HMK_ROWB + (uint32_t)((w >> (5 * j)) & 31u) * 4u;
+                    for (; t + 8 <= gend; t += 8) {
+                        uint32_t x = 0;
+                        // two blocks of four queries; unrolled only at a fixed length, where the predicate-free look-ups
+                        // leave the registers for it (the general-length build would spill)
 #pragma unroll OCT_UNROLL
-                    for (int u = 0; u < 2; u++) {
-                        const uint32_t f0 = bound(0), f1 = bound(1), f2 = bound(2), f3 = bound(3);
-                        x = (x >> 1) | (f0 & 0x80808080u); x = (x >> 1) | (f1 & 0x80808080u);
-                        x = (x >> 1) | (f2 & 0x80808080u); x = (x >> 1) | (f3 & 0x80808080u);
+                        for (int u = 0; u < 2; u++) {
+                            // t + 4u is a multiple of 4: one broadcast LDS.128 for the four queries' prefix sums
+                            const uint4 p = U ? *reinterpret_cast<const uint4*>(pfx + t + 4 * u) : make_uint4(0u, 0u, 0u, 0u);
+                            const uint32_t f0 = bound(0, p.x), f1 = bound(1, p.y), f2 = bound(2, p.z), f3 = bound(3, p.w);
+                            x = (x >> 1) | (f0 & 0x80808080u); x = (x >> 1) | (f1 & 0x80808080u);
+                            x = (x >> 1) | (f2 & 0x80808080u); x = (x >> 1) | (f3 & 0x80808080u);
 #pragma unroll
-                        for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += 4 * PWB;
+                            for (int j = U; j < HMK_MAXL1; j++) rowp[j] += 4 * PWB;
+                        }
+                        octet(x, 8);
                     }
-                    octet(x, 8);
-                }
-                if (t < gend) {                             // last, part-filled octet of the group
-                    const int c = gend - t;
-                    uint32_t x = 0;
-                    for (; t < gend; t++) {
-                        x = (x >> 1) | (bound(0) & 0x80808080u);
+                    if (t < gend) {                             // last, part-filled octet of the group
+                        const int c = gend - t;
+                        uint32_t x = 0;
+                        for (; t < gend; t++) {
+                            x = (x >> 1) | (bound(0, U ? pfx[t] : 0u) & 0x80808080u);
 #pragma unroll
-                        for (int j = 0; j < HMK_MAXL1; j++) rowp[j] += PWB;
+                            for (int j = U; j < HMK_MAXL1; j++) rowp[j] += PWB;
+                        }
+                        octet(x, c);
                     }
-                    octet(x, c);
+                    const int octets = (gend - g0 + 7) >> 3;     // the first octet sits in the lowest byte
+                    m0 >>= 8 * (4 - octets);
+                    m1 >>= 8 * (4 - octets);
+                    resolve(g0);
+                    m0 = 0; m1 = 0;
                 }
-                const int octets = (gend - g0 + 7) >> 3;     // the first octet sits in the lowest byte
-                m0 >>= 8 * (4 - octets);
-                m1 >>= 8 * (4 - octets);
-                resolve(g0);
-                m0 = 0; m1 = 0;
-            }
+            };
+            if (PREFIX && shared) scan(std::integral_constant<int, PREFIX ? HMK_PREFIX_RES : 0>());
+            else scan(std::integral_constant<int, 0>());
         }
         if (rfill) verify();      // the round must be empty before the tile (and with it q0) can change
     }
