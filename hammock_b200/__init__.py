@@ -11,6 +11,7 @@ from .host import (ALPHABET, Cluster, CudaError, DataException, FileFormatExcept
                    pack_sequences, rebuild_clusters, run_greedy_clustering, set_greedy_threshold, sort_sequences,
                    get_sorted_labels, java_hashmap_order, save_cluster_sequences_to_csv,
                    save_cluster_sequences_to_csv_ordered, save_clusters_to_csv, save_input_statistics, result_digest, ClinkageSequenceClusterer, UnsupportedInput,
-                   clinkage_cluster_arrays, run_clinkage_clustering, set_clinkage_threshold)
+                   clinkage_cluster_arrays, run_clinkage_clustering, set_clinkage_threshold, EDGE_DTYPE, score_graph,
+                   save_score_graph)
 
 __all__ = [n for n in dir() if not n.startswith("_")]

@@ -37,8 +37,11 @@ HMK_HD int32_t hmk_wmul(int32_t a, int32_t b) { return (int32_t)((uint32_t)a * (
 // Requires max_shift < shorter length (checked by the caller -> status 1).
 // `st1` / `st2`: element strides of the two residue arrays (1 = contiguous; the generic bulk kernel keeps the thread-side
 // sequences position-major in shared memory, stride = block size).
+// `shift` (may be NULL; the callers that only want the score pass NULL and compile to the score-only loop) receives
+// what ShiftedScorer.scoreWithShift reports (:86-93): the lowest diagonal reaching the best score, negated when seq1 is
+// the shorter sequence.
 HMK_HD int32_t hmk_pair_score_strided(const uint8_t* seq1, int st1, int len1, const uint8_t* seq2, int st2, int len2,
-                                      const int32_t* M, int X, int P) {
+                                      const int32_t* M, int X, int P, int* shift = nullptr) {
     const uint8_t* s;
     const uint8_t* l;
     int ls, ll, ss, sl;
@@ -46,6 +49,7 @@ HMK_HD int32_t hmk_pair_score_strided(const uint8_t* seq1, int st1, int len1, co
     else              { s = seq1; ls = len1; ss = st1; l = seq2; ll = len2; sl = st2; }
     const int d = ll - ls;
     int32_t best = HMK_JMIN;
+    int best_k = 0;
     for (int k = -X; k <= X + d; k++) {
         // longer index j pairs with shorter index j-k
         int j0 = k > 0 ? k : 0;
@@ -55,13 +59,19 @@ HMK_HD int32_t hmk_pair_score_strided(const uint8_t* seq1, int st1, int len1, co
         sc = hmk_wadd(sc, hmk_wmul(d, P));
         if (k < 0) sc = hmk_wadd(sc, hmk_wmul(-2 * k, P));
         if (k > d) sc = hmk_wadd(sc, hmk_wmul(2 * (k - d), P));
-        if (sc > best) best = sc;
+        if (sc > best) { best = sc; best_k = k; }
     }
+    if (shift) *shift = len1 >= len2 ? best_k : -best_k;
     return best;
 }
 HMK_HD int32_t hmk_pair_score(const uint8_t* seq1, int len1, const uint8_t* seq2, int len2,
                               const int32_t* M, int X, int P) {
     return hmk_pair_score_strided(seq1, 1, len1, seq2, 1, len2, M, X, P);
+}
+// ShiftedScorer.scoreWithShift(seq1, seq2) (ShiftedScorer.java:48-95, AligningScorerResult = score + shift)
+HMK_HD int32_t hmk_score_with_shift(const uint8_t* seq1, int len1, const uint8_t* seq2, int len2,
+                                    const int32_t* M, int X, int P, int* shift) {
+    return hmk_pair_score_strided(seq1, 1, len1, seq2, 1, len2, M, X, P, shift);
 }
 
 // cells / shifts summed by one pair score (SURVEY.md 3.2) -- work accounting only

@@ -182,6 +182,7 @@ struct Options {
     int64_t xhit_cap = 0;         // capacity of the kept-hit buffer (0 = automatic: the last run's need, else 96 per sequence)
     int64_t clinkage_dense_max = 32768;   // exact complete linkage: largest n that takes the dense n x n path
     int64_t clinkage_threads = 0;         // threads of the sparse chain kernel (0 = automatic, from the row lengths)
+    int64_t graph_cap = 0;                // score graph: hits one query batch may hold (0 = automatic, 1 << 22; at least n)
 };
 
 class Engine {
@@ -254,6 +255,8 @@ public:
     void batch_probe(const int32_t* member_off, const int32_t* members, int32_t ncl, int32_t cur, int32_t nq, int32_t capq,
                      int32_t tail_stream, hmk_batch_probe_out* out);
     int clinkage(const hmk_greedy_in* in, hmk_greedy_out* out);
+    int score_graph(int64_t* cursor, hmk_graph_edge* out, int64_t cap, int64_t* n_out);
+    int score_pairs(const int32_t* seq1, const int32_t* seq2, int32_t np, int32_t* scores, int32_t* shifts);
     std::string status_msg;      // details of the last non-zero status, when there are any
     hmk_stats stats{};
     int error_step = -1;
@@ -371,6 +374,21 @@ private:
     DevBuf<uint64_t> d_clrows_, d_clalt_;
     DevBuf<int32_t> d_cltwin_, d_clrel_;
     int clinkage_rows(int* threads);
+    size_t emit_hits(int q0, int sn, size_t cap, bool count = true);
+    // score graph: the batch of query rows [q0, q1) kept on the device as edges in graph order, row r's edges at
+    // row_off[r - q0] .. row_off[r - q0 + 1]; (next_i, next_r) = the cursor the last hmk_score_graph call returned
+    struct GraphBatch {
+        bool valid = false;
+        int q0 = 0, q1 = 0, sn = HMK_MAXBATCH;   // sn: queries the next batch tries (cut while a batch overflows)
+        std::vector<int64_t> row_off;
+        int64_t next_i = -1, next_r = -1;
+        DevBuf<unsigned long long> key[2], val[2];
+        DevBuf<unsigned int> kept;
+        DevBuf<int4> edges;
+    } graph_;
+    void graph_batch(int q0);
+    void shift_pass(const int4* pairs, const unsigned int* count, unsigned int cap, int q0, int jbits,
+                    unsigned long long* keys, unsigned long long* vals, unsigned int* kept, int32_t* score, int32_t* shift);
     bool lsort_ = false;
     // phase-1 partner-search hits kept for phase 2 (opt.reuse): buffer, 64-bit counters [0] appended, [1] valid
     DevBuf<int4> d_xhits_;
@@ -539,6 +557,7 @@ void Engine::upload(const hmk_greedy_in* in) {
     CK(cudaSetDevice(device_));
     uploaded_ = false;      // a rejected upload leaves nothing to run
     ran_ = false;
+    graph_.valid = false; graph_.next_i = graph_.next_r = -1; graph_.sn = HMK_MAXBATCH;
     if (!in || in->n < 0 || (in->n > 0 && (!in->residues || !in->offsets || !in->abundance)) || !in->matrix)
         throw std::invalid_argument("hmk_upload: null input");
     if (in->n > 0 && in->offsets[0] != 0) throw std::invalid_argument("hmk_upload: offsets[0] must be 0");
@@ -1972,27 +1991,9 @@ int Engine::clinkage_rows(int* threads) {
     d_cldeg_.reserve((size_t)n + 1); d_cloff_.reserve((size_t)n + 1);
     CK(cudaMemsetAsync(d_cldeg_.p, 0, sizeof(unsigned long long) * ((size_t)n + 1), st_));
     d_hits_.reserve(std::max<size_t>(d_hits_.cap, (size_t)1 << 20));
-    auto score_batch = [&](int q0, int sn) {
-        CK(cudaMemsetAsync(d_counts_.p, 0, sizeof(unsigned int), st_));
-        if (fast_) launch_profiles(HMK_PROF_QUERY, d_sidx_.p + q0, sn, d_prof_.p, sc_, st_);
-        HmkBulkArgs a{};
-        a.prof = d_prof_.p; a.nq = sn;
-        a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = q0; a.ndb = n - q0;
-        a.hits = d_hits_.p; a.hit_count = d_counts_.p; a.hit_cap = (unsigned int)std::min<size_t>(d_hits_.cap, UINT32_MAX);
-        launch_bulk(HMK_MODE_EMIT, a, d_sidx_.p + q0, 1);
-        stats.bulk_pairs += (int64_t)sn * (n - q0);
-    };
     const int grid = sm_count_ * 4;
     for (int q0 = 0; q0 < n; q0 += chunk) {          // pass 1: entries per row
-        const int sn = std::min(chunk, n - q0);
-        for (;;) {
-            score_batch(q0, sn);
-            CK(cudaMemcpyAsync(h_scalars_, d_counts_.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st_));
-            CK(cudaStreamSynchronize(st_));
-            const size_t cnt = *reinterpret_cast<unsigned int*>(h_scalars_);
-            if (cnt <= d_hits_.cap) break;
-            d_hits_.reserve(cnt + cnt / 4);          // the hit counter kept counting past the capacity: re-run the batch
-        }
+        emit_hits(q0, std::min(chunk, n - q0), 0);
         hmk_cl_count_hits<<<grid, 256, 0, st_>>>(d_hits_.p, d_counts_.p, (unsigned int)d_hits_.cap, q0, n, d_cldeg_.p);
         CK(cudaGetLastError());
         launches_++;
@@ -2035,7 +2036,7 @@ int Engine::clinkage_rows(int* threads) {
     stats.xhits_capacity = (int64_t)d_clrows_.cap;
     CK(cudaMemsetAsync(d_cldeg_.p, 0, sizeof(unsigned long long) * ((size_t)n + 1), st_));
     for (int q0 = 0; q0 < n; q0 += chunk) {          // pass 2: the same hits (the buffer already fits every batch), scattered
-        score_batch(q0, std::min(chunk, n - q0));
+        emit_hits(q0, std::min(chunk, n - q0), d_hits_.cap, false);
         hmk_cl_scatter_hits<<<grid, 256, 0, st_>>>(d_hits_.p, d_counts_.p, (unsigned int)d_hits_.cap, q0, n, d_cloff_.p,
                                                    d_cldeg_.p, d_clrows_.p);
         CK(cudaGetLastError());
@@ -2068,6 +2069,187 @@ int Engine::clinkage_rows(int* threads) {
     int t = 128;
     while (t < HMK_CL_THREADS && (size_t)t * n < E) t *= 2;
     *threads = opt.clinkage_threads > 0 ? (int)opt.clinkage_threads : t;
+    return HMK_OK;
+}
+
+// One query batch of the upper-triangle pair search (clinkage_rows, the score graph): the bulk kernel's EMIT mode scores
+// the queries [q0, q0 + sn) (profiles, seq2; d_sidx_[q0 ..] holds their ids) against the thread-side ids [q0, n) (seq1)
+// and writes every pair scoring >= T to d_hits_ as (query - q0, thread-side id, score); pairs with id <= query are among
+// them and are the caller's to drop.  Returns the hit count (count = false: returns 0 without waiting for the batch).
+// cap == 0: a batch whose hits overflow d_hits_ is re-run with a bigger buffer; else at most cap (<= d_hits_.cap) hits
+// are stored, and a count above cap tells the caller to split the batch.
+size_t Engine::emit_hits(int q0, int sn, size_t cap, bool count) {
+    for (;;) {
+        const size_t c = cap ? cap : d_hits_.cap;
+        CK(cudaMemsetAsync(d_counts_.p, 0, sizeof(unsigned int), st_));
+        if (fast_) launch_profiles(HMK_PROF_QUERY, d_sidx_.p + q0, sn, d_prof_.p, sc_, st_);
+        HmkBulkArgs a{};
+        a.prof = d_prof_.p; a.nq = sn;
+        a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = q0; a.ndb = n_ - q0;
+        a.hits = d_hits_.p; a.hit_count = d_counts_.p; a.hit_cap = (unsigned int)std::min<size_t>(c, UINT32_MAX);
+        launch_bulk(HMK_MODE_EMIT, a, d_sidx_.p + q0, 1);
+        stats.bulk_pairs += (int64_t)sn * (n_ - q0);
+        if (!count) return 0;
+        CK(cudaMemcpyAsync(h_scalars_, d_counts_.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st_));
+        CK(cudaStreamSynchronize(st_));
+        const size_t cnt = *reinterpret_cast<unsigned int*>(h_scalars_);
+        if (cap || cnt <= d_hits_.cap) return cnt;
+        d_hits_.reserve(cnt + cnt / 4);          // the hit counter kept counting past the capacity: re-run the batch
+    }
+}
+
+// hmk_score_shift over `cap` pairs (graph: the first min(*count, cap) EMIT hits of the batch at q0)
+void Engine::shift_pass(const int4* pairs, const unsigned int* count, unsigned int cap, int q0, int jbits,
+                        unsigned long long* keys, unsigned long long* vals, unsigned int* kept, int32_t* score, int32_t* shift) {
+    HmkShiftArgs s{};
+    s.pairs = pairs; s.count = count; s.cap = cap; s.q0 = q0; s.jbits = jbits;
+    s.res = d_res_.p; s.off = d_off_.p; s.M = d_M_.p; s.X = X_; s.P = P_; s.n = n_;
+    s.keys = keys; s.vals = vals; s.kept = kept; s.score = score; s.shift = shift;
+    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(sm_count_ * 8, ((int64_t)cap + 255) / 256));
+    hmk_score_shift<<<grid, 256, 0, st_>>>(s);
+    CK(cudaGetLastError());
+    launches_++;
+}
+
+// ---------------------------------------------------------------- score graph (hmk_score_graph)
+static_assert(sizeof(hmk_graph_edge) == sizeof(int4), "hmk_graph_edge is copied from the int4 edges of hmk_graph_edges");
+// Every pair i < j with scoreWithShift(seq1 = j, seq2 = i) >= T, as (i, j, score, shift) ordered by i, then j: the
+// upper-triangle pairs emit_hits finds (the same pairs clinkage_rows keeps), the shift of each from hmk_score_shift, and
+// a radix sort of the batch on (i, j).  Device memory is bounded by one batch: a batch whose hits overflow the buffer
+// (at least n entries, so that one query always fits) is re-run with fewer queries.
+void Engine::graph_batch(int q0) {
+    GraphBatch& g = graph_;
+    g.valid = false;
+    const int n = n_;
+    const size_t H = std::min<size_t>(UINT32_MAX, std::max<size_t>(opt.graph_cap > 0 ? (size_t)opt.graph_cap : (size_t)1 << 22, (size_t)n));
+    // every buffer at its bound before the timed passes: no allocation inside a batch
+    d_hits_.reserve(H);
+    if (fast_) d_prof_.reserve((size_t)HMK_MAXBATCH * sc_.prof_words);
+    for (auto& b : g.key) b.reserve(H);
+    for (auto& b : g.val) b.reserve(H);
+    g.kept.reserve(HMK_MAXBATCH + 1);
+    g.edges.reserve(H);
+    {
+        cub::DoubleBuffer<unsigned long long> dk(g.key[0].p, g.key[1].p), dv(g.val[0].p, g.val[1].p);
+        size_t bytes = 0;
+        CK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, dk, dv, (int)H, 0, 64, st_));
+        d_cub_.reserve(bytes);
+    }
+    int sn = std::min(g.sn, n - q0);
+    std::vector<int32_t> ids(sn);      // profile ids (d_sidx_ also serves phase 2 as an index map)
+    std::iota(ids.begin(), ids.end(), q0);
+    CK(cudaMemcpyAsync(d_sidx_.p + q0, ids.data(), sizeof(int32_t) * sn, cudaMemcpyHostToDevice, st_));
+    if (opt.profile) {          // the bulk launches' event pairs of earlier batches are complete
+        ev_used_ = 0; bulk_events_.clear();
+        CK(cudaEventRecord(ev_a_, st_));
+    }
+    for (size_t cnt; (cnt = emit_hits(q0, sn, H)) > H;) {
+        if (sn == 1) throw std::logic_error("score graph: one query row exceeds the hit buffer");
+        sn = std::max(1, std::min(sn / 2, (int)((double)sn * H / cnt)));
+    }
+    if (opt.profile) CK(cudaEventRecord(ev_b_, st_));
+    int jbits = 1, tbits = 1;
+    while (((int64_t)1 << jbits) < n) jbits++;
+    while ((1 << tbits) < sn) tbits++;
+    CK(cudaMemsetAsync(g.kept.p, 0, sizeof(unsigned int) * (sn + 1), st_));
+    shift_pass(d_hits_.p, d_counts_.p, (unsigned int)H, q0, jbits, g.key[0].p, g.val[0].p, g.kept.p, nullptr, nullptr);
+    std::vector<unsigned int> kept(sn + 1);
+    CK(cudaMemcpyAsync(kept.data(), g.kept.p, sizeof(unsigned int) * (sn + 1), cudaMemcpyDeviceToHost, st_));
+    CK(cudaStreamSynchronize(st_));
+    const unsigned int m = kept[0];
+    if (m > 1) {
+        cub::DoubleBuffer<unsigned long long> dk(g.key[0].p, g.key[1].p), dv(g.val[0].p, g.val[1].p);
+        size_t bytes = 0;
+        CK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, dk, dv, (int)m, 0, jbits + tbits, st_));
+        d_cub_.reserve(bytes);      // within the bound reserved above
+        CK(cub::DeviceRadixSort::SortPairs(d_cub_.p, bytes, dk, dv, (int)m, 0, jbits + tbits, st_));
+        launches_ += 4;
+        hmk_graph_edges<<<std::min<int64_t>(sm_count_ * 8, (m + 255) / 256), 256, 0, st_>>>(dk.Current(), dv.Current(), m, q0, jbits, g.edges.p);
+    } else if (m == 1) {
+        hmk_graph_edges<<<1, 32, 0, st_>>>(g.key[0].p, g.val[0].p, m, q0, jbits, g.edges.p);
+    }
+    CK(cudaGetLastError());
+    if (opt.profile) {
+        CK(cudaEventRecord(ev_c_, st_));
+        CK(cudaEventSynchronize(ev_c_));
+        float a = 0, b = 0;
+        CK(cudaEventElapsedTime(&a, ev_a_, ev_b_));
+        CK(cudaEventElapsedTime(&b, ev_b_, ev_c_));
+        section_ms[0] += a;
+        section_ms[1] += b;
+    }
+    g.row_off.assign(sn + 1, 0);
+    for (int t = 0; t < sn; t++) g.row_off[t + 1] = g.row_off[t] + kept[t + 1];
+    g.q0 = q0; g.q1 = q0 + sn;
+    g.sn = std::min(HMK_MAXBATCH, 2 * sn);      // rows only get shorter: the next batch may take more queries again
+    g.valid = true;
+}
+
+int Engine::score_graph(int64_t* cursor, hmk_graph_edge* out, int64_t cap, int64_t* n_out) {
+    CK(cudaSetDevice(device_));
+    if (!uploaded_) throw std::invalid_argument("hmk_score_graph before hmk_upload");
+    if (!cursor || !n_out || cap < 0 || (cap > 0 && !out)) throw std::invalid_argument("hmk_score_graph: bad argument");
+    *n_out = 0;
+    if (bad_residue_) return HMK_ERR_BAD_RESIDUE;
+    if (n_ >= 2 && X_ >= min_len_) return HMK_ERR_SHIFT_TOO_BIG;
+    int64_t i = cursor[0], r = cursor[1];
+    if (i < 0 || r < 0 || i > n_ || (i == n_ && r != 0) || (n_ < 2 && r != 0))
+        throw std::invalid_argument("hmk_score_graph: cursor outside the graph");
+    GraphBatch& g = graph_;
+    if (i == 0 && r == 0 && opt.profile) section_ms[0] = section_ms[1] = 0;
+    if (!(g.valid && i == g.next_i && r == g.next_r)) g.valid = false;   // only a continuing cursor reuses the kept batch
+    if (n_ < 2) i = n_;
+    int64_t got = 0;
+    for (bool first = true; i < n_; first = false) {
+        if (!g.valid || i < g.q0 || i >= g.q1) graph_batch((int)i);
+        const int64_t* ro = g.row_off.data();
+        const int64_t t = i - g.q0, end = ro[g.q1 - g.q0];
+        if (first && r > ro[t + 1] - ro[t]) throw std::invalid_argument("hmk_score_graph: cursor beyond the row's edges");
+        const int64_t p = ro[t] + r, take = std::min(cap - got, end - p);
+        if (take > 0) {
+            CK(cudaMemcpyAsync(out + got, g.edges.p + p, sizeof(hmk_graph_edge) * take, cudaMemcpyDeviceToHost, st_));
+            CK(cudaStreamSynchronize(st_));
+            got += take;
+        }
+        const int64_t e = p + take;
+        if (e == end) {          // batch done
+            i = g.q1; r = 0;
+            if (got == cap) break;
+            continue;
+        }
+        const int64_t row = std::upper_bound(ro, ro + (g.q1 - g.q0) + 1, e) - ro - 1;   // ro[row] <= e < ro[row + 1]
+        i = g.q0 + row; r = e - ro[row];
+        break;
+    }
+    cursor[0] = i; cursor[1] = r;
+    g.next_i = i; g.next_r = r;
+    *n_out = got;
+    return HMK_OK;
+}
+
+int Engine::score_pairs(const int32_t* seq1, const int32_t* seq2, int32_t np, int32_t* scores, int32_t* shifts) {
+    CK(cudaSetDevice(device_));
+    if (!uploaded_) throw std::invalid_argument("hmk_score_pairs before hmk_upload");
+    if (np < 0 || (np > 0 && (!seq1 || !seq2 || !scores || !shifts))) throw std::invalid_argument("hmk_score_pairs: bad argument");
+    std::vector<int4> pairs(np);
+    bool too_big = false;
+    for (int32_t e = 0; e < np; e++) {
+        if (seq1[e] < 0 || seq1[e] >= n_ || seq2[e] < 0 || seq2[e] >= n_) throw std::invalid_argument("hmk_score_pairs: id out of range");
+        const int l1 = h_off_[seq1[e] + 1] - h_off_[seq1[e]], l2 = h_off_[seq2[e] + 1] - h_off_[seq2[e]];
+        too_big |= X_ >= std::min(l1, l2);
+        pairs[e] = make_int4(seq2[e], seq1[e], 0, 0);
+    }
+    if (bad_residue_) return HMK_ERR_BAD_RESIDUE;
+    if (too_big) return HMK_ERR_SHIFT_TOO_BIG;
+    if (np == 0) return HMK_OK;
+    DevBuf<int4> d_pairs;
+    DevBuf<int32_t> d_out;
+    d_pairs.reserve(np); d_out.reserve(2 * (size_t)np);
+    CK(cudaMemcpyAsync(d_pairs.p, pairs.data(), sizeof(int4) * np, cudaMemcpyHostToDevice, st_));
+    shift_pass(d_pairs.p, nullptr, (unsigned int)np, 0, 0, nullptr, nullptr, nullptr, d_out.p, d_out.p + np);
+    CK(cudaMemcpyAsync(scores, d_out.p, sizeof(int32_t) * np, cudaMemcpyDeviceToHost, st_));
+    CK(cudaMemcpyAsync(shifts, d_out.p + np, sizeof(int32_t) * np, cudaMemcpyDeviceToHost, st_));
+    CK(cudaStreamSynchronize(st_));
     return HMK_OK;
 }
 
@@ -2298,6 +2480,7 @@ int hmk_set_option(hmk_ctx* ctx, const char* name, int64_t value) {
         {"min_iters", &o.min_iters, 1, 64},         {"bucket_aux", &o.bucket_aux, 0, 1},
         {"clinkage_dense_max", &o.clinkage_dense_max, 0, 32768},
         {"clinkage_threads", &o.clinkage_threads, 0, HMK_CL_THREADS},
+        {"graph_cap", &o.graph_cap, 0, (int64_t)1 << 30},
     };
     for (const Knob& k : knobs) {
         if (s != k.name) continue;
@@ -2315,6 +2498,26 @@ int hmk_score_block(hmk_ctx* ctx, const int32_t* first_ids, int32_t n_first, con
     return guarded(errbuf, errlen, [&] {
         ctx->engine.score_block(first_ids, n_first, second_ids, n_second, scores);
         return HMK_STATUS_OK;
+    });
+}
+
+int hmk_score_graph(hmk_ctx* ctx, int64_t cursor[2], hmk_graph_edge* out, int64_t cap, int64_t* n_out, char* errbuf,
+                    size_t errlen) {
+    if (!ctx) return HMK_STATUS_BAD_ARG;
+    return guarded(errbuf, errlen, [&] {
+        int rc = ctx->engine.score_graph(cursor, out, cap, n_out);
+        if (rc) set_err(errbuf, errlen, status_text(rc));
+        return rc;
+    });
+}
+
+int hmk_score_pairs(hmk_ctx* ctx, const int32_t* seq1_ids, const int32_t* seq2_ids, int32_t n_pairs, int32_t* scores,
+                    int32_t* shifts, char* errbuf, size_t errlen) {
+    if (!ctx) return HMK_STATUS_BAD_ARG;
+    return guarded(errbuf, errlen, [&] {
+        int rc = ctx->engine.score_pairs(seq1_ids, seq2_ids, n_pairs, scores, shifts);
+        if (rc) set_err(errbuf, errlen, status_text(rc));
+        return rc;
     });
 }
 

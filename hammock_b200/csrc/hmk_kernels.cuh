@@ -2923,3 +2923,72 @@ __global__ void hmk_cl_twins(const int64_t* __restrict__ row_off, const uint64_t
         }
     }
 }
+
+// ---- score graph (Engine::graph_batch) and hmk_score_pairs: ShiftedScorer.scoreWithShift, one thread per pair, with the
+// one-at-a-time scorer of the generic kernel.  pairs[i] = (seq2 = q0 + x, seq1 = y, score z).
+//   graph (keys != NULL): the EMIT hits of one query batch (count = the kernel's hit counter, at most cap stored).  A
+//     pair with seq1 <= seq2 is dropped; a kept one gets the sort key (x << jbits) | y, the value (score, shift) and a
+//     count in its query's row.  The recomputed score equals the emitted one.
+//   pairs (keys == NULL): the first cap pairs, none dropped; score[i] / shift[i] in input order.
+struct HmkShiftArgs {
+    const int4* pairs;
+    const unsigned int* count;
+    unsigned int cap;
+    int32_t q0, jbits;
+    const uint8_t* res;
+    const int32_t* off;
+    const int32_t* M;
+    int32_t X, P, n;
+    unsigned long long* keys;
+    unsigned long long* vals;
+    unsigned int* kept;     // [0] kept pairs, [1 + x] pairs kept in query row x
+    int32_t* score;
+    int32_t* shift;
+};
+
+__global__ void hmk_score_shift(HmkShiftArgs a) {
+    const unsigned int m = a.count ? min(*a.count, a.cap) : a.cap;
+    const int lane = threadIdx.x & 31;
+    const unsigned int stride = gridDim.x * blockDim.x;
+    // every lane of a warp takes the same number of turns: the kept pairs are counted with one atomic per warp
+    for (unsigned int base = blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < m; base += stride) {
+        const unsigned int i = base + lane;
+        bool keep = false;
+        int4 h = make_int4(0, 0, 0, 0);
+        int32_t s = 0;
+        int k = 0;
+        if (i < m) {
+            h = a.pairs[i];
+            const int32_t q = a.q0 + h.x;
+            HMK_CHECK(q >= 0 && q < a.n && h.y >= 0 && h.y < a.n);
+            if (!a.keys || h.y > q) {
+                s = hmk_score_with_shift(a.res + a.off[h.y], a.off[h.y + 1] - a.off[h.y], a.res + a.off[q], a.off[q + 1] - a.off[q],
+                                         a.M, a.X, a.P, &k);
+                if (!a.keys) { a.score[i] = s; a.shift[i] = k; }
+                else { HMK_CHECK(s == h.z); keep = true; }
+            }
+        }
+        if (!a.keys) continue;
+        const unsigned int km = __ballot_sync(0xffffffffu, keep);
+        if (!km) continue;
+        unsigned int pos = 0;
+        const int leader = __ffs(km) - 1;
+        if (lane == leader) pos = atomicAdd(a.kept, (unsigned int)__popc(km));
+        pos = __shfl_sync(0xffffffffu, pos, leader) + __popc(km & ((1u << lane) - 1u));
+        if (keep) {
+            HMK_CHECK(pos < a.cap);
+            a.keys[pos] = ((unsigned long long)(uint32_t)h.x << a.jbits) | (uint32_t)h.y;
+            a.vals[pos] = ((unsigned long long)(uint32_t)s << 32) | (uint32_t)k;
+            atomicAdd(a.kept + 1 + h.x, 1u);
+        }
+    }
+}
+
+// the sorted (key, value) pairs of a graph batch as edges (seq, partner, score, shift) == hmk_graph_edge
+__global__ void hmk_graph_edges(const unsigned long long* __restrict__ keys, const unsigned long long* __restrict__ vals,
+                                unsigned int m, int32_t q0, int32_t jbits, int4* __restrict__ edges) {
+    for (unsigned int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
+        const unsigned long long k = keys[i], v = vals[i];
+        edges[i] = make_int4(q0 + (int32_t)(k >> jbits), (int32_t)(k & ((1ull << jbits) - 1)), (int32_t)(v >> 32), (int32_t)(uint32_t)v);
+    }
+}

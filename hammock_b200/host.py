@@ -516,6 +516,10 @@ def _raise_status(rc: int, err: bytes, step: int = -1):
     raise CudaError(msg or f"status {rc}")
 
 
+# one score-graph edge, laid out as hmk_graph_edge
+EDGE_DTYPE = np.dtype([("seq", "<i4"), ("partner", "<i4"), ("score", "<i4"), ("shift", "<i4")])
+
+
 class GreedyResult:
     def __init__(self, cluster_id, member_rank, result_order, n_multi, stats):
         self.cluster_id, self.member_rank, self.result_order = cluster_id, member_rank, result_order
@@ -670,6 +674,42 @@ class GreedyContext:
         if rc:
             _raise_status(rc, err.value)
         return out
+
+    def graph_page(self, cursor, cap: int):
+        """hmk_score_graph: at most `cap` edges of the score graph from `cursor` = (row, edges of the row already taken)
+        -> (EDGE_DTYPE array, next cursor); the cursor (n, 0) means done."""
+        cur = (C.c_int64 * 2)(int(cursor[0]), int(cursor[1]))
+        out = np.empty(max(int(cap), 1), dtype=EDGE_DTYPE)
+        got = C.c_int64(0)
+        err = C.create_string_buffer(512)
+        rc = self._L.hmk_score_graph(self._h, cur, out.ctypes.data_as(C.c_void_p), int(cap), C.byref(got), err, 512)
+        if rc:
+            _raise_status(rc, err.value)
+        return out[:got.value], (int(cur[0]), int(cur[1]))
+
+    def score_graph(self, chunk: int = 1 << 22):
+        """Yields the score graph of the uploaded sequences as EDGE_DTYPE arrays of at most `chunk` edges, in graph order
+        (seq, then partner): every pair seq < partner with ShiftedScorer.scoreWithShift(partner, seq) >= threshold."""
+        cursor = (0, 0)
+        while cursor != (self.n, 0):
+            edges, cursor = self.graph_page(cursor, chunk)
+            if len(edges):
+                yield edges
+
+    def score_pairs(self, seq1_ids, seq2_ids):
+        """hmk_score_pairs: ShiftedScorer.scoreWithShift(seq1 = seq1_ids[e], seq2 = seq2_ids[e]) -> (scores, shifts)."""
+        a = np.ascontiguousarray(seq1_ids, dtype=np.int32)
+        b = np.ascontiguousarray(seq2_ids, dtype=np.int32)
+        if a.shape != b.shape:
+            raise ValueError("seq1_ids and seq2_ids differ in length")
+        scores = np.empty(max(len(a), 1), dtype=np.int32)
+        shifts = np.empty(max(len(a), 1), dtype=np.int32)
+        err = C.create_string_buffer(512)
+        rc = self._L.hmk_score_pairs(self._h, _ptr(a, C.c_int32), _ptr(b, C.c_int32), len(a), _ptr(scores, C.c_int32),
+                                     _ptr(shifts, C.c_int32), err, 512)
+        if rc:
+            _raise_status(rc, err.value)
+        return scores[:len(a)], shifts[:len(a)]
 
     _KERNELS = {-1: "none", 0: "generic", 1: "fast", 2: "filter", 3: "long"}
 
@@ -837,6 +877,17 @@ class ShiftedScorer:
         """ShiftedScorer.sequenceScore (ShiftedScorer.java:97-100)."""
         return int(self.score_block([seq1], [seq2])[0, 0])
 
+    def score_with_shift(self, seq1: UniqueSequence, seq2: UniqueSequence):
+        """AligningSequenceScorer.scoreWithShift (ShiftedScorer.java:48-95) -> (score, shift), the AligningScorerResult."""
+        res, offs, ab = pack_sequences([seq1, seq2])
+        ctx = GreedyContext(self.device)
+        try:
+            ctx.upload(res, offs, ab, self.scoring_matrix, 0, self.max_shift, self.shift_penalty, 0)
+            scores, shifts = ctx.score_pairs([0], [1])
+            return int(scores[0]), int(shifts[0])
+        finally:
+            ctx.close()
+
     def score_block(self, firsts: Sequence[UniqueSequence], seconds: Sequence[UniqueSequence]) -> np.ndarray:
         seqs = list(firsts) + list(seconds)
         if min(len(s.sequence) for s in seqs) <= self.max_shift:        # ShiftedScorer.java:59-62
@@ -910,6 +961,39 @@ def run_clinkage_clustering(sequences: List[UniqueSequence], scoring_matrix, thr
     if threshold is None:
         threshold = set_clinkage_threshold(sequences)
     return ClinkageSequenceClusterer(ShiftedScorer(scoring_matrix, shift_penalty, max_shift, device), threshold).cluster(list(sequences))
+
+
+def score_graph(sequences: Sequence[UniqueSequence], scoring_matrix, threshold: Optional[int] = None,
+                max_shift: Optional[int] = None, shift_penalty: int = 0, device: int = 0) -> np.ndarray:
+    """The score graph both initial clusterings are built from: every pair i < j of `sequences` (input order, as
+    run_clinkage_clustering) with ShiftedScorer.scoreWithShift(seq j, seq i) >= threshold, as an EDGE_DTYPE array
+    ordered by i, then j.  Defaults: setClinkageThreshold and getMaxShift.  GreedyContext.score_graph streams it."""
+    if len(sequences) == 0:
+        return np.zeros(0, dtype=EDGE_DTYPE)
+    max_shift = get_max_shift(sequences) if max_shift is None else check_max_shift(sequences, max_shift)
+    if threshold is None:
+        threshold = set_clinkage_threshold(sequences)
+    res, offs, ab = pack_sequences(sequences)
+    ctx = GreedyContext(device)
+    try:
+        ctx.upload(res, offs, ab, scoring_matrix, threshold, max_shift, shift_penalty, 0)
+        parts = list(ctx.score_graph())
+    finally:
+        ctx.close()
+    return np.concatenate(parts) if parts else np.zeros(0, dtype=EDGE_DTYPE)
+
+
+def save_score_graph(sequences: Sequence[UniqueSequence], edges, path: str) -> None:
+    """score_graph.tsv: header `sequence, partner, score, shift`, one row per edge in the order given, sequences as
+    strings.  `edges`: one EDGE_DTYPE array or an iterable of them (GreedyContext.score_graph)."""
+    strs = [s.get_sequence_string() for s in sequences]
+    chunks = [edges] if isinstance(edges, np.ndarray) else edges
+    with open(path, "w", newline="") as w:
+        w.write("sequence\tpartner\tscore\tshift\n")
+        for e in chunks:
+            w.write("".join(f"{strs[i]}\t{strs[j]}\t{s}\t{k}\n"
+                            for i, j, s, k in zip(e["seq"].tolist(), e["partner"].tolist(), e["score"].tolist(),
+                                                  e["shift"].tolist())))
 
 
 def rebuild_clusters(sequences: Sequence[UniqueSequence], r: GreedyResult) -> List[Cluster]:

@@ -4,6 +4,8 @@
 // (`java -jar Hammock.jar cluster -i <outdir>/initial_clusters_sequences.tsv`) can take over.
 // `hammock_greedy clinkage ...` is the `clinkage` mode (Hammock.java:236-252, 449-489): the exact complete-linkage
 // clusterer on the sequences in INPUT order (no sorting, no cluster limit), same result files.
+// `hammock_greedy graph ...` writes the score graph both clusterings are built from: every pair of sequences (input order,
+// clinkage's automatic threshold and max shift) scoring >= threshold with its score and shift, to score_graph.tsv.
 // Flags keep the reference's names (Hammock.java:824-970).  Multiple alignments are NOT built here
 // (that is the Clustal-Omega stage, outside this path): the alignment column is "NA" for multi-member
 // clusters, which `cluster` mode accepts.
@@ -15,7 +17,7 @@
 using namespace hammock;
 
 static void usage() {
-    std::cerr << "usage: hammock_greedy [greedy|clinkage] -i <input.fa> -d <outdir> [-f fasta|tab] [-m <matrix.txt>] [-g <threshold>] [-x <max_shift>]\n"
+    std::cerr << "usage: hammock_greedy [greedy|clinkage|graph] -i <input.fa> -d <outdir> [-f fasta|tab] [-m <matrix.txt>] [-g <threshold>] [-x <max_shift>]\n"
                  "                      [-p <gap_penalty>] [--initial_clusters_limit <n>] [-R size|alphabetic|random|input|<label>]\n"
                  "                      [-S <seed>] [-l label1,label2,...] [--device <n>] [--dump-prepared]\n";
 }
@@ -23,7 +25,7 @@ static void usage() {
 int main(int argc, char** argv) {
     std::string input, outdir, format = "fasta", matrixPath, order = "size";
     bool haveT = false, haveX = false, haveK = false, dump = false, haveLabels = false, timeHost = false, hostOnly = false;
-    bool clinkage = false;
+    bool clinkage = false, graph = false;   // graph: input order and clinkage's automatic parameters, like clinkage
     int32_t threshold = 0, maxShift = 0, shiftPenalty = 0, limit = 0;   // shiftPenalty default 0 (Hammock.java:82)
     int64_t seed = 42;                                                   // Hammock.java:67
     int device = 0;
@@ -37,6 +39,7 @@ int main(int argc, char** argv) {
             };
             if (a == "greedy") continue;
             else if (a == "clinkage" && i == 1) clinkage = true;
+            else if (a == "graph" && i == 1) clinkage = graph = true;
             else if (a == "-i" || a == "--input") input = next();
             else if (a == "-d" || a == "--outputDirectory") outdir = next();
             else if (a == "-f" || a == "--file_format") format = next();
@@ -106,6 +109,23 @@ int main(int argc, char** argv) {
         }
 
         const std::vector<int32_t> matrix = loadScoringMatrix(matrixPath);
+        if (graph) {
+            if (outdir.empty()) throw CLIException("Error. Parameter output directory (-d) missing: graph mode writes score_graph.tsv.");
+            std::string d = outdir;
+            if (d.back() != '/') d.push_back('/');
+            std::cerr << "Score graph... (" << sequences.size() << " unique sequences, threshold " << threshold << ", max shift " << maxShift << ")\n";
+            auto t0 = std::chrono::steady_clock::now();
+            int64_t edges = 0;
+            {
+                TsvWriter w(d + "score_graph.tsv");
+                writeScoreGraphHeader(w);
+                edges = GpuScoreGraph{matrix, shiftPenalty, maxShift, threshold, device}.pull(
+                    sequences, [&](const hmk_graph_edge* e, size_t count) { writeScoreGraphEdges(w, sequences, e, count); });
+            }
+            auto ms = std::chrono::duration_cast<std::chrono::milliseconds>(std::chrono::steady_clock::now() - t0).count();
+            std::cerr << "Ready. Time: " << ms << "\nEdges: " << edges << "\nScore graph in: " << d << "score_graph.tsv\n";
+            return 0;
+        }
         std::cerr << (clinkage ? "Clinkage" : "Greedy") << " clustering... (" << sequences.size() << " unique sequences, threshold " << threshold
                   << ", max shift " << maxShift;
         if (!clinkage) std::cerr << ", clusters limit " << limit;

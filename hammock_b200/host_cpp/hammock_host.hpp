@@ -546,6 +546,41 @@ struct GpuClinkageSequenceClusterer {
     }
 };
 
+// The score graph of `seqs` in the caller's order (hmk_score_graph on a context of its own): every pair i < j with
+// scoreWithShift(seq j, seq i) >= threshold, handed to fn(edges, count) one page of at most `page` edges at a time, in
+// graph order.  Returns the number of edges.
+struct GpuScoreGraph {
+    std::vector<int32_t> matrix;
+    int32_t shiftPenalty, maxShift, threshold;
+    int device = 0;
+
+    template <class Fn>
+    int64_t pull(const std::vector<UniqueSequence>& seqs, Fn&& fn, int64_t page = 1 << 20) const {
+        const int32_t n = (int32_t)seqs.size();
+        const PackedSequences packed(seqs);
+        hmk_greedy_in in{n, packed.res.data(), packed.off.data(), packed.ab.data(), matrix.data(), threshold, maxShift, shiftPenalty, 0};
+        char err[512] = {0};
+        auto check = [&](int rc) {
+            if (rc == HMK_STATUS_SHIFT_TOO_BIG) throw DataException(err);
+            if (rc == HMK_STATUS_BAD_RESIDUE) throw FileFormatException(err);
+            if (rc != HMK_STATUS_OK) throw CudaException(std::string("hammock_b200: ") + err);
+        };
+        hmk_ctx* ctx = nullptr;
+        check(hmk_create(&ctx, device, err, sizeof err));
+        struct Destroy { hmk_ctx* c; ~Destroy() { hmk_destroy(c); } } destroy{ctx};
+        check(hmk_upload(ctx, &in, err, sizeof err));
+        std::vector<hmk_graph_edge> buf((size_t)page);
+        int64_t cursor[2] = {0, 0}, total = 0;
+        while (cursor[0] != n || cursor[1] != 0) {
+            int64_t got = 0;
+            check(hmk_score_graph(ctx, cursor, buf.data(), page, &got, err, sizeof err));
+            fn(buf.data(), (size_t)got);
+            total += got;
+        }
+        return total;
+    }
+};
+
 // ---------------------------------------------------------------- result files (FileIOManager.java)
 static const char SEP = '\t';   // Hammock.CSV_SEPARATOR (Hammock.java:35)
 
@@ -670,6 +705,14 @@ inline void SaveClustersToCsv(const std::vector<Cluster>& clusters, const std::v
         }
         w << '\n';
     }
+}
+
+// score_graph.tsv (graph mode): the header, then one row per edge as sequence strings -- the same bytes as the Python
+// host's save_score_graph
+inline void writeScoreGraphHeader(TsvWriter& w) { w << "sequence" << SEP << "partner" << SEP << "score" << SEP << "shift" << '\n'; }
+inline void writeScoreGraphEdges(TsvWriter& w, const std::vector<UniqueSequence>& seqs, const hmk_graph_edge* e, size_t count) {
+    for (size_t k = 0; k < count; k++)
+        w << seqs[e[k].seq].sequence << SEP << seqs[e[k].partner].sequence << SEP << e[k].score << SEP << e[k].shift << '\n';
 }
 
 // saveInputStatistics (FileIOManager.java:709-729); no newline after the last line

@@ -160,7 +160,9 @@ int hmk_measure_peaks(hmk_ctx* ctx, double* out4, char* errbuf, size_t errlen);
  * p2_base, p2_iterate, p2_commit, final
  * After hmk_clinkage_run the first three slots hold the stages of the complete-linkage call instead: [0] scoring (dense:
  * the n x n matrix; sparse: the counting pass), [1] sparse row build (the filling pass, row sort and twin index; 0 on the
- * dense path), [2] nearest-neighbour chain; the others are 0. */
+ * dense path), [2] nearest-neighbour chain; the others are 0.
+ * hmk_score_graph adds to slots [0] (scoring passes) and [1] (shift, sort and edge passes) the device time of the batches
+ * it computes; a call at cursor {0, 0} sets both to 0 first. */
 #define HMK_NSECTIONS 13
 int hmk_get_section_ms(hmk_ctx* ctx, double* out, int n);
 /* tuning knobs; unknown names and out-of-range values return HMK_STATUS_BAD_ARG.  None of them changes the result.
@@ -185,6 +187,8 @@ int hmk_get_section_ms(hmk_ctx* ctx, double* out, int n);
  *              larger inputs take the sparse path
  *   clinkage_threads  complete linkage, sparse path: threads of the chain kernel (0 = automatic from the mean row length,
  *              else a multiple of 32 up to 1024)
+ *   graph_cap  hmk_score_graph: pairs scoring >= threshold one batch of query rows may hold on the device (0 = automatic,
+ *              4 194 304; never fewer than n); a batch with more is split
  *   profile    1 = time every bulk launch with CUDA events (hmk_stats.bulk_kernel_ms) */
 int hmk_set_option(hmk_ctx* ctx, const char* name, int64_t value);
 
@@ -193,6 +197,31 @@ int hmk_set_option(hmk_ctx* ctx, const char* name, int64_t value);
  * seq2 = second_ids[b]) for the uploaded sequences.  Used by the parity tests of the kernel. */
 int hmk_score_block(hmk_ctx* ctx, const int32_t* first_ids, int32_t n_first, const int32_t* second_ids,
                     int32_t n_second, int32_t* scores, char* errbuf, size_t errlen);
+
+/* One edge of the score graph: scoreWithShift(seq1 = partner, seq2 = seq) = (score, shift), seq < partner. */
+typedef struct {
+    int32_t seq, partner, score, shift;
+} hmk_graph_edge;
+
+/* The score graph of the uploaded sequences: every pair seq < partner (ids in upload order) whose
+ * AligningSequenceScorer.scoreWithShift(seq1 = partner, seq2 = seq) (ShiftedScorer.java:48-95) reaches the threshold,
+ * with that score and shift (the lowest winning diagonal, negated when seq1 is the shorter sequence), ordered by seq,
+ * then partner.  For a symmetric matrix these are the pairs complete linkage keeps; an asymmetric matrix is accepted.
+ * Paged pull: cursor = {i, r} continues at row i (the edges with seq == i) after its first r edges; {0, 0} starts.  The call
+ * writes min(cap, remaining) edges to out, *n_out = their number, and advances the cursor; {n, 0} means done.  Every valid
+ * cursor gives the same suffix, so a host may restart from a saved one.  A cursor that continues the previous call reuses
+ * the batch of rows kept on the device; any other cursor scores the rows from its row on again.  Device memory stays
+ * bounded by one batch (option graph_cap).  Status: HMK_STATUS_SHIFT_TOO_BIG when n >= 2 and max_shift >= the shortest
+ * length, HMK_STATUS_BAD_RESIDUE, HMK_STATUS_BAD_ARG for a call before hmk_upload, a negative cap, a negative cursor,
+ * i > n, or r beyond row i's length.  n of 0 or 1: an empty graph. */
+int hmk_score_graph(hmk_ctx* ctx, int64_t cursor[2], hmk_graph_edge* out, int64_t cap, int64_t* n_out, char* errbuf,
+                    size_t errlen);
+/* AligningSequenceScorer.scoreWithShift for arbitrary pairs of the uploaded sequences, on the GPU:
+ * (scores[e], shifts[e]) = scoreWithShift(seq1 = seq1_ids[e], seq2 = seq2_ids[e]).  Status: HMK_STATUS_SHIFT_TOO_BIG when
+ * max_shift >= the shorter length of some pair, HMK_STATUS_BAD_RESIDUE, HMK_STATUS_BAD_ARG for ids out of range or a
+ * call before hmk_upload. */
+int hmk_score_pairs(hmk_ctx* ctx, const int32_t* seq1_ids, const int32_t* seq2_ids, int32_t n_pairs, int32_t* scores,
+                    int32_t* shifts, char* errbuf, size_t errlen);
 
 /* One bulk scoring launch over the uploaded sequences with the context's scheme and options.  Used by the kernel tests.
  * Profile side: query_ids[0 .. n_query), as seq2.  Thread side (seq1): db_ids[0 .. n_db), or with db_ids NULL the ids
