@@ -12,6 +12,6 @@ from .host import (ALPHABET, Cluster, CudaError, DataException, FileFormatExcept
                    get_sorted_labels, java_hashmap_order, save_cluster_sequences_to_csv,
                    save_cluster_sequences_to_csv_ordered, save_clusters_to_csv, save_input_statistics, result_digest, ClinkageSequenceClusterer, UnsupportedInput,
                    clinkage_cluster_arrays, run_clinkage_clustering, set_clinkage_threshold, EDGE_DTYPE, score_graph,
-                   save_score_graph)
+                   save_score_graph, nearest_partners, save_nearest_partners)
 
 __all__ = [n for n in dir() if not n.startswith("_")]

@@ -53,7 +53,7 @@ class BatchProbeOut(C.Structure):
 
 EXPORTS = ["hmk_abi_version", "hmk_greedy_cluster", "hmk_greedy_cluster_multi", "hmk_clinkage_cluster", "hmk_clinkage_run", "hmk_create", "hmk_destroy", "hmk_upload", "hmk_run",
            "hmk_download", "hmk_get_stats", "hmk_get_section_ms", "hmk_set_option", "hmk_score_block", "hmk_bulk_probe",
-           "hmk_batch_probe", "hmk_score_graph", "hmk_score_pairs",
+           "hmk_batch_probe", "hmk_score_graph", "hmk_score_pairs", "hmk_nearest",
            "hmk_timer_begin", "hmk_timer_end", "hmk_measure_peaks", "hmk_nccl_unique_id", "hmk_init_distributed", "hmk_release_cached"]
 SECTIONS = ["p1_select", "p1_partner", "p1_cluster", "p1_intra", "p1_resolve", "p2_setup", "p2_filter", "p2_check",
             "p2_sort", "p2_base", "p2_iterate", "p2_commit", "final"]
@@ -122,5 +122,7 @@ def load():
     L.hmk_score_graph.argtypes = [vp, C.POINTER(C.c_int64), vp, C.c_int64, C.POINTER(C.c_int64), cp, sz]
     L.hmk_score_pairs.restype = C.c_int
     L.hmk_score_pairs.argtypes = [vp, i32p, i32p, C.c_int32, i32p, i32p, cp, sz]
+    L.hmk_nearest.restype = C.c_int
+    L.hmk_nearest.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, i32p, i32p, i32p, i32p, i32p, cp, sz]
     _lib = L
     return L

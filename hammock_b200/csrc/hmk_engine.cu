@@ -257,6 +257,8 @@ public:
     int clinkage(const hmk_greedy_in* in, hmk_greedy_out* out);
     int score_graph(int64_t* cursor, hmk_graph_edge* out, int64_t cap, int64_t* n_out);
     int score_pairs(const int32_t* seq1, const int32_t* seq2, int32_t np, int32_t* scores, int32_t* shifts);
+    int nearest(int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partner, int32_t* score, int32_t* shift,
+                int32_t* count, int32_t* more);
     std::string status_msg;      // details of the last non-zero status, when there are any
     hmk_stats stats{};
     int error_step = -1;
@@ -389,6 +391,10 @@ private:
     void graph_batch(int q0);
     void shift_pass(const int4* pairs, const unsigned int* count, unsigned int cap, int q0, int jbits,
                     unsigned long long* keys, unsigned long long* vals, unsigned int* kept, int32_t* score, int32_t* shift);
+    // nearest partners (hmk_nearest): the query batch's ids, profiles, top-k lists and gmin bounds, and its output rows --
+    // the nearest search's own, so that nothing of it reaches a clustering run's batch buffers
+    BatchBuf near_bb_;
+    DevBuf<int32_t> d_near_out_;
     bool lsort_ = false;
     // phase-1 partner-search hits kept for phase 2 (opt.reuse): buffer, 64-bit counters [0] appended, [1] valid
     DevBuf<int4> d_xhits_;
@@ -2253,6 +2259,93 @@ int Engine::score_pairs(const int32_t* seq1, const int32_t* seq2, int32_t np, in
     return HMK_OK;
 }
 
+// ---------------------------------------------------------------- nearest partners (hmk_nearest)
+// Row i's list: the k best ids j != i with scoreWithShift(seq1 = j, seq2 = i) >= T under the partner search's key
+// (score desc, then tie-break rank: abundance desc, id asc).  Per batch of rows: the partner search's TOPK launch with
+// kb = k + 1 over every thread-side id [0, n) (no q_minid: the row's own id competes too), the stripe merge, and
+// hmk_nearest_rows, which drops the row's own id, cuts the list to k and adds each entry's score and shift.  The top
+// k + 1 keys of all ids contain the top k of the others, so the lists are exact, and so is `more` (see the kernel).
+int Engine::nearest(int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partner, int32_t* score, int32_t* shift,
+                    int32_t* count, int32_t* more) {
+    CK(cudaSetDevice(device_));
+    if (!uploaded_) throw std::invalid_argument("hmk_nearest before hmk_upload");
+    if (k < 1 || k > HMK_NEAREST_MAX_K) throw std::invalid_argument("hmk_nearest: k outside 1 .. 31");
+    if (row_begin < 0 || n_rows < 0 || (int64_t)row_begin + n_rows > n_)
+        throw std::invalid_argument("hmk_nearest: row range outside [0, n]");
+    if (n_rows > 0 && (!partner || !score || !shift || !count || !more)) throw std::invalid_argument("hmk_nearest: null output");
+    if (bad_residue_) return HMK_ERR_BAD_RESIDUE;
+    if (n_ >= 2 && X_ >= min_len_) return HMK_ERR_SHIFT_TOO_BIG;
+    if (opt.profile) section_ms[0] = section_ms[1] = 0;
+    if (n_ < 2) {        // no partner exists
+        for (int64_t e = 0; e < (int64_t)n_rows * k; e++) { partner[e] = -1; score[e] = 0; shift[e] = 0; }
+        for (int32_t t = 0; t < n_rows; t++) { count[t] = 0; more[t] = 0; }
+        return HMK_OK;
+    }
+    // the bulk launch path (qt_max, launch_bulk, launch_planned) reads the list length from opt.kb
+    struct KbScope { Options& o; int64_t saved; ~KbScope() { o.kb = saved; } } kb_scope{opt, opt.kb};
+    opt.kb = k + 1;
+    const int kb = k + 1;
+    BatchBuf& bb = near_bb_;
+    bb.qid.reserve(HMK_MAXBATCH); bb.gmin.reserve(HMK_MAXBATCH);
+    bb.bk_key.reserve((size_t)HMK_MAXBATCH * kb); bb.bk_cnt.reserve(HMK_MAXBATCH); bb.bk_ovf.reserve(HMK_MAXBATCH);
+    if (fast_) bb.prof.reserve((size_t)HMK_MAXBATCH * sc_.prof_words);
+    d_near_out_.reserve((size_t)HMK_MAXBATCH * (3 * k + 2));
+    int32_t* const o_partner = d_near_out_.p;
+    int32_t* const o_score = o_partner + (size_t)HMK_MAXBATCH * k;
+    int32_t* const o_shift = o_score + (size_t)HMK_MAXBATCH * k;
+    int32_t* const o_count = o_shift + (size_t)HMK_MAXBATCH * k;
+    int32_t* const o_more = o_count + HMK_MAXBATCH;
+    std::vector<int32_t> ids(HMK_MAXBATCH);
+    for (int32_t r0 = row_begin; r0 < row_begin + n_rows; r0 += HMK_MAXBATCH) {
+        const int sn = std::min<int32_t>(HMK_MAXBATCH, row_begin + n_rows - r0);
+        std::iota(ids.begin(), ids.begin() + sn, r0);
+        CK(cudaMemcpyAsync(bb.qid.p, ids.data(), sizeof(int32_t) * sn, cudaMemcpyHostToDevice, st_));
+        if (opt.profile) {          // the bulk launches' event pairs of earlier batches are complete
+            ev_used_ = 0; bulk_events_.clear();
+            CK(cudaEventRecord(ev_a_, st_));
+        }
+        CK(cudaMemsetAsync(bb.gmin.p, 0, sizeof(unsigned long long) * sn, st_));
+        if (fast_) launch_profiles(HMK_PROF_QUERY, bb.qid.p, sn, bb.prof.p, sc_, st_);
+        HmkBulkArgs a{};
+        a.prof = bb.prof.p; a.nq = sn;
+        a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = 0; a.ndb = n_;
+        a.tierank = identity_rank_ ? nullptr : d_tierank_.p;
+        a.tk_gmin = bb.gmin.p;
+        const HmkBulkArgs p = launch_bulk(HMK_MODE_TOPK, a, bb.qid.p, 1, st_, &bb);
+        stats.bulk_pairs += (int64_t)sn * n_;
+        if (opt.profile) CK(cudaEventRecord(ev_b_, st_));
+        hmk_topk_merge<<<(sn * 32 + 255) / 256, 256, 0, st_>>>(sn, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
+                                                               bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p,
+                                                               p.sched ? p.sched + p.nqt : nullptr, p.qt);
+        CK(cudaGetLastError());
+        HmkNearestArgs na{};
+        na.nq = sn; na.k = k; na.r0 = r0; na.n = n_;
+        na.key = bb.bk_key.p; na.cnt = bb.bk_cnt.p; na.ovf = bb.bk_ovf.p;
+        na.id_of_rank = identity_rank_ ? nullptr : d_id_of_rank_.p;
+        na.res = d_res_.p; na.off = d_off_.p; na.M = d_M_.p; na.X = X_; na.P = P_;
+        na.partner = o_partner; na.score = o_score; na.shift = o_shift; na.count = o_count; na.more = o_more;
+        hmk_nearest_rows<<<(sn * 32 + 255) / 256, 256, 0, st_>>>(na);
+        CK(cudaGetLastError());
+        launches_ += 2;
+        if (opt.profile) CK(cudaEventRecord(ev_c_, st_));
+        const size_t e0 = (size_t)(r0 - row_begin) * k, t0 = (size_t)(r0 - row_begin), ne = (size_t)sn * k;
+        CK(cudaMemcpyAsync(partner + e0, o_partner, sizeof(int32_t) * ne, cudaMemcpyDeviceToHost, st_));
+        CK(cudaMemcpyAsync(score + e0, o_score, sizeof(int32_t) * ne, cudaMemcpyDeviceToHost, st_));
+        CK(cudaMemcpyAsync(shift + e0, o_shift, sizeof(int32_t) * ne, cudaMemcpyDeviceToHost, st_));
+        CK(cudaMemcpyAsync(count + t0, o_count, sizeof(int32_t) * sn, cudaMemcpyDeviceToHost, st_));
+        CK(cudaMemcpyAsync(more + t0, o_more, sizeof(int32_t) * sn, cudaMemcpyDeviceToHost, st_));
+        CK(cudaStreamSynchronize(st_));
+        if (opt.profile) {
+            float ta = 0, tb = 0;
+            CK(cudaEventElapsedTime(&ta, ev_a_, ev_b_));
+            CK(cudaEventElapsedTime(&tb, ev_b_, ev_c_));
+            section_ms[0] += ta;
+            section_ms[1] += tb;
+        }
+    }
+    return HMK_OK;
+}
+
 void Engine::init_distributed(int rank, int world, const void* id128) {
     CK(cudaSetDevice(device_));
     if (world < 1 || rank < 0 || rank >= world || !id128) throw std::invalid_argument("hmk_init_distributed: bad rank/world/id");
@@ -2516,6 +2609,16 @@ int hmk_score_pairs(hmk_ctx* ctx, const int32_t* seq1_ids, const int32_t* seq2_i
     if (!ctx) return HMK_STATUS_BAD_ARG;
     return guarded(errbuf, errlen, [&] {
         int rc = ctx->engine.score_pairs(seq1_ids, seq2_ids, n_pairs, scores, shifts);
+        if (rc) set_err(errbuf, errlen, status_text(rc));
+        return rc;
+    });
+}
+
+int hmk_nearest(hmk_ctx* ctx, int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partner, int32_t* score,
+                int32_t* shift, int32_t* count, int32_t* more, char* errbuf, size_t errlen) {
+    if (!ctx) return HMK_STATUS_BAD_ARG;
+    return guarded(errbuf, errlen, [&] {
+        int rc = ctx->engine.nearest(k, row_begin, n_rows, partner, score, shift, count, more);
         if (rc) set_err(errbuf, errlen, status_text(rc));
         return rc;
     });

@@ -2992,3 +2992,62 @@ __global__ void hmk_graph_edges(const unsigned long long* __restrict__ keys, con
         edges[i] = make_int4(q0 + (int32_t)(k >> jbits), (int32_t)(k & ((1ull << jbits) - 1)), (int32_t)(v >> 32), (int32_t)(uint32_t)v);
     }
 }
+
+// ---- nearest partners (Engine::nearest): one warp per row t of a query batch (row id r0 + t) over its merged list of
+// the k + 1 best keys among the thread-side ids [0, n).  The row's own id is dropped and the list cut to k: lane o fills
+// output slot o with the partner id, scoreWithShift(seq1 = partner, seq2 = row) and its shift, or partner -1, score 0,
+// shift 0 past the row's count.  The recomputed score equals the key's.  more[t] = 1 when more than k other ids qualify:
+// with the row's own id in the list that is the merged overflow flag (more than k + 1 keys), without it a full list of
+// k + 1 keys (the row's own key, if it qualifies, ranks behind all of them).
+struct HmkNearestArgs {
+    int32_t nq, k, r0, n;
+    const uint64_t* key;        // [nq][k + 1] merged lists (hmk_topk_merge)
+    const int32_t* cnt;
+    const int32_t* ovf;
+    const int32_t* id_of_rank;  // NULL: rank == id
+    const uint8_t* res;
+    const int32_t* off;
+    const int32_t* M;
+    int32_t X, P;
+    int32_t* partner;           // [nq][k]
+    int32_t* score;
+    int32_t* shift;
+    int32_t* count;             // [nq]
+    int32_t* more;
+};
+
+__global__ void hmk_nearest_rows(HmkNearestArgs a) {
+    const int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+    if (t >= a.nq) return;      // warp-uniform
+    const int kb = a.k + 1, row = a.r0 + t;
+    const int c = a.cnt[t];
+    HMK_CHECK(kb <= 32 && c >= 0 && c <= kb && row < a.n);
+    const uint64_t* key = a.key + (size_t)t * kb;
+    int32_t id = -1;
+    if (lane < c) {
+        const uint32_t r = hmk_key_rank(key[lane]);
+        id = a.id_of_rank ? a.id_of_rank[r] : (int32_t)r;
+    }
+    const unsigned self = __ballot_sync(0xffffffffu, lane < c && id == row);
+    const int s = self ? __ffs(self) - 1 : kb;                  // list position of the row's own id
+    const int src = lane < s ? lane : lane + 1;                 // the list entry output slot `lane` takes
+    const int m = min(c - (self ? 1 : 0), a.k);
+    const int32_t p = __shfl_sync(0xffffffffu, id, src & 31);
+    if (lane < a.k) {
+        int32_t sc = 0, sh = 0;
+        if (lane < m) {
+            HMK_CHECK(p >= 0 && p < a.n && p != row);
+            sc = hmk_score_with_shift(a.res + a.off[p], a.off[p + 1] - a.off[p], a.res + a.off[row], a.off[row + 1] - a.off[row],
+                                      a.M, a.X, a.P, &sh);
+            HMK_CHECK(sc == hmk_key_score(key[src]));
+        }
+        const size_t o = (size_t)t * a.k + lane;
+        a.partner[o] = lane < m ? p : -1;
+        a.score[o] = sc;
+        a.shift[o] = sh;
+    }
+    if (lane == 0) {
+        a.count[t] = m;
+        a.more[t] = self ? (a.ovf[t] ? 1 : 0) : (c == kb ? 1 : 0);
+    }
+}

@@ -711,6 +711,23 @@ class GreedyContext:
             _raise_status(rc, err.value)
         return scores[:len(a)], shifts[:len(a)]
 
+    def nearest(self, k: int, rows=None):
+        """hmk_nearest: the k best-scoring partners of every row in `rows` = (begin, end) (default: all uploaded
+        sequences) -> (partner, score, shift) [rows, k] and (count, more) [rows], all int32.  Row i's entries are the
+        sequences j != i with ShiftedScorer.scoreWithShift(seq1 = j, seq2 = i) >= threshold, best first under (score
+        desc, abundance[j] desc, j asc); slots past count[i] hold partner -1.  more = 1: more than k qualify."""
+        begin, end = (0, self.n) if rows is None else (int(rows[0]), int(rows[1]))
+        m = max(end - begin, 0)
+        partner = np.empty((m, max(int(k), 0)), dtype=np.int32)
+        score, shift = np.empty_like(partner), np.empty_like(partner)
+        count, more = np.empty(m, dtype=np.int32), np.empty(m, dtype=np.int32)
+        err = C.create_string_buffer(512)
+        rc = self._L.hmk_nearest(self._h, int(k), begin, end - begin, _ptr(partner, C.c_int32), _ptr(score, C.c_int32),
+                                 _ptr(shift, C.c_int32), _ptr(count, C.c_int32), _ptr(more, C.c_int32), err, 512)
+        if rc:
+            _raise_status(rc, err.value)
+        return partner, score, shift, count, more
+
     _KERNELS = {-1: "none", 0: "generic", 1: "fast", 2: "filter", 3: "long"}
 
     def bulk_probe(self, mode: int, query_ids, db=None, db_range=None, clustered=None, hit_cap: int = 0):
@@ -994,6 +1011,40 @@ def save_score_graph(sequences: Sequence[UniqueSequence], edges, path: str) -> N
             w.write("".join(f"{strs[i]}\t{strs[j]}\t{s}\t{k}\n"
                             for i, j, s, k in zip(e["seq"].tolist(), e["partner"].tolist(), e["score"].tolist(),
                                                   e["shift"].tolist())))
+
+
+def nearest_partners(sequences: Sequence[UniqueSequence], scoring_matrix, k: int = 8, threshold: Optional[int] = None,
+                     max_shift: Optional[int] = None, shift_penalty: int = 0, device: int = 0):
+    """The k nearest partners of every sequence of `sequences` (input order, as score_graph): the sequences j != i with
+    ShiftedScorer.scoreWithShift(seq j, seq i) >= threshold, best first under (score desc, size desc, j asc) ->
+    (partner, score, shift) [n, k] and (count, more) [n] as GreedyContext.nearest returns them.  Defaults:
+    setClinkageThreshold and getMaxShift."""
+    if len(sequences) == 0:
+        z = np.zeros((0, k), dtype=np.int32)
+        return z, z.copy(), z.copy(), np.zeros(0, np.int32), np.zeros(0, np.int32)
+    max_shift = get_max_shift(sequences) if max_shift is None else check_max_shift(sequences, max_shift)
+    if threshold is None:
+        threshold = set_clinkage_threshold(sequences)
+    res, offs, ab = pack_sequences(sequences)
+    ctx = GreedyContext(device)
+    try:
+        ctx.upload(res, offs, ab, scoring_matrix, threshold, max_shift, shift_penalty, 0)
+        return ctx.nearest(k)
+    finally:
+        ctx.close()
+
+
+def save_nearest_partners(sequences: Sequence[UniqueSequence], nearest, path: str) -> None:
+    """nearest_partners.tsv: header `sequence, rank, partner, score, shift`, then for every sequence in input order its
+    entries rank 1 .. count, sequences as strings.  `nearest`: what nearest_partners returns, for all sequences."""
+    partner, score, shift, count = (np.asarray(a) for a in nearest[:4])
+    strs = [s.get_sequence_string() for s in sequences]
+    with open(path, "w", newline="") as w:
+        w.write("sequence\trank\tpartner\tscore\tshift\n")
+        for i, c in enumerate(count.tolist()):
+            w.write("".join(f"{strs[i]}\t{r + 1}\t{strs[j]}\t{s}\t{h}\n"
+                            for r, (j, s, h) in enumerate(zip(partner[i, :c].tolist(), score[i, :c].tolist(),
+                                                              shift[i, :c].tolist()))))
 
 
 def rebuild_clusters(sequences: Sequence[UniqueSequence], r: GreedyResult) -> List[Cluster]:

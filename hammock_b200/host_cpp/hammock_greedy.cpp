@@ -6,6 +6,8 @@
 // clusterer on the sequences in INPUT order (no sorting, no cluster limit), same result files.
 // `hammock_greedy graph ...` writes the score graph both clusterings are built from: every pair of sequences (input order,
 // clinkage's automatic threshold and max shift) scoring >= threshold with its score and shift, to score_graph.tsv.
+// `hammock_greedy nearest ... [-k n]` writes, on the same sequences and parameters, the n (default 8) best-scoring
+// partners of every sequence with score and shift to nearest_partners.tsv, pulling rows in ranges.
 // Flags keep the reference's names (Hammock.java:824-970).  Multiple alignments are NOT built here
 // (that is the Clustal-Omega stage, outside this path): the alignment column is "NA" for multi-member
 // clusters, which `cluster` mode accepts.
@@ -17,15 +19,16 @@
 using namespace hammock;
 
 static void usage() {
-    std::cerr << "usage: hammock_greedy [greedy|clinkage|graph] -i <input.fa> -d <outdir> [-f fasta|tab] [-m <matrix.txt>] [-g <threshold>] [-x <max_shift>]\n"
+    std::cerr << "usage: hammock_greedy [greedy|clinkage|graph|nearest] -i <input.fa> -d <outdir> [-f fasta|tab] [-m <matrix.txt>] [-g <threshold>] [-x <max_shift>]\n"
                  "                      [-p <gap_penalty>] [--initial_clusters_limit <n>] [-R size|alphabetic|random|input|<label>]\n"
-                 "                      [-S <seed>] [-l label1,label2,...] [--device <n>] [--dump-prepared]\n";
+                 "                      [-S <seed>] [-l label1,label2,...] [-k <partners>] [--device <n>] [--dump-prepared]\n";
 }
 
 int main(int argc, char** argv) {
     std::string input, outdir, format = "fasta", matrixPath, order = "size";
     bool haveT = false, haveX = false, haveK = false, dump = false, haveLabels = false, timeHost = false, hostOnly = false;
-    bool clinkage = false, graph = false;   // graph: input order and clinkage's automatic parameters, like clinkage
+    bool clinkage = false, graph = false, nearest = false;   // graph, nearest: input order and clinkage's automatic parameters
+    int32_t nearestK = 8;
     int32_t threshold = 0, maxShift = 0, shiftPenalty = 0, limit = 0;   // shiftPenalty default 0 (Hammock.java:82)
     int64_t seed = 42;                                                   // Hammock.java:67
     int device = 0;
@@ -40,6 +43,8 @@ int main(int argc, char** argv) {
             if (a == "greedy") continue;
             else if (a == "clinkage" && i == 1) clinkage = true;
             else if (a == "graph" && i == 1) clinkage = graph = true;
+            else if (a == "nearest" && i == 1) clinkage = nearest = true;
+            else if (a == "-k" && nearest) nearestK = decode_int(next());
             else if (a == "-i" || a == "--input") input = next();
             else if (a == "-d" || a == "--outputDirectory") outdir = next();
             else if (a == "-f" || a == "--file_format") format = next();
@@ -65,6 +70,7 @@ int main(int argc, char** argv) {
             } else if (a == "-h" || a == "--help") { usage(); return 0; }
             else throw CLIException("Error. Unknown parameter: " + a);
         }
+        if (nearest && (nearestK < 1 || nearestK > HMK_NEAREST_MAX_K)) throw CLIException("Error. Parameter -k must be between 1 and 31.");
         if (input.empty()) throw CLIException("Error. Parameter input file (-i) missing with no default.");
         if (matrixPath.empty() && !dump) throw CLIException("Error. Parameter matrix (-m) missing (e.g. matrices/blosum62.txt of the Hammock distribution).");
         if (format != "fasta" && format != "tab") throw CLIException("Error. Wrong input file format. Use \"fasta\" or \"tab\"");
@@ -104,6 +110,7 @@ int main(int argc, char** argv) {
             std::cout << "threshold\t" << threshold << "\nmax_shift\t" << maxShift << "\nlimit\t" << limit << "\nlabels";
             for (auto& l : labels) std::cout << '\t' << l;
             std::cout << '\n';
+            if (nearest) std::cout << "k\t" << nearestK << '\n';
             for (auto& s : sequences) std::cout << s.sequence << '\t' << s.size() << '\n';
             return 0;
         }
@@ -124,6 +131,27 @@ int main(int argc, char** argv) {
             }
             auto ms = std::chrono::duration_cast<std::chrono::milliseconds>(std::chrono::steady_clock::now() - t0).count();
             std::cerr << "Ready. Time: " << ms << "\nEdges: " << edges << "\nScore graph in: " << d << "score_graph.tsv\n";
+            return 0;
+        }
+        if (nearest) {
+            if (outdir.empty()) throw CLIException("Error. Parameter output directory (-d) missing: nearest mode writes nearest_partners.tsv.");
+            std::string d = outdir;
+            if (d.back() != '/') d.push_back('/');
+            std::cerr << "Nearest partners... (" << sequences.size() << " unique sequences, k " << nearestK << ", threshold " << threshold
+                      << ", max shift " << maxShift << ")\n";
+            auto t0 = std::chrono::steady_clock::now();
+            int64_t entries = 0;
+            {
+                TsvWriter w(d + "nearest_partners.tsv");
+                writeNearestHeader(w);
+                entries = GpuNearestPartners{matrix, shiftPenalty, maxShift, threshold, nearestK, device}.pull(
+                    sequences, [&](int32_t r0, int32_t m, const int32_t* partner, const int32_t* score, const int32_t* shift,
+                                   const int32_t* count, const int32_t*) {
+                        writeNearestRows(w, sequences, r0, m, nearestK, partner, score, shift, count);
+                    });
+            }
+            auto ms = std::chrono::duration_cast<std::chrono::milliseconds>(std::chrono::steady_clock::now() - t0).count();
+            std::cerr << "Ready. Time: " << ms << "\nEntries: " << entries << "\nNearest partners in: " << d << "nearest_partners.tsv\n";
             return 0;
         }
         std::cerr << (clinkage ? "Clinkage" : "Greedy") << " clustering... (" << sequences.size() << " unique sequences, threshold " << threshold

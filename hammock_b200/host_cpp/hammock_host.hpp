@@ -581,6 +581,43 @@ struct GpuScoreGraph {
     }
 };
 
+// The k nearest partners of every sequence of `seqs` in the caller's order (hmk_nearest on a context of its own): for
+// each i, the sequences j != i with scoreWithShift(seq j, seq i) >= threshold, best first under (score desc, size desc,
+// j asc).  Handed to fn(row_begin, n_rows, partner, score, shift, count, more) `rows` rows at a time (partner, score,
+// shift: [n_rows][k]), so that host memory stays bounded.  Returns the number of entries.
+struct GpuNearestPartners {
+    std::vector<int32_t> matrix;
+    int32_t shiftPenalty, maxShift, threshold, k;
+    int device = 0;
+
+    template <class Fn>
+    int64_t pull(const std::vector<UniqueSequence>& seqs, Fn&& fn, int32_t rows = 1 << 16) const {
+        const int32_t n = (int32_t)seqs.size();
+        const PackedSequences packed(seqs);
+        hmk_greedy_in in{n, packed.res.data(), packed.off.data(), packed.ab.data(), matrix.data(), threshold, maxShift, shiftPenalty, 0};
+        char err[512] = {0};
+        auto check = [&](int rc) {
+            if (rc == HMK_STATUS_SHIFT_TOO_BIG) throw DataException(err);
+            if (rc == HMK_STATUS_BAD_RESIDUE) throw FileFormatException(err);
+            if (rc != HMK_STATUS_OK) throw CudaException(std::string("hammock_b200: ") + err);
+        };
+        hmk_ctx* ctx = nullptr;
+        check(hmk_create(&ctx, device, err, sizeof err));
+        struct Destroy { hmk_ctx* c; ~Destroy() { hmk_destroy(c); } } destroy{ctx};
+        check(hmk_upload(ctx, &in, err, sizeof err));
+        const size_t cap = (size_t)std::min(rows, std::max(n, 1));
+        std::vector<int32_t> partner(cap * std::max(k, 1)), score(partner.size()), shift(partner.size()), count(cap), more(cap);
+        int64_t total = 0;
+        for (int32_t r0 = 0; r0 < n; r0 += (int32_t)cap) {
+            const int32_t m = std::min<int32_t>((int32_t)cap, n - r0);
+            check(hmk_nearest(ctx, k, r0, m, partner.data(), score.data(), shift.data(), count.data(), more.data(), err, sizeof err));
+            fn(r0, m, partner.data(), score.data(), shift.data(), count.data(), more.data());
+            for (int32_t t = 0; t < m; t++) total += count[t];
+        }
+        return total;
+    }
+};
+
 // ---------------------------------------------------------------- result files (FileIOManager.java)
 static const char SEP = '\t';   // Hammock.CSV_SEPARATOR (Hammock.java:35)
 
@@ -713,6 +750,21 @@ inline void writeScoreGraphHeader(TsvWriter& w) { w << "sequence" << SEP << "par
 inline void writeScoreGraphEdges(TsvWriter& w, const std::vector<UniqueSequence>& seqs, const hmk_graph_edge* e, size_t count) {
     for (size_t k = 0; k < count; k++)
         w << seqs[e[k].seq].sequence << SEP << seqs[e[k].partner].sequence << SEP << e[k].score << SEP << e[k].shift << '\n';
+}
+
+// nearest_partners.tsv (nearest mode): the header, then for each row its entries rank 1 .. count as sequence strings --
+// the same bytes as the Python host's save_nearest_partners
+inline void writeNearestHeader(TsvWriter& w) {
+    w << "sequence" << SEP << "rank" << SEP << "partner" << SEP << "score" << SEP << "shift" << '\n';
+}
+inline void writeNearestRows(TsvWriter& w, const std::vector<UniqueSequence>& seqs, int32_t row_begin, int32_t n_rows, int32_t k,
+                             const int32_t* partner, const int32_t* score, const int32_t* shift, const int32_t* count) {
+    for (int32_t t = 0; t < n_rows; t++)
+        for (int32_t r = 0; r < count[t]; r++) {
+            const size_t e = (size_t)t * k + r;
+            w << seqs[row_begin + t].sequence << SEP << (r + 1) << SEP << seqs[partner[e]].sequence << SEP << score[e] << SEP
+              << shift[e] << '\n';
+        }
 }
 
 // saveInputStatistics (FileIOManager.java:709-729); no newline after the last line

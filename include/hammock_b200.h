@@ -162,7 +162,9 @@ int hmk_measure_peaks(hmk_ctx* ctx, double* out4, char* errbuf, size_t errlen);
  * the n x n matrix; sparse: the counting pass), [1] sparse row build (the filling pass, row sort and twin index; 0 on the
  * dense path), [2] nearest-neighbour chain; the others are 0.
  * hmk_score_graph adds to slots [0] (scoring passes) and [1] (shift, sort and edge passes) the device time of the batches
- * it computes; a call at cursor {0, 0} sets both to 0 first. */
+ * it computes; a call at cursor {0, 0} sets both to 0 first.
+ * hmk_nearest sets slots [0] (scoring pass: profiles and the top-k launch) and [1] (list merge, score and shift) to the
+ * device time of the row batches of the call. */
 #define HMK_NSECTIONS 13
 int hmk_get_section_ms(hmk_ctx* ctx, double* out, int n);
 /* tuning knobs; unknown names and out-of-range values return HMK_STATUS_BAD_ARG.  None of them changes the result.
@@ -222,6 +224,22 @@ int hmk_score_graph(hmk_ctx* ctx, int64_t cursor[2], hmk_graph_edge* out, int64_
  * call before hmk_upload. */
 int hmk_score_pairs(hmk_ctx* ctx, const int32_t* seq1_ids, const int32_t* seq2_ids, int32_t n_pairs, int32_t* scores,
                     int32_t* shifts, char* errbuf, size_t errlen);
+
+/* Nearest partners: for each row i in [row_begin, row_begin + n_rows) of the uploaded sequences (ids in upload order), the
+ * k best-scoring other sequences j with s = scoreWithShift(seq1 = j, seq2 = i).score >= threshold (the partner search's
+ * argument order), ordered by (s desc, abundance[j] desc, j asc) -- the partner search's candidate order, for any order
+ * of the abundances.  partner, score and shift are [n_rows][k], row-major: entry r of row i is its (r + 1)-th partner
+ * with that score and its shift (the lowest winning diagonal, negated when seq1 is the shorter sequence); slots past
+ * count[i - row_begin] hold partner -1, score 0, shift 0.  more[i - row_begin] = 1 when more than k sequences qualify.
+ * For j > i an entry is the score graph's edge (i, j); with a symmetric matrix every score equals the graph's.  An
+ * asymmetric matrix is accepted.  Rows are independent and the call keeps no state, so a host may bound its memory by
+ * pulling row ranges, or split the rows over contexts.  Option kb does not apply.  Status: HMK_STATUS_SHIFT_TOO_BIG when
+ * n >= 2 and max_shift >= the shortest length, HMK_STATUS_BAD_RESIDUE, HMK_STATUS_BAD_ARG for a call before hmk_upload,
+ * k outside 1 .. HMK_NEAREST_MAX_K, a row range outside [0, n], or a null output with n_rows > 0.  n of 0 or 1: empty
+ * lists. */
+#define HMK_NEAREST_MAX_K 31
+int hmk_nearest(hmk_ctx* ctx, int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partner, int32_t* score,
+                int32_t* shift, int32_t* count, int32_t* more, char* errbuf, size_t errlen);
 
 /* One bulk scoring launch over the uploaded sequences with the context's scheme and options.  Used by the kernel tests.
  * Profile side: query_ids[0 .. n_query), as seq2.  Thread side (seq1): db_ids[0 .. n_db), or with db_ids NULL the ids

@@ -1,5 +1,5 @@
 """Builds the library with -DHMK_CHECKED (in-kernel bounds assertions, hmk_common.h) next to the normal one and runs the
-bulk-kernel and batch-table tests, the randomised differential tier, the boundary tests and the clinkage tests (dense and sparse path) against it (HMK_LIB selects the library the
+bulk-kernel and batch-table tests, the randomised differential tier, the boundary tests, the clinkage tests (dense and sparse path) and the nearest-partner tests against it (HMK_LIB selects the library the
 host layer loads).  A failing assertion prints `file:line: ... Assertion ... failed` from the device and the call
 returns HMK_STATUS_CUDA, so the test fails with the line in the log.  compute-sanitizer is not available on the pool.
 
@@ -21,7 +21,7 @@ def main():
     cmd = [sys.executable, "-m", "pytest", "-m", "gpu", "-q", "-x", "tests/test_bulk_kernels.py", "tests/test_batch_tables.py",
            "tests/test_gpu_fuzz.py",
            "tests/test_gpu_boundary.py", "tests/test_clinkage.py", "tests/test_clinkage_large.py", "tests/test_gpu_parity.py",
-           "tests/test_p1_pipeline.py"] + sys.argv[1:]
+           "tests/test_p1_pipeline.py", "tests/test_nearest.py"] + sys.argv[1:]
     with open(os.path.join(ROOT, "gpurun_out", "checked_fuzz.log"), "w") as log:
         log.write("library: " + lib + "\n$ " + " ".join(cmd) + "\n")
         log.flush()
