@@ -302,6 +302,8 @@ private:
     std::vector<int32_t> h_bucket_[HMK_MAXLEN + 1];   // ids per length, ascending
     DevBuf<int32_t> d_bucket_[HMK_MAXLEN + 1];
     DevBuf<int32_t> d_sidx_, d_sb_ids_, d_sb_cnt_;
+    DevBuf<int32_t> d_ids_;      // 0 .. n - 1: the profile ids of the whole-input calls (identity_ids)
+    bool ids_filled_ = false;
     DevBuf<uint32_t> d_pcells_, d_pops_;
     bool fast_scalar_ = false;   // every length <= 12: the one-at-a-time scorer works on the packed words (which carry the lengths)
     HmkScheme sc_{};
@@ -391,7 +393,7 @@ private:
     void graph_batch(int q0);
     void shift_pass(const int4* pairs, const unsigned int* count, unsigned int cap, int q0, int jbits,
                     unsigned long long* keys, unsigned long long* vals, unsigned int* kept, int32_t* score, int32_t* shift);
-    // nearest partners (hmk_nearest): the query batch's ids, profiles, top-k lists and gmin bounds, and its output rows --
+    // nearest partners (hmk_nearest): the query batch's profiles, top-k lists and gmin bounds, and its output rows --
     // the nearest search's own, so that nothing of it reaches a clustering run's batch buffers
     BatchBuf near_bb_;
     DevBuf<int32_t> d_near_out_;
@@ -440,11 +442,15 @@ private:
         return S;
     }
     void choose_scheme(const int32_t* M);
-    int qt_max() const { return qt_max(sc_); }
-    int qt_max(const HmkScheme& sc) const;
+    int qt_max(const HmkScheme& sc, int kb) const;
     HmkScheme scheme_for(int n) const;
     void launch_profiles(int mode, const int32_t* ids, int nq, uint32_t* prof, const HmkScheme& sc, cudaStream_t s,
                          uint32_t* cells = nullptr, uint32_t* ops = nullptr);
+    const int32_t* identity_ids();
+    HmkBulkArgs query_batch(const int32_t* ids, int nq, uint32_t* prof, int kb);
+    void merge_topk(int nq, int nstripes, int kb, const uint64_t* key, const int32_t* cnt, const int32_t* ovf, BatchBuf& out,
+                    cudaStream_t s, const int32_t* slots = nullptr, int qt = 1);
+    void report_kernel(const BulkKernel& k, bool persistent, int32_t* out) const;
     void plan_bulk(int mode, HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched = nullptr) const;
     BulkKernel launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch, const int32_t* prof_ids, int prof_is_query,
                               cudaStream_t s);
@@ -463,6 +469,13 @@ private:
         sec_open_ = id;
         sec_start_ = e;
     }
+    void reset_timing() {   // a call's timing starts empty: no recorded events, no open section
+        ev_used_ = 0;
+        bulk_events_.clear();
+        sections_.clear();
+        sec_open_ = -1;
+    }
+    double fold_timing();
 public:
     double section_ms[HMK_NSECTIONS] = {0};
 private:
@@ -563,6 +576,7 @@ void Engine::upload(const hmk_greedy_in* in) {
     CK(cudaSetDevice(device_));
     uploaded_ = false;      // a rejected upload leaves nothing to run
     ran_ = false;
+    ids_filled_ = false;
     graph_.valid = false; graph_.next_i = graph_.next_r = -1; graph_.sn = HMK_MAXBATCH;
     if (!in || in->n < 0 || (in->n > 0 && (!in->residues || !in->offsets || !in->abundance)) || !in->matrix)
         throw std::invalid_argument("hmk_upload: null input");
@@ -630,7 +644,6 @@ void Engine::upload(const hmk_greedy_in* in) {
     }
     fast_scalar_ = n_ > 0 && min_len_ >= 1 && max_len_ <= HMK_MAXL1 && X_ >= 0 && X_ < min_len_;
     // validate residues + pack 5 bits/residue on the device
-    words_ = max_len_ <= HMK_MAXLEN ? std::max(1, (max_len_ + HMK_MAXL1 - 1) / HMK_MAXL1) : 1;
     d_packed_.reserve((size_t)std::max(n_, 1) * words_);
     d_flags_.reserve(8);
     CK(cudaMemsetAsync(d_flags_.p, 0, 8 * sizeof(int32_t), st_));
@@ -662,14 +675,34 @@ cudaEvent_t Engine::next_event() {
     return ev_pool_[ev_used_++];
 }
 
-int Engine::qt_max(const HmkScheme& sc) const {
+// adds each closed section's device time to its slot of section_ms and returns the summed time of the recorded bulk
+// launches, then recycles the event pool; the events on other streams than st_ must be complete
+double Engine::fold_timing() {
+    if (opt.profile) CK(cudaStreamSynchronize(st_));
+    double bulk_ms = 0;
+    for (auto& pr : bulk_events_) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, pr.first, pr.second));
+        bulk_ms += ms;
+    }
+    for (auto& sct : sections_) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, sct.second.first, sct.second.second));
+        section_ms[sct.first] += ms;
+    }
+    reset_timing();
+    return bulk_ms;
+}
+
+// kb: the per-query list length of the launch (HmkBulkArgs::kb); EMIT and DENSE launches are sized with it too
+int Engine::qt_max(const HmkScheme& sc, int kb) const {
     if (opt.qt > 0) return (int)opt.qt;
     // a profile with its share of the carve-up, beside the hit queues of a 768-thread block and 128 bytes for the barrier
     // and alignment.  The 512-thread long kernel is sized the same way: its tiles are the ones it was measured with.
     // The filter kernel adds a prefix sum per profile and warp (hmk_packed_smem), with up to 12 bytes of alignment per warp.
     const size_t warps = HMK_BULK_THREADS / 32;
-    const size_t per = (size_t)sc.prof_words * 4 + hmk_carve_bytes(1, (int)opt.kb, 0, false) + (sc.filter ? warps * 4 : 0);
-    const size_t fixed = 128 + hmk_carve_bytes(0, (int)opt.kb, HMK_BULK_THREADS, false) + (sc.filter ? 16 + warps * 12 : 0);
+    const size_t per = (size_t)sc.prof_words * 4 + hmk_carve_bytes(1, kb, 0, false) + (sc.filter ? warps * 4 : 0);
+    const size_t fixed = 128 + hmk_carve_bytes(0, kb, HMK_BULK_THREADS, false) + (sc.filter ? 16 + warps * 12 : 0);
     // the filter kernel's tile stays at the 56 profiles the batch size and chunking were measured with (more would fit)
     const size_t cap = sc.filter ? HMK_FILTER_QT : 255;
     return (int)std::min<size_t>(cap, std::max<size_t>(1, (smem_optin_ - fixed) / per));
@@ -690,6 +723,57 @@ void Engine::launch_profiles(int mode, const int32_t* ids, int nq, uint32_t* pro
     hmk_build_profiles<<<nq, 128, 0, s>>>(sc, mode, ids, nq, d_res_.p, d_off_.p, d_M_.p, prof, cells, ops);
     CK(cudaGetLastError());
     launches_++;
+}
+
+// the ids 0 .. n - 1 on the device, copied once per upload when a call first needs them
+const int32_t* Engine::identity_ids() {
+    if (!ids_filled_) {
+        std::vector<int32_t> ids(n_);
+        std::iota(ids.begin(), ids.end(), 0);
+        d_ids_.reserve(std::max(n_, 1));
+        CK(cudaMemcpyAsync(d_ids_.p, ids.data(), sizeof(int32_t) * n_, cudaMemcpyHostToDevice, st_));
+        ids_filled_ = true;
+    }
+    return d_ids_.p;
+}
+
+// the profile side of a bulk launch on st_ over the query ids[0 .. nq): their profiles in `prof` (packed kernels) and
+// the list length kb; the caller sets the thread side and the mode's fields
+HmkBulkArgs Engine::query_batch(const int32_t* ids, int nq, uint32_t* prof, int kb) {
+    if (fast_) launch_profiles(HMK_PROF_QUERY, ids, nq, prof, sc_, st_);
+    HmkBulkArgs a{};
+    a.prof = prof; a.nq = nq; a.kb = kb;
+    a.packed = d_packed_.p;
+    return a;
+}
+
+// merges nstripes lists of kb keys per query ([nstripes][nq][kb]) into out.bk_*; slots / qt: the slot counters of a
+// persistent launch (HmkBulkArgs::sched + nqt) and its profiles per tile
+void Engine::merge_topk(int nq, int nstripes, int kb, const uint64_t* key, const int32_t* cnt, const int32_t* ovf, BatchBuf& out,
+                        cudaStream_t s, const int32_t* slots, int qt) {
+    hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, s>>>(nq, nstripes, kb, key, cnt, ovf, out.bk_key.p, out.bk_cnt.p, out.bk_ovf.p,
+                                                         slots, qt);
+    CK(cudaGetLastError());
+    launches_++;
+}
+
+// which kernel a probe's launch ran (kind -1: none, the launch was empty): kind, the filter kernel's compile-time length,
+// words per profile entry, lane bits, persistent grid
+void Engine::report_kernel(const BulkKernel& k, bool persistent, int32_t* out) const {
+    const bool packed = k.kind > BulkKernel::GENERIC;
+    out[0] = k.kind;
+    out[1] = k.lt;
+    out[2] = packed ? sc_.nw : 0;
+    out[3] = packed ? (sc_.lane16 ? 16 : 8) : k.fn ? 32 : 0;
+    out[4] = persistent ? 1 : 0;
+}
+
+// (x, y, z) of the first `stored` hits of a device buffer, as int32 triples
+static void copy_hit_triples(const int4* d_hits, size_t stored, int32_t* out) {
+    if (!stored) return;
+    std::vector<int4> h(stored);
+    CK(cudaMemcpy(h.data(), d_hits, sizeof(int4) * stored, cudaMemcpyDeviceToHost));
+    for (size_t e = 0; e < stored; e++) { out[3 * e] = h[e].x; out[3 * e + 1] = h[e].y; out[3 * e + 2] = h[e].z; }
 }
 
 // the bulk kernel of a (MODE, scheme) pair; `sch` NULL: the generic kernel
@@ -722,7 +806,7 @@ static BulkKernel bulk_kernel(int mode, const HmkScheme* sch) {
 void Engine::plan_bulk(int mode, HmkBulkArgs& a, const HmkScheme* sch, int32_t* sched) const {
     const int threads = bulk_kernel(mode, sch).threads;
     const int sms = plan_sms_ > 0 ? plan_sms_ : sm_count_;
-    int qmax = sch ? qt_max(*sch) : 128;
+    int qmax = sch ? qt_max(*sch, a.kb) : 128;
     if (!sch) {     // generic kernel: a thread scores its item against the whole tile, one pair after the other -- small
                     // databases get small tiles, so that there are about two CTAs per SM instead of a few long threads
         const int64_t blocks = (a.ndb + threads - 1) / threads;
@@ -775,7 +859,6 @@ BulkKernel Engine::launch_planned(int mode, HmkBulkArgs a, const HmkScheme* sch,
                                   cudaStream_t s) {
     a.sc = sch ? *sch : sc_;
     a.pair_counter = d_pairctr_.p;
-    a.kb = (int)opt.kb;
     const int grid = a.sched ? a.nstripes : a.nqt * a.nstripes;
     if (a.sched) CK(cudaMemsetAsync(a.sched, 0, sizeof(int32_t) * 2 * a.nqt, s));
     const BulkKernel k = bulk_kernel(mode, sch);
@@ -819,7 +902,7 @@ HmkBulkArgs Engine::launch_bulk(int mode, HmkBulkArgs a, const int32_t* prof_ids
     plan_bulk(mode, a, sch, mode == HMK_MODE_DENSE ? nullptr : sched.p);
     if (mode == HMK_MODE_TOPK) {
         const size_t slots = (size_t)a.nstripes * a.nq;
-        bb->tk_key.reserve(slots * opt.kb); bb->tk_cnt.reserve(slots); bb->tk_ovf.reserve(slots);
+        bb->tk_key.reserve(slots * a.kb); bb->tk_cnt.reserve(slots); bb->tk_ovf.reserve(slots);
         a.tk_key = bb->tk_key.p; a.tk_cnt = bb->tk_cnt.p; a.tk_ovf = bb->tk_ovf.p;
         a.stripe_base = 0;
     }
@@ -859,7 +942,7 @@ void Engine::sort_pairs(unsigned long long* keys, int32_t* vals, int n, int begi
 void Engine::founder_hits(BatchBuf& bb, int from, int to, cudaStream_t s, DevBuf<int32_t>& sched) {
     if (to <= from) return;
     HmkBulkArgs a{};
-    a.prof = bb.prof.p; a.nq = bb.nq;
+    a.prof = bb.prof.p; a.nq = bb.nq; a.kb = (int)opt.kb;
     a.packed = d_packed_.p; a.db_ids = d_cf_.p + from; a.db_begin = 0; a.ndb = to - from;
     a.hits = bb.hits.p; a.hit_count = bb.hcount.p; a.hit_cap = (unsigned int)bb.hit_cap;
     a.discards = &d_ctl_.p->discards; a.discards_seen = h_ctl_->discards;
@@ -917,7 +1000,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
         CK(cudaMemcpyAsync(bb.qid.p, bb.gqid.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToDevice, s));
     }
     HmkBulkArgs a{};
-    a.nq = nq;
+    a.nq = nq; a.kb = kb;
     a.packed = d_packed_.p; a.slot = d_slot_.p; a.q_minid = bb.qid.p;
     a.tierank = identity_rank_ ? nullptr : d_tierank_.p;
     a.discards = &d_ctl_.p->discards; a.discards_seen = h_ctl_->discards;
@@ -1002,11 +1085,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
         CK(cudaMemsetAsync(bb.bk_ovf.p, 0, sizeof(int32_t) * nq, s));
     }
     auto merge_stripe_lists = [&](cudaStream_t ms) {
-        if (merge_stripes == 0) return;
-        hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, ms>>>(nq, merge_stripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
-                                                              bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p, merge_slots, merge_qt);
-        CK(cudaGetLastError());
-        launches_++;
+        if (merge_stripes) merge_topk(nq, merge_stripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p, bb, ms, merge_slots, merge_qt);
     };
     if (world_ > 1) {
         merge_stripe_lists(s);
@@ -1022,14 +1101,8 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
     // ---- tail, on `t`
     CK(cudaEventRecord(bb.searched, s));
     if (t != s) CK(cudaStreamWaitEvent(t, bb.searched, 0));
-    if (world_ > 1) {
-        hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, t>>>(nq, world_, kb, bb.gk_key.p, bb.gk_cnt.p, bb.gk_ovf.p,
-                                                             bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p);
-        CK(cudaGetLastError());
-        launches_++;
-    } else {
-        merge_stripe_lists(t);
-    }
+    if (world_ > 1) merge_topk(nq, world_, kb, bb.gk_key.p, bb.gk_cnt.p, bb.gk_ovf.p, bb, t);
+    else merge_stripe_lists(t);
     // intra-batch scores S(member = q_b2, query = q_b); row strides padded to 16 bytes for the TMA row prefetch
     const int ib_stride = (nq + 3) & ~3, pd_stride = (nq * kb + 3) & ~3, nw = (nq + 31) / 32;
     bb.ib.reserve((size_t)HMK_MAXBATCH * (HMK_MAXBATCH + 4)); bb.ibm.reserve((size_t)HMK_MAXBATCH * (HMK_MAXBATCH / 32)); bb.ibm2.reserve((size_t)HMK_MAXBATCH * (HMK_MAXBATCH / 32));
@@ -1041,7 +1114,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
         launches_++;
     } else {
         HmkBulkArgs d{};
-        d.prof = bb.prof.p; d.nq = nq;
+        d.prof = bb.prof.p; d.nq = nq; d.kb = kb;
         d.packed = d_packed_.p; d.db_ids = bb.qid.p; d.db_begin = 0; d.ndb = nq;
         d.dense = bb.ib.p; d.dense_stride = ib_stride;
         launch_bulk(HMK_MODE_DENSE, d, bb.qid.p, 1, t);
@@ -1061,7 +1134,7 @@ void Engine::stage_partner_search(BatchBuf& bb, int nq, int db_from, const int32
             launches_++;
         } else {
             HmkBulkArgs d{};
-            d.prof = bb.prof.p; d.nq = nq;
+            d.prof = bb.prof.p; d.nq = nq; d.kb = kb;
             d.packed = d_packed_.p; d.db_ids = bb.pcand.p; d.db_begin = 0; d.ndb = npc;
             d.dense = bb.pd.p; d.dense_stride = pd_stride;
             launch_bulk(HMK_MODE_DENSE, d, bb.qid.p, 1, t);
@@ -1112,9 +1185,8 @@ void Engine::check_members(const BatchBuf& cb, int ncl, int capq) {
 
 int Engine::phase1() {
     int B = (int)opt.batch;
-    if (B <= 0) B = fast_ ? (sc_.filter ? 8 : 3) * qt_max() : 192;   // measured optimum on the 1 M workload
+    if (B <= 0) B = fast_ ? (sc_.filter ? 8 : 3) * qt_max(sc_, (int)opt.kb) : 192;   // measured optimum on the 1 M workload
     B = std::max(1, std::min(B, HMK_MAXBATCH));
-    opt.kb = std::max<int64_t>(1, std::min<int64_t>(opt.kb, 32));
     const size_t resolve_avail = smem_optin_ - 3 * HMK_HASH_SIZE * 4 - 1024;   // minus the kernel's static shared memory
     {   // the resolver keeps the whole batch's bookkeeping in shared memory
         auto need = [&](int b) { return hmk_resolve_fixed_bytes(b, (b + 31) / 32, (int)opt.kb) + 64; };
@@ -1273,7 +1345,7 @@ void Engine::phase2() {
             sec(SEC_P2_FILTER);
             CK(cudaMemsetAsync(d_counts_.p, 0, sizeof(unsigned int), st_));
             HmkBulkArgs a{};
-            a.prof = d_fprof_.p; a.nq = ncl;
+            a.prof = d_fprof_.p; a.nq = ncl; a.kb = (int)opt.kb;
             a.packed = d_packed_.p; a.db_ids = ids + c0; a.db_begin = 0; a.ndb = cn;
             a.hits = d_hits_.p; a.hit_count = d_counts_.p; a.hit_cap = (unsigned int)hit_cap;
             if (sch && mixed_) { a.prof_cells = d_pcells_.p; a.prof_ops = d_pops_.p; }
@@ -1522,10 +1594,7 @@ int Engine::run() {
     stats.error_step = -1;
     error_step = -1;
     launches_ = bulk_launches_ = 0;
-    ev_used_ = 0;
-    bulk_events_.clear();
-    sections_.clear();
-    sec_open_ = -1;
+    reset_timing();
     for (double& v : section_ms) v = 0;
     ran_ = false;
     if (bad_residue_) return HMK_ERR_BAD_RESIDUE;
@@ -1573,18 +1642,7 @@ int Engine::run() {
     CK(cudaEventElapsedTime(&ms1, ev_a_, ev_b_));
     CK(cudaEventElapsedTime(&ms2, ev_b_, ev_c_));
     stats.phase1_ms = ms1; stats.phase2_ms = ms2; stats.total_ms = ms1 + ms2;
-    double bulk_ms = 0;
-    for (auto& pr : bulk_events_) {
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, pr.first, pr.second));
-        bulk_ms += ms;
-    }
-    for (auto& sct : sections_) {
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, sct.second.first, sct.second.second));
-        section_ms[sct.first] += ms;
-    }
-    stats.bulk_kernel_ms = bulk_ms;
+    stats.bulk_kernel_ms = fold_timing();
     stats.bulk_pairs = (int64_t)pc[0];
     stats.scalar_pairs = h_ctl_->scalar_pairs + (int64_t)scalar_sharded;
 #ifdef HMK_DEBUG
@@ -1645,10 +1703,8 @@ void Engine::score_block(const int32_t* first, int32_t nf, const int32_t* second
     for (int s0 = 0; s0 < ns; s0 += chunk) {
         const int sn = std::min(chunk, ns - s0);
         CK(cudaMemcpyAsync(d_second.p, second + s0, sizeof(int32_t) * sn, cudaMemcpyHostToDevice, st_));
-        if (fast_) launch_profiles(HMK_PROF_QUERY, d_second.p, sn, d_prof.p, sc_, st_);
-        HmkBulkArgs a{};
-        a.prof = d_prof.p; a.nq = sn;
-        a.packed = d_packed_.p; a.db_ids = d_first.p; a.db_begin = 0; a.ndb = nf;
+        HmkBulkArgs a = query_batch(d_second.p, sn, d_prof.p, (int)opt.kb);
+        a.db_ids = d_first.p; a.db_begin = 0; a.ndb = nf;
         a.dense = d_out.p; a.dense_stride = nf;
         launch_bulk(HMK_MODE_DENSE, a, d_second.p, 1);
         CK(cudaMemcpyAsync(tmp.data(), d_out.p, sizeof(int32_t) * (size_t)sn * nf, cudaMemcpyDeviceToHost, st_));
@@ -1680,9 +1736,8 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
     BatchBuf bb;
     d_q.reserve(std::max(nq, 1));
     if (nq) CK(cudaMemcpyAsync(d_q.p, qids, sizeof(int32_t) * nq, cudaMemcpyHostToDevice, st_));
-    HmkBulkArgs a{};
-    a.nq = nq;
-    a.packed = d_packed_.p;
+    if (fast_) bb.prof.reserve((size_t)std::max(nq, 1) * sc_.prof_words);
+    HmkBulkArgs a = query_batch(d_q.p, nq, bb.prof.p, kb);
     a.db_begin = db_begin; a.ndb = ndb;
     if (db_ids) {
         d_db.reserve(std::max(ndb, 1));
@@ -1696,11 +1751,6 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
         d_slot.reserve(h_slot.size());
         CK(cudaMemcpyAsync(d_slot.p, h_slot.data(), sizeof(int32_t) * h_slot.size(), cudaMemcpyHostToDevice, st_));
         a.slot = d_slot.p;
-    }
-    if (fast_) {
-        bb.prof.reserve((size_t)std::max(nq, 1) * sc_.prof_words);
-        launch_profiles(HMK_PROF_QUERY, d_q.p, nq, bb.prof.p, sc_, st_);
-        a.prof = bb.prof.p;
     }
     DevBuf<int4> d_hits;
     DevBuf<unsigned long long> d_count;
@@ -1719,11 +1769,7 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
         p = launch_bulk(HMK_MODE_TOPK, a, d_q.p, 1, st_, &bb, nullptr, &k);
         bb.bk_key.reserve((size_t)std::max(nq, 1) * kb); bb.bk_cnt.reserve(std::max(nq, 1)); bb.bk_ovf.reserve(std::max(nq, 1));
         if (nq && ndb) {
-            hmk_topk_merge<<<(nq * 32 + 255) / 256, 256, 0, st_>>>(nq, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
-                                                                  bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p,
-                                                                  p.sched ? p.sched + p.nqt : nullptr, p.qt);
-            CK(cudaGetLastError());
-            launches_++;
+            merge_topk(nq, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p, bb, st_, p.sched ? p.sched + p.nqt : nullptr, p.qt);
             CK(cudaMemcpyAsync(keys, bb.bk_key.p, sizeof(uint64_t) * nq * kb, cudaMemcpyDeviceToHost, st_));
             CK(cudaMemcpyAsync(cnt, bb.bk_cnt.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
             CK(cudaMemcpyAsync(ovf, bb.bk_ovf.p, sizeof(int32_t) * nq, cudaMemcpyDeviceToHost, st_));
@@ -1741,20 +1787,8 @@ void Engine::bulk_probe(int mode, const int32_t* qids, int32_t nq, const int32_t
     if (mode == 0) total = *reinterpret_cast<unsigned long long*>(h_scalars_);
     else total = *reinterpret_cast<unsigned int*>(h_scalars_);
     *hit_count = (int64_t)total;
-    const size_t stored = (size_t)std::min<unsigned long long>(total, (unsigned long long)hit_cap);
-    if (stored) {
-        std::vector<int4> h((size_t)stored);
-        CK(cudaMemcpy(h.data(), d_hits.p, sizeof(int4) * stored, cudaMemcpyDeviceToHost));
-        for (size_t e = 0; e < stored; e++) { hits[3 * e] = h[e].x; hits[3 * e + 1] = h[e].y; hits[3 * e + 2] = h[e].z; }
-    }
-    // which kernel ran (kind -1: none, the launch was empty): kind, the filter kernel's compile-time length, words per
-    // profile entry, lane bits, persistent grid
-    const bool packed = k.kind > BulkKernel::GENERIC;
-    kernel[0] = k.kind;
-    kernel[1] = k.lt;
-    kernel[2] = packed ? sc_.nw : 0;
-    kernel[3] = packed ? (sc_.lane16 ? 16 : 8) : k.fn ? 32 : 0;
-    kernel[4] = k.fn && p.sched ? 1 : 0;
+    copy_hit_triples(d_hits.p, (size_t)std::min<unsigned long long>(total, (unsigned long long)hit_cap), hits);
+    report_kernel(k, k.fn && p.sched, kernel);
 }
 
 // Phase 1's per-batch work on a clustering state given by the caller (hmk_batch_probe): the state goes into the
@@ -1806,7 +1840,6 @@ void Engine::batch_probe(const int32_t* member_off, const int32_t* members, int3
     d_pairparts_.reserve(HMK_PAIR_SHARDS * 16);
     CK(cudaStreamSynchronize(st_));      // the side streams start from here
     // ---- one batch, as phase1 runs it (no kept hits for phase 2, every SM for the bulk launches)
-    opt.kb = std::max<int64_t>(1, std::min<int64_t>(opt.kb, 32));      // as phase1
     const int kb = (int)opt.kb;
     const int cq = capq > 0 ? capq : (int)std::max<int64_t>(1, opt.capq);
     nq = std::min(nq, unproc);
@@ -1852,20 +1885,9 @@ void Engine::batch_probe(const int32_t* member_off, const int32_t* members, int3
         out->ac_best[4 * b] = r.x; out->ac_best[4 * b + 1] = r.y; out->ac_best[4 * b + 2] = r.z; out->ac_best[4 * b + 3] = r.w;
     }
     out->fhit_count = hcount;
-    const size_t stored = std::min<size_t>({(size_t)hcount, bb.hit_cap, (size_t)out->fhit_cap});
-    if (stored) {
-        std::vector<int4> h(stored);
-        CK(cudaMemcpy(h.data(), bb.hits.p, sizeof(int4) * stored, cudaMemcpyDeviceToHost));
-        for (size_t e = 0; e < stored; e++) { out->fhits[3 * e] = h[e].x; out->fhits[3 * e + 1] = h[e].y; out->fhits[3 * e + 2] = h[e].z; }
-    }
-    const BulkKernel& k = log.last[HMK_MODE_TOPK];
-    const bool packed = k.kind > BulkKernel::GENERIC;
+    copy_hit_triples(bb.hits.p, std::min<size_t>({(size_t)hcount, bb.hit_cap, (size_t)out->fhit_cap}), out->fhits);
     int32_t* kr = out->kernel;
-    kr[0] = k.kind;
-    kr[1] = k.lt;
-    kr[2] = packed ? sc_.nw : 0;
-    kr[3] = packed ? (sc_.lane16 ? 16 : 8) : k.fn ? 32 : 0;
-    kr[4] = log.persistent ? 1 : 0;
+    report_kernel(log.last[HMK_MODE_TOPK], log.persistent, kr);
     kr[5] = log.count[HMK_MODE_TOPK];
     kr[6] = log.last[HMK_MODE_DENSE].kind;
     kr[7] = log.count[HMK_MODE_DENSE];
@@ -1884,7 +1906,7 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     stats.error_step = -1;
     status_msg.clear();
     launches_ = bulk_launches_ = 0;
-    ev_used_ = 0; bulk_events_.clear(); sections_.clear(); sec_open_ = -1;
+    reset_timing();
     for (double& v : section_ms) v = 0;
     if (!out || (n_ > 0 && (!out->cluster_id || !out->member_rank || !out->result_order)))
         throw std::invalid_argument("hmk_clinkage_cluster: null output array");
@@ -1901,20 +1923,15 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     int threads = HMK_CL_THREADS;
     if (!sparse) {   // D[q][i] = sequenceScore(seq i, seq q) (symmetric), one batch of profiles at a time
         d_clD_.reserve(n * n);
-        std::vector<int32_t> ids(n_);
-        std::iota(ids.begin(), ids.end(), 0);
-        CK(cudaMemcpyAsync(d_sidx_.p, ids.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, st_));
-        CK(cudaStreamSynchronize(st_));
+        const int32_t* ids = identity_ids();
         const int chunk = HMK_MAXBATCH;
         if (fast_) d_prof_.reserve((size_t)chunk * sc_.prof_words);
         for (int q0 = 0; q0 < n_; q0 += chunk) {
             const int sn = std::min(chunk, n_ - q0);
-            if (fast_) launch_profiles(HMK_PROF_QUERY, d_sidx_.p + q0, sn, d_prof_.p, sc_, st_);
-            HmkBulkArgs a{};
-            a.prof = d_prof_.p; a.nq = sn;
-            a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = 0; a.ndb = n_;
+            HmkBulkArgs a = query_batch(ids + q0, sn, d_prof_.p, (int)opt.kb);
+            a.db_ids = nullptr; a.db_begin = 0; a.ndb = n_;
             a.dense = d_clD_.p + (size_t)q0 * n; a.dense_stride = n_;
-            launch_bulk(HMK_MODE_DENSE, a, d_sidx_.p + q0, 1);
+            launch_bulk(HMK_MODE_DENSE, a, ids + q0, 1);
         }
         hmk_clinkage_threshold<<<sm_count_ * 8, 256, 0, st_>>>(d_clD_.p, n * n, T_);
         stats.bulk_pairs = (int64_t)n * (int64_t)n;
@@ -1953,18 +1970,7 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, ev_a_, ev_c_));
     stats.total_ms = ms; stats.phase1_ms = ms;
-    double bulk_ms = 0;
-    for (auto& pr : bulk_events_) {
-        float t = 0;
-        CK(cudaEventElapsedTime(&t, pr.first, pr.second));
-        bulk_ms += t;
-    }
-    for (auto& sct : sections_) {
-        float t = 0;
-        CK(cudaEventElapsedTime(&t, sct.second.first, sct.second.second));
-        section_ms[sct.first] += t;
-    }
-    stats.bulk_kernel_ms = bulk_ms;
+    stats.bulk_kernel_ms = fold_timing();
     stats.bulk_launches = bulk_launches_; stats.total_launches = launches_;
     stats.p1_steps = sc[3];                          // nearest-neighbour searches
     stats.fast_path = fast_ ? 1 : 0;
@@ -1989,9 +1995,6 @@ int Engine::clinkage(const hmk_greedy_in* in, hmk_greedy_out* out) {
 int Engine::clinkage_rows(int* threads) {
     const int n = n_;
     d_clD_.release();     // the dense matrix of an earlier call on this context
-    std::vector<int32_t> ids(n);
-    std::iota(ids.begin(), ids.end(), 0);
-    CK(cudaMemcpyAsync(d_sidx_.p, ids.data(), sizeof(int32_t) * n, cudaMemcpyHostToDevice, st_));
     const int chunk = HMK_MAXBATCH;
     if (fast_) d_prof_.reserve((size_t)chunk * sc_.prof_words);
     d_cldeg_.reserve((size_t)n + 1); d_cloff_.reserve((size_t)n + 1);
@@ -2079,21 +2082,20 @@ int Engine::clinkage_rows(int* threads) {
 }
 
 // One query batch of the upper-triangle pair search (clinkage_rows, the score graph): the bulk kernel's EMIT mode scores
-// the queries [q0, q0 + sn) (profiles, seq2; d_sidx_[q0 ..] holds their ids) against the thread-side ids [q0, n) (seq1)
+// the queries [q0, q0 + sn) (profiles, seq2) against the thread-side ids [q0, n) (seq1)
 // and writes every pair scoring >= T to d_hits_ as (query - q0, thread-side id, score); pairs with id <= query are among
 // them and are the caller's to drop.  Returns the hit count (count = false: returns 0 without waiting for the batch).
 // cap == 0: a batch whose hits overflow d_hits_ is re-run with a bigger buffer; else at most cap (<= d_hits_.cap) hits
 // are stored, and a count above cap tells the caller to split the batch.
 size_t Engine::emit_hits(int q0, int sn, size_t cap, bool count) {
+    const int32_t* ids = identity_ids() + q0;
     for (;;) {
         const size_t c = cap ? cap : d_hits_.cap;
         CK(cudaMemsetAsync(d_counts_.p, 0, sizeof(unsigned int), st_));
-        if (fast_) launch_profiles(HMK_PROF_QUERY, d_sidx_.p + q0, sn, d_prof_.p, sc_, st_);
-        HmkBulkArgs a{};
-        a.prof = d_prof_.p; a.nq = sn;
-        a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = q0; a.ndb = n_ - q0;
+        HmkBulkArgs a = query_batch(ids, sn, d_prof_.p, (int)opt.kb);
+        a.db_ids = nullptr; a.db_begin = q0; a.ndb = n_ - q0;
         a.hits = d_hits_.p; a.hit_count = d_counts_.p; a.hit_cap = (unsigned int)std::min<size_t>(c, UINT32_MAX);
-        launch_bulk(HMK_MODE_EMIT, a, d_sidx_.p + q0, 1);
+        launch_bulk(HMK_MODE_EMIT, a, ids, 1);
         stats.bulk_pairs += (int64_t)sn * (n_ - q0);
         if (!count) return 0;
         CK(cudaMemcpyAsync(h_scalars_, d_counts_.p, sizeof(unsigned int), cudaMemcpyDeviceToHost, st_));
@@ -2142,18 +2144,12 @@ void Engine::graph_batch(int q0) {
         d_cub_.reserve(bytes);
     }
     int sn = std::min(g.sn, n - q0);
-    std::vector<int32_t> ids(sn);      // profile ids (d_sidx_ also serves phase 2 as an index map)
-    std::iota(ids.begin(), ids.end(), q0);
-    CK(cudaMemcpyAsync(d_sidx_.p + q0, ids.data(), sizeof(int32_t) * sn, cudaMemcpyHostToDevice, st_));
-    if (opt.profile) {          // the bulk launches' event pairs of earlier batches are complete
-        ev_used_ = 0; bulk_events_.clear();
-        CK(cudaEventRecord(ev_a_, st_));
-    }
+    sec(0);
     for (size_t cnt; (cnt = emit_hits(q0, sn, H)) > H;) {
         if (sn == 1) throw std::logic_error("score graph: one query row exceeds the hit buffer");
         sn = std::max(1, std::min(sn / 2, (int)((double)sn * H / cnt)));
     }
-    if (opt.profile) CK(cudaEventRecord(ev_b_, st_));
+    sec(1);
     int jbits = 1, tbits = 1;
     while (((int64_t)1 << jbits) < n) jbits++;
     while ((1 << tbits) < sn) tbits++;
@@ -2175,15 +2171,8 @@ void Engine::graph_batch(int q0) {
         hmk_graph_edges<<<1, 32, 0, st_>>>(g.key[0].p, g.val[0].p, m, q0, jbits, g.edges.p);
     }
     CK(cudaGetLastError());
-    if (opt.profile) {
-        CK(cudaEventRecord(ev_c_, st_));
-        CK(cudaEventSynchronize(ev_c_));
-        float a = 0, b = 0;
-        CK(cudaEventElapsedTime(&a, ev_a_, ev_b_));
-        CK(cudaEventElapsedTime(&b, ev_b_, ev_c_));
-        section_ms[0] += a;
-        section_ms[1] += b;
-    }
+    sec(-1);
+    fold_timing();
     g.row_off.assign(sn + 1, 0);
     for (int t = 0; t < sn; t++) g.row_off[t + 1] = g.row_off[t] + kept[t + 1];
     g.q0 = q0; g.q1 = q0 + sn;
@@ -2203,6 +2192,7 @@ int Engine::score_graph(int64_t* cursor, hmk_graph_edge* out, int64_t cap, int64
         throw std::invalid_argument("hmk_score_graph: cursor outside the graph");
     GraphBatch& g = graph_;
     if (i == 0 && r == 0 && opt.profile) section_ms[0] = section_ms[1] = 0;
+    reset_timing();
     if (!(g.valid && i == g.next_i && r == g.next_r)) g.valid = false;   // only a continuing cursor reuses the kept batch
     if (n_ < 2) i = n_;
     int64_t got = 0;
@@ -2281,12 +2271,9 @@ int Engine::nearest(int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partn
         for (int32_t t = 0; t < n_rows; t++) { count[t] = 0; more[t] = 0; }
         return HMK_OK;
     }
-    // the bulk launch path (qt_max, launch_bulk, launch_planned) reads the list length from opt.kb
-    struct KbScope { Options& o; int64_t saved; ~KbScope() { o.kb = saved; } } kb_scope{opt, opt.kb};
-    opt.kb = k + 1;
     const int kb = k + 1;
     BatchBuf& bb = near_bb_;
-    bb.qid.reserve(HMK_MAXBATCH); bb.gmin.reserve(HMK_MAXBATCH);
+    bb.gmin.reserve(HMK_MAXBATCH);
     bb.bk_key.reserve((size_t)HMK_MAXBATCH * kb); bb.bk_cnt.reserve(HMK_MAXBATCH); bb.bk_ovf.reserve(HMK_MAXBATCH);
     if (fast_) bb.prof.reserve((size_t)HMK_MAXBATCH * sc_.prof_words);
     d_near_out_.reserve((size_t)HMK_MAXBATCH * (3 * k + 2));
@@ -2295,29 +2282,20 @@ int Engine::nearest(int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partn
     int32_t* const o_shift = o_score + (size_t)HMK_MAXBATCH * k;
     int32_t* const o_count = o_shift + (size_t)HMK_MAXBATCH * k;
     int32_t* const o_more = o_count + HMK_MAXBATCH;
-    std::vector<int32_t> ids(HMK_MAXBATCH);
+    const int32_t* ids = identity_ids();
+    reset_timing();
     for (int32_t r0 = row_begin; r0 < row_begin + n_rows; r0 += HMK_MAXBATCH) {
         const int sn = std::min<int32_t>(HMK_MAXBATCH, row_begin + n_rows - r0);
-        std::iota(ids.begin(), ids.begin() + sn, r0);
-        CK(cudaMemcpyAsync(bb.qid.p, ids.data(), sizeof(int32_t) * sn, cudaMemcpyHostToDevice, st_));
-        if (opt.profile) {          // the bulk launches' event pairs of earlier batches are complete
-            ev_used_ = 0; bulk_events_.clear();
-            CK(cudaEventRecord(ev_a_, st_));
-        }
+        sec(0);
         CK(cudaMemsetAsync(bb.gmin.p, 0, sizeof(unsigned long long) * sn, st_));
-        if (fast_) launch_profiles(HMK_PROF_QUERY, bb.qid.p, sn, bb.prof.p, sc_, st_);
-        HmkBulkArgs a{};
-        a.prof = bb.prof.p; a.nq = sn;
-        a.packed = d_packed_.p; a.db_ids = nullptr; a.db_begin = 0; a.ndb = n_;
+        HmkBulkArgs a = query_batch(ids + r0, sn, bb.prof.p, kb);
+        a.db_ids = nullptr; a.db_begin = 0; a.ndb = n_;
         a.tierank = identity_rank_ ? nullptr : d_tierank_.p;
         a.tk_gmin = bb.gmin.p;
-        const HmkBulkArgs p = launch_bulk(HMK_MODE_TOPK, a, bb.qid.p, 1, st_, &bb);
+        const HmkBulkArgs p = launch_bulk(HMK_MODE_TOPK, a, ids + r0, 1, st_, &bb);
         stats.bulk_pairs += (int64_t)sn * n_;
-        if (opt.profile) CK(cudaEventRecord(ev_b_, st_));
-        hmk_topk_merge<<<(sn * 32 + 255) / 256, 256, 0, st_>>>(sn, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p,
-                                                               bb.bk_key.p, bb.bk_cnt.p, bb.bk_ovf.p,
-                                                               p.sched ? p.sched + p.nqt : nullptr, p.qt);
-        CK(cudaGetLastError());
+        sec(1);
+        merge_topk(sn, p.nstripes, kb, bb.tk_key.p, bb.tk_cnt.p, bb.tk_ovf.p, bb, st_, p.sched ? p.sched + p.nqt : nullptr, p.qt);
         HmkNearestArgs na{};
         na.nq = sn; na.k = k; na.r0 = r0; na.n = n_;
         na.key = bb.bk_key.p; na.cnt = bb.bk_cnt.p; na.ovf = bb.bk_ovf.p;
@@ -2326,8 +2304,8 @@ int Engine::nearest(int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partn
         na.partner = o_partner; na.score = o_score; na.shift = o_shift; na.count = o_count; na.more = o_more;
         hmk_nearest_rows<<<(sn * 32 + 255) / 256, 256, 0, st_>>>(na);
         CK(cudaGetLastError());
-        launches_ += 2;
-        if (opt.profile) CK(cudaEventRecord(ev_c_, st_));
+        launches_++;
+        sec(-1);
         const size_t e0 = (size_t)(r0 - row_begin) * k, t0 = (size_t)(r0 - row_begin), ne = (size_t)sn * k;
         CK(cudaMemcpyAsync(partner + e0, o_partner, sizeof(int32_t) * ne, cudaMemcpyDeviceToHost, st_));
         CK(cudaMemcpyAsync(score + e0, o_score, sizeof(int32_t) * ne, cudaMemcpyDeviceToHost, st_));
@@ -2335,13 +2313,7 @@ int Engine::nearest(int32_t k, int32_t row_begin, int32_t n_rows, int32_t* partn
         CK(cudaMemcpyAsync(count + t0, o_count, sizeof(int32_t) * sn, cudaMemcpyDeviceToHost, st_));
         CK(cudaMemcpyAsync(more + t0, o_more, sizeof(int32_t) * sn, cudaMemcpyDeviceToHost, st_));
         CK(cudaStreamSynchronize(st_));
-        if (opt.profile) {
-            float ta = 0, tb = 0;
-            CK(cudaEventElapsedTime(&ta, ev_a_, ev_b_));
-            CK(cudaEventElapsedTime(&tb, ev_b_, ev_c_));
-            section_ms[0] += ta;
-            section_ms[1] += tb;
-        }
+        fold_timing();
     }
     return HMK_OK;
 }

@@ -416,6 +416,63 @@ def test_row_ranges(blosum62):
 
 
 @pytest.mark.gpu
+def test_list_length_is_independent_of_option_kb(blosum62):
+    """the nearest search keeps k + 1 keys per row whatever option kb is, and leaves the option to the partner search:
+    after nearest(31), mode-0 probes on the context return lists of kb keys, equal to those of a context without nearest
+    calls"""
+    n = 1500
+    d = synth.generate(n, 12, 12, seed=5)
+    T, X, _ = synth.default_params(d["lengths"])
+    res, offs, ab = d["residues"], d["offsets"], d["abundance"]
+    want = ref_nearest(res, offs, ab, blosum62, T, X, 0, 31)
+    assert want[4].any()                  # some rows have more than 31 partners
+    q = np.arange(200)
+    ctx = hb.GreedyContext(0)
+    try:
+        ctx.upload(res, offs, ab, blosum62, T, X, 0, 0)
+        for kb in (1, 32):
+            ctx.set_option("kb", kb)
+            _same(ctx.nearest(31), want, kb)
+            got = ctx.bulk_probe(0, q, db_range=(0, n))
+            fresh = hb.GreedyContext(0, kb=kb)
+            try:
+                fresh.upload(res, offs, ab, blosum62, T, X, 0, 0)
+                base = fresh.bulk_probe(0, q, db_range=(0, n))
+            finally:
+                fresh.close()
+            assert got["keys"].shape == (len(q), kb) and got["cnt"].max() == kb
+            assert np.array_equal(got["cnt"], base["cnt"]) and np.array_equal(got["ovf"], base["ovf"]), kb
+            kept = np.arange(kb)[None, :] < got["cnt"][:, None]     # the slots past a list's count are not written
+            assert np.array_equal(got["keys"][kept], base["keys"][kept]), kb
+    finally:
+        ctx.close()
+
+
+@pytest.mark.gpu
+def test_profile_sections(blosum62):
+    """option profile: each call sets section slot 0 to the device time of its scoring passes and slot 1 to that of its
+    merge, score and shift passes; the other slots stay 0"""
+    d = synth.generate(3000, 12, 12, seed=8)
+    T, X, _ = synth.default_params(d["lengths"])
+    ctx = hb.GreedyContext(0, profile=1)
+    try:
+        ctx.upload(d["residues"], d["offsets"], d["abundance"], blosum62, T, X, 0, 0)
+
+        def slots():
+            s = list(ctx.section_ms().values())
+            assert s[0] > 0 and s[1] > 0 and not any(s[2:]), s
+            return s[:2]
+
+        ctx.nearest(8)                    # six batches of rows
+        full = slots()
+        ctx.nearest(8, (0, 10))           # one batch of ten rows: replaces the slots
+        part = slots()
+        assert part[0] < full[0] and part[1] < full[1], (full, part)
+    finally:
+        ctx.close()
+
+
+@pytest.mark.gpu
 def test_statuses(blosum62):
     ctx = hb.GreedyContext(0)
     try:

@@ -351,6 +351,35 @@ def test_paging_and_cursors(blosum62):
 
 
 @pytest.mark.gpu
+def test_profile_sections(blosum62):
+    """option profile: a pull adds the device time of the batches it computes to section slot 0 (scoring passes) and
+    slot 1 (shift, sort and edge passes), and a pull from {0, 0} starts both at 0; the other slots stay 0"""
+    n = 4000
+    d = synth.generate(n, 12, 12, seed=8)
+    T, X, _ = synth.default_params(d["lengths"])
+    ctx = hb.GreedyContext(0, profile=1)
+    try:
+        ctx.upload(d["residues"], d["offsets"], d["abundance"], blosum62, T, X, 0, 0)
+
+        def slots():
+            s = list(ctx.section_ms().values())
+            assert s[0] > 0 and s[1] > 0 and not any(s[2:]), s
+            return s[:2]
+
+        _, cursor = ctx.graph_page((0, 0), 1)       # the first batch of rows
+        first = slots()
+        _, end = ctx.graph_page(cursor, 1 << 24)    # continues through the other seven batches
+        assert end == (n, 0)
+        total = slots()
+        assert total[0] > first[0] and total[1] > first[1], (first, total)
+        ctx.graph_page((0, 0), 1)                   # restarts: the first batch only
+        again = slots()
+        assert again[0] < total[0] and again[1] < total[1], (total, again)
+    finally:
+        ctx.close()
+
+
+@pytest.mark.gpu
 def test_statuses(blosum62):
     ctx = hb.GreedyContext(0)
     try:
